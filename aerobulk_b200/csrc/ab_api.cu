@@ -104,16 +104,6 @@ const double *device_alias(const double *p)
     }
     return (a.type == cudaMemoryTypeHost && a.devicePointer) ? static_cast<const double *>(a.devicePointer) : nullptr;
 }
-// aliases of n host pointers (NULL entries stay NULL); false unless every non-NULL one is pinned
-bool alias_all(int n, const double *const *h, const double **d)
-{
-    if (zerocopy_mode() != 3) return false;
-    for (int k = 0; k < n; ++k) {
-        d[k] = nullptr;
-        if (h[k] && !(d[k] = device_alias(h[k]))) return false;
-    }
-    return true;
-}
 long long min_chunk_points()
 {
     static long long v = [] {
@@ -241,7 +231,7 @@ struct Session {
     // ---- the same for the other host-array entry points (turb, series, ice): arrays packed back to back
     double *hx = nullptr, *hx_dev = nullptr;
     long long cap_hx = 0;
-    // ---- staging of aerobulk_gpu_turb host-array calls (one slab, grow-only)
+    // ---- device slab of the other host-array entry points: staging and scratch (grow-only, see ensure_turb_slab)
     double *d_turb = nullptr;
     long long cap_turb = 0;
     // ---- stability-sort permutation (one uint16 per point, see classify_kernel)
@@ -523,111 +513,50 @@ void free_bounce()
     g.hx = g.hx_dev = nullptr;
     g.cap_hx = 0;
 }
-// false (and the session stays usable) when the host has no pinned memory to spare: the caller then keeps the
-// driver-staged copies
+// Grows a mapped pinned slab to n rows of `rows` doubles (cap counts n).  False, with the slab released, when the host
+// has no pinned memory to spare: the session stays usable and the caller keeps the driver-staged copies.
+bool grow_mapped(double *&h, double *&d, long long &cap, long long n, int rows)
+{
+    if (n <= cap) return true;
+    if (h) cudaFreeHost(h);
+    h = d = nullptr;
+    cap = 0;
+    if (cudaHostAlloc(&h, sizeof(double) * (size_t)n * rows, cudaHostAllocPortable | cudaHostAllocMapped) != cudaSuccess ||
+        cudaHostGetDevicePointer(&d, h, 0) != cudaSuccess) {
+        cudaGetLastError();
+        if (h) cudaFreeHost(h);
+        h = d = nullptr;
+        return false;
+    }
+    cap = n;
+    return true;
+}
 bool ensure_bounce(long long n)
 {
     if (n <= g.cap_hb) return true;
     if (sizeof(double) * (size_t)n * 14 > bounce_max_bytes()) return false;
     free_bounce();
-    if (cudaHostAlloc(&g.hb, sizeof(double) * (size_t)n * 14, cudaHostAllocPortable | cudaHostAllocMapped) != cudaSuccess ||
-        cudaHostGetDevicePointer(&g.hb_dev, g.hb, 0) != cudaSuccess) {
-        cudaGetLastError();
-        if (g.hb) cudaFreeHost(g.hb);
-        g.hb = g.hb_dev = nullptr;
-        return false;
-    }
-    g.cap_hb = n;
-    return true;
+    return grow_mapped(g.hb, g.hb_dev, g.cap_hb, n, 14);
+}
+// appends the copy of len doubles from src to dst, cut into COPY_PIECE_BYTES pieces for the copy threads
+void add_pieces(std::vector<CopyPiece> &pieces, double *dst, const double *src, long long len)
+{
+    const long long step = (long long)(COPY_PIECE_BYTES / sizeof(double));
+    for (long long o = 0; o < len; o += step)
+        pieces.push_back(CopyPiece{dst + o, src + o, sizeof(double) * (size_t)(len - o < step ? len - o : step)});
 }
 // copy points [s0, s0+len) of nf fields between the caller's arrays and the bounce slab rows row0.., on the copy threads
 void bounce_copy(int nf, double *const *user, int row0, long long s0, long long len, bool to_slab)
 {
     static thread_local std::vector<CopyPiece> pieces;
     pieces.clear();
-    const long long step = (long long)(COPY_PIECE_BYTES / sizeof(double));
     for (int k = 0; k < nf; ++k) {
         if (!user[k]) continue;
-        double *slab = g.hb + (long long)(row0 + k) * g.cap_hb;
-        for (long long o = 0; o < len; o += step) {
-            const long long m = len - o < step ? len - o : step;
-            double *u = user[k] + s0 + o, *b = slab + s0 + o;
-            pieces.push_back(to_slab ? CopyPiece{b, u, sizeof(double) * (size_t)m} : CopyPiece{u, b, sizeof(double) * (size_t)m});
-        }
+        double *u = user[k] + s0, *b = g.hb + (long long)(row0 + k) * g.cap_hb + s0;
+        if (to_slab) add_pieces(pieces, b, u, len);
+        else add_pieces(pieces, u, b, len);
     }
     pool_run(pieces.data(), (int)pieces.size());
-}
-
-
-// Host arrays of the entry points other than aerobulk_gpu_model (turb, series, turb_ice, oce_ice).  Every array pinned:
-// device aliases (zero-copy).  Otherwise, from BOUNCE_MIN_POINTS elements per array up, the copy threads pack the
-// inputs into a pinned slab, the kernel works on the slab zero-copy, and bounce_finish() brings the outputs home
-// (pageable cudaMemcpy is staged by the driver on one thread at ~14 GB/s; the copy threads move 55-70 GB/s).
-struct HostBounce {
-    int cnt = 0;
-    double *user[64];
-    long long len[64], off[64];
-    unsigned char dir[64];   // bit 0: input, bit 1: output
-    bool active = false;
-};
-void bounce_run(const HostBounce &hb, unsigned char which, bool to_slab)
-{
-    static thread_local std::vector<CopyPiece> pieces;
-    pieces.clear();
-    const long long step = (long long)(COPY_PIECE_BYTES / sizeof(double));
-    for (int k = 0; k < hb.cnt; ++k) {
-        if (!hb.user[k] || !(hb.dir[k] & which)) continue;
-        for (long long o = 0; o < hb.len[k]; o += step) {
-            const long long m = hb.len[k] - o < step ? hb.len[k] - o : step;
-            double *u = hb.user[k] + o, *b = g.hx + hb.off[k] + o;
-            pieces.push_back(to_slab ? CopyPiece{b, u, sizeof(double) * (size_t)m} : CopyPiece{u, b, sizeof(double) * (size_t)m});
-        }
-    }
-    pool_run(pieces.data(), (int)pieces.size());
-}
-// 0: use the staged path of the entry point; 1: d = aliases of the caller's pinned arrays; 2: d = aliases of slab rows
-// holding copies of the inputs (call bounce_finish after the launch); < 0: -error code
-int alias_or_bounce(int cnt, const double *const *h, const long long *len, const unsigned char *dir, const double **d,
-                    HostBounce &hb)
-{
-    hb.active = false;
-    if (alias_all(cnt, h, d)) return 1;
-    if (!bounce_on() || zerocopy_mode() != 3 || cnt > 64) return 0;
-    long long total = 0, longest = 0;
-    for (int k = 0; k < cnt; ++k) {
-        hb.user[k] = const_cast<double *>(h[k]);
-        hb.len[k] = h[k] ? len[k] : 0;
-        hb.dir[k] = dir[k];
-        hb.off[k] = total;
-        total += (hb.len[k] + 63) / 64 * 64;   // rows start on 512-byte boundaries
-        longest = hb.len[k] > longest ? hb.len[k] : longest;
-    }
-    hb.cnt = cnt;
-    if (longest < BOUNCE_MIN_POINTS || sizeof(double) * (size_t)total > bounce_max_bytes()) return 0;
-    if (total > g.cap_hx) {
-        if (g.hx) cudaFreeHost(g.hx);
-        g.hx = g.hx_dev = nullptr;
-        g.cap_hx = 0;
-        if (cudaHostAlloc(&g.hx, sizeof(double) * (size_t)total, cudaHostAllocPortable | cudaHostAllocMapped) != cudaSuccess ||
-            cudaHostGetDevicePointer(&g.hx_dev, g.hx, 0) != cudaSuccess) {
-            cudaGetLastError();   // no pinned memory to spare: the staged path still works
-            if (g.hx) cudaFreeHost(g.hx);
-            g.hx = g.hx_dev = nullptr;
-            return 0;
-        }
-        g.cap_hx = total;
-    }
-    bounce_run(hb, 1, true);
-    for (int k = 0; k < cnt; ++k) d[k] = h[k] ? g.hx_dev + hb.off[k] : nullptr;
-    hb.active = true;
-    return 2;
-}
-int bounce_finish(const HostBounce &hb, int rc)
-{
-    if (!hb.active || rc) return rc;
-    CUDA_TRY(cudaStreamSynchronize(compute_stream()));
-    bounce_run(hb, 2, false);
-    return 0;
 }
 
 int algo_id(const char *calgo)
@@ -1559,6 +1488,120 @@ int model_host(int jt, int Nt, const char *calgo, double zt, double zu, int Ni, 
     return rc;
 }
 
+// device slab of the staged host-array calls and of device-only scratch (grow-only)
+int ensure_turb_slab(long long need)
+{
+    if (need > g.cap_turb) {
+        if (g.d_turb) cudaFree(g.d_turb);
+        g.d_turb = nullptr;
+        g.cap_turb = 0;
+        if (need > 0) CUDA_TRY(cudaMalloc(&g.d_turb, sizeof(double) * (size_t)need));
+        g.cap_turb = need;
+    }
+    return 0;
+}
+
+// ---------------------------------------------------------------------------
+// Caller arrays of the entry points other than aerobulk_gpu_model (turb, series, turb_ice, oce_ice, series_ice).  The
+// entry point registers each array with its length and role and asks for device-only scratch; open() stores a device
+// pointer in every registered slot, close() brings the outputs home.  open() picks the first mode that applies:
+//   DEVICE  the caller passed device pointers: they pass through, nothing moves, close() does nothing;
+//   ALIAS   every array is pinned (cudaHostAlloc / cudaHostRegister) and zerocopy_mode() == 3: the kernel works on the
+//           caller's memory through its device aliases;
+//   BOUNCE  from BOUNCE_MIN_POINTS elements up, the copy threads pack the inputs into the pinned slab g.hx, the kernel
+//           works on the slab zero-copy and the copy threads bring the outputs home (pageable cudaMemcpy is staged by
+//           the driver on one thread at ~14 GB/s; the copy threads move 55-70 GB/s);
+//   STAGED  cudaMemcpyAsync through the device slab g.d_turb on the compute stream.
+// The three host modes block in close().  Scratch lives in g.d_turb in every mode.
+// ---------------------------------------------------------------------------
+struct HostTransport {
+    enum Mode { DEVICE, ALIAS, BOUNCE, STAGED };
+    struct Array {
+        double **slot;          // receives the device pointer
+        double *host;           // the caller's pointer; NULL: absent (the slot gets NULL)
+        long long len, off;     // elements; offset in the packed slab
+        bool in, home;          // copied in before the launch / home after it
+        double *dev;            // what open() stores in the slot
+    };
+    std::vector<Array> arrays, scratch_rows;
+    Mode mode = DEVICE;
+
+    void in(const double **slot, const double *h, long long len)
+    {
+        arrays.push_back({const_cast<double **>(slot), const_cast<double *>(h), len, 0, true, false, nullptr});
+    }
+    void out(double **slot, double *h, long long len, bool home = true) { arrays.push_back({slot, h, len, 0, false, home, nullptr}); }
+    void inout(double **slot, double *h, long long len, bool home) { arrays.push_back({slot, h, len, 0, true, home, nullptr}); }
+    void scratch(double **slot, long long len) { scratch_rows.push_back({slot, nullptr, len, 0, false, false, nullptr}); }
+
+    Mode pick(long long total, long long longest)
+    {
+        if (zerocopy_mode() != 3) return STAGED;
+        bool pinned = true;
+        for (Array &a : arrays)
+            if (a.host && !(a.dev = const_cast<double *>(device_alias(a.host)))) {
+                pinned = false;
+                break;
+            }
+        if (pinned) return ALIAS;
+        if (!bounce_on() || longest < BOUNCE_MIN_POINTS || sizeof(double) * (size_t)total > bounce_max_bytes() ||
+            !grow_mapped(g.hx, g.hx_dev, g.cap_hx, total, 1))
+            return STAGED;
+        return BOUNCE;
+    }
+    // the copy threads move every array with `in` (to the slab) or `home` (from it)
+    void bounce(bool to_slab)
+    {
+        std::vector<CopyPiece> pieces;
+        for (const Array &a : arrays)
+            if (a.host && (to_slab ? a.in : a.home)) {
+                if (to_slab) add_pieces(pieces, g.hx + a.off, a.host, a.len);
+                else add_pieces(pieces, a.host, g.hx + a.off, a.len);
+            }
+        pool_run(pieces.data(), (int)pieces.size());
+    }
+    int open(int on_device)
+    {
+        long long total = 0, longest = 0;
+        for (Array &a : arrays) {
+            const long long m = (a.host && a.len > 0) ? a.len : 0;
+            a.off = total;
+            total += (m + 63) / 64 * 64;   // rows start on 512-byte boundaries
+            longest = m > longest ? m : longest;
+        }
+        mode = on_device ? DEVICE : pick(total, longest);
+        long long need = mode == STAGED ? total : 0;
+        for (Array &s : scratch_rows) {
+            s.off = need;
+            need += (s.len + 63) / 64 * 64;
+        }
+        const int rc = ensure_turb_slab(need);
+        if (rc) return rc;
+        for (Array &s : scratch_rows) *s.slot = g.d_turb + s.off;
+        for (Array &a : arrays) {
+            if (!a.host || mode == DEVICE) a.dev = a.host;
+            else if (mode == BOUNCE) a.dev = g.hx_dev + a.off;
+            else if (mode == STAGED) a.dev = g.d_turb + a.off;
+            if (mode == STAGED && a.host && a.in && a.len > 0)
+                CUDA_TRY(cudaMemcpyAsync(a.dev, a.host, sizeof(double) * (size_t)a.len, cudaMemcpyHostToDevice, compute_stream()));
+            *a.slot = a.dev;
+        }
+        if (mode == BOUNCE) bounce(true);
+        return 0;
+    }
+    int close()
+    {
+        if (mode == DEVICE) return 0;
+        if (mode == STAGED)
+            for (const Array &a : arrays)
+                if (a.host && a.home && a.len > 0)
+                    CUDA_TRY(cudaMemcpyAsync(a.host, a.dev, sizeof(double) * (size_t)a.len, cudaMemcpyDeviceToHost, compute_stream()));
+        CUDA_TRY(cudaStreamSynchronize(compute_stream()));
+        if (mode == BOUNCE) bounce(false);
+        return 0;
+    }
+};
+
 // ---------------------------------------------------------------------------
 // TURB_* (SURVEY.md 8f row 1)
 // ---------------------------------------------------------------------------
@@ -1615,41 +1658,18 @@ int turb_impl(const char *calgo, int kt, double zt, double zu, int Ni, int Nj, d
     a.n = n;
     a.first_step = (kt == 1);
     double *optp[10] = {nullptr};
-    if (opt) {
-        optp[0] = opt->CdN; optp[1] = opt->ChN; optp[2] = opt->CeN; optp[3] = opt->xz0; optp[4] = opt->xu_star;
-        optp[5] = opt->xL; optp[6] = opt->xUN10; optp[7] = opt->pdT_cs; optp[8] = opt->pdT_wl; optp[9] = opt->pHz_wl;
-    }
-    // host arrays: 5 in/out + 4 skin inputs + 6 outputs + 10 optionals staged in one slab
-    const double *hin[9] = {T_s, q_s, t_zt, q_zt, U_zu, Qsw, rad_lw, slp, plong};
-    double *hout[18] = {T_s, q_s, Cd, Ch, Ce, t_zu, q_zu, Ubzu, optp[0], optp[1], optp[2], optp[3], optp[4],
-                        optp[5], optp[6], optp[7], optp[8], optp[9]};
-    double *din[9], *dout[18];
-    if (on_device) {
-        for (int k = 0; k < 9; ++k) din[k] = const_cast<double *>(hin[k]);
-        for (int k = 0; k < 18; ++k) dout[k] = hout[k];
-    } else {
-        const long long need = n * 25;
-        if (need > g.cap_turb) {
-            if (g.d_turb) cudaFree(g.d_turb);
-            g.d_turb = nullptr;
-            g.cap_turb = 0;
-            if (need > 0) CUDA_TRY(cudaMalloc(&g.d_turb, sizeof(double) * (size_t)need));
-            g.cap_turb = need;
-        }
-        for (int k = 0; k < 9; ++k) {
-            din[k] = hin[k] ? g.d_turb + (long long)k * n : nullptr;
-            if (hin[k] && n > 0)
-                CUDA_TRY(cudaMemcpyAsync(din[k], hin[k], sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, cs_));
-        }
-        dout[0] = din[0];
-        dout[1] = din[1];
-        for (int k = 2; k < 18; ++k) dout[k] = hout[k] ? g.d_turb + (long long)(7 + k) * n : nullptr;
-    }
-    a.T_s = dout[0]; a.q_s = dout[1];
-    a.t_zt = din[2]; a.q_zt = din[3]; a.U_zu = din[4];
-    a.Qsw = din[5]; a.rad_lw = din[6]; a.slp = din[7]; a.lon = din[8];
-    a.Cd = dout[2]; a.Ch = dout[3]; a.Ce = dout[4]; a.t_zu = dout[5]; a.q_zu = dout[6]; a.Ubzu = dout[7];
-    for (int k = 0; k < 10; ++k) a.opt[k] = dout[8 + k];
+    static_assert(sizeof(aerobulk_gpu_turb_optional) == 10 * sizeof(double *), "10 optional outputs");
+    if (opt) memcpy(optp, opt, sizeof(*opt));
+    HostTransport t;
+    t.inout(&a.T_s, T_s, n, cs || wl);   // T_s, q_s come back only from the skin schemes
+    t.inout(&a.q_s, q_s, n, cs || wl);
+    t.in(&a.t_zt, t_zt, n); t.in(&a.q_zt, q_zt, n); t.in(&a.U_zu, U_zu, n);
+    t.in(&a.Qsw, Qsw, n); t.in(&a.rad_lw, rad_lw, n); t.in(&a.slp, slp, n); t.in(&a.lon, plong, n);
+    t.out(&a.Cd, Cd, n); t.out(&a.Ch, Ch, n); t.out(&a.Ce, Ce, n); t.out(&a.t_zu, t_zu, n); t.out(&a.q_zu, q_zu, n);
+    t.out(&a.Ubzu, Ubzu, n);
+    for (int k = 0; k < 10; ++k) t.out(&a.opt[k], optp[k], n);
+    rc = t.open(on_device);
+    if (rc) return rc;
     if (wl) {
         if (ialgo == abd::ECMWF) {
             a.dT_wl = g.e_dT_wl;
@@ -1659,16 +1679,11 @@ int turb_impl(const char *calgo, int kt, double zt, double zu, int Ni, int Nj, d
     }
     CUDA_TRY(abk::launch_turb(ialgo, cs, wl, fabs(zu - zt) < 0.01, a, cs_));
     g.launches += 1;
-    if (!on_device) {
-        const bool skin = cs || wl;
-        for (int k = skin ? 0 : 2; k < 18; ++k)
-            if (hout[k] && n > 0)
-                CUDA_TRY(cudaMemcpyAsync(hout[k], dout[k], sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, cs_));
-        CUDA_TRY(cudaStreamSynchronize(cs_));
-    }
+    rc = t.close();
+    if (rc) return rc;
     // kt == nitend -> *_EXIT
     if (wl && kt == g.nitend) {
-        if (on_device) CUDA_TRY(cudaStreamSynchronize(cs_));
+        CUDA_TRY(cudaStreamSynchronize(cs_));
         if (ialgo == abd::ECMWF) release_ecmwf_state();
         else release_coare_state();
     }
@@ -1704,7 +1719,6 @@ int series_impl(const char *calgo, int Nt, long long S, double zt, double zu, co
         out->rho_zu, out->QL, out->QH, out->Qlw, out->QNS, out->Qsw, out->dT_cs, out->dT_wl, out->TAU, out->dT,
         out->Hz_wl, out->Qnt_ac, out->Tau_ac, out->Cd, out->Ce, out->Ch, out->theta_zu, out->q_zu, out->t_zu,
         out->RiB, out->z0, out->u_star, out->L, out->UN10, out->Ts, out->Evap, out->q_zt, out->theta_zt};
-    const double *hin[7] = {sst, t_zt, hum_zt, wind, slp, rad_sw, rad_lw};
 
     abk::SeriesArgs a;
     memset(&a, 0, sizeof(a));
@@ -1714,51 +1728,22 @@ int series_impl(const char *calgo, int Nt, long long S, double zt, double zu, co
     a.u = make_uniform(zt, zu);
     a.bad_index = g.d_bad;
 
-    // one slab: [isd as doubles' worth of ints | lon | 7 inputs | wanted outputs]
-    int nout = 0;
-    for (int k = 0; k < abk::NSERIES_OUT; ++k) nout += hout[k] ? 1 : 0;
-    const long long isd_words = ((long long)Nt * (long long)sizeof(int) + 7) / 8;
-    const long long need = isd_words + (on_device ? 0 : S + (7 + nout) * n);
-    if (need > g.cap_turb) {
-        if (g.d_turb) cudaFree(g.d_turb);
-        g.d_turb = nullptr;
-        g.cap_turb = 0;
-        CUDA_TRY(cudaMalloc(&g.d_turb, sizeof(double) * (size_t)need));
-        g.cap_turb = need;
-    }
-    int *d_isd = reinterpret_cast<int *>(g.d_turb);
+    HostTransport t;
+    double *d_isd;   // isecday_utc is a host array in every mode
+    t.scratch(&d_isd, ((long long)Nt * (long long)sizeof(int) + 7) / 8);
+    t.in(&a.lon, lon, S);
+    t.in(&a.sst, sst, n); t.in(&a.t_zt, t_zt, n); t.in(&a.hum_zt, hum_zt, n); t.in(&a.wnd, wind, n); t.in(&a.slp, slp, n);
+    t.in(&a.rad_sw, rad_sw, n); t.in(&a.rad_lw, rad_lw, n);
+    for (int k = 0; k < abk::NSERIES_OUT; ++k) t.out(&a.out[k], hout[k], n);
+    rc = t.open(on_device);
+    if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(d_isd, isd, sizeof(int) * (size_t)Nt, cudaMemcpyHostToDevice, cs_));
-    a.isd = d_isd;
-    double *dout[abk::NSERIES_OUT];
-    if (on_device) {
-        a.lon = lon;
-        a.sst = sst; a.t_zt = t_zt; a.hum_zt = hum_zt; a.wnd = wind; a.slp = slp; a.rad_sw = rad_sw; a.rad_lw = rad_lw;
-        for (int k = 0; k < abk::NSERIES_OUT; ++k) dout[k] = hout[k];
-    } else {
-        double *p = g.d_turb + isd_words;
-        CUDA_TRY(cudaMemcpyAsync(p, lon, sizeof(double) * (size_t)S, cudaMemcpyHostToDevice, cs_));
-        a.lon = p;
-        p += S;
-        const double *din[7];
-        for (int k = 0; k < 7; ++k) {
-            CUDA_TRY(cudaMemcpyAsync(p, hin[k], sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, cs_));
-            din[k] = p;
-            p += n;
-        }
-        a.sst = din[0]; a.t_zt = din[1]; a.hum_zt = din[2]; a.wnd = din[3]; a.slp = din[4]; a.rad_sw = din[5]; a.rad_lw = din[6];
-        for (int k = 0; k < abk::NSERIES_OUT; ++k) {
-            dout[k] = hout[k] ? p : nullptr;
-            if (hout[k]) p += n;
-        }
-    }
-    for (int k = 0; k < abk::NSERIES_OUT; ++k) a.out[k] = dout[k];
+    a.isd = reinterpret_cast<const int *>(d_isd);
     CUDA_TRY(abk::launch_series(ialgo, skin, fabs(zu - zt) < 0.01, a, cs_));
     g.launches += 1;
     CUDA_TRY(cudaMemcpyAsync(g.h_bad, g.d_bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, cs_));
-    if (!on_device)
-        for (int k = 0; k < abk::NSERIES_OUT; ++k)
-            if (hout[k])
-                CUDA_TRY(cudaMemcpyAsync(hout[k], dout[k], sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, cs_));
+    rc = t.close();
+    if (rc) return rc;
     CUDA_TRY(cudaStreamSynchronize(cs_));
     const unsigned long long bad = *g.h_bad;
     if (bad != ~0ull) {
@@ -1991,18 +1976,6 @@ int finish_ice_call(cudaStream_t cs_, const char *what)
     return 0;
 }
 
-int ensure_turb_slab(long long need)
-{
-    if (need > g.cap_turb) {
-        if (g.d_turb) cudaFree(g.d_turb);
-        g.d_turb = nullptr;
-        g.cap_turb = 0;
-        if (need > 0) CUDA_TRY(cudaMalloc(&g.d_turb, sizeof(double) * (size_t)need));
-        g.cap_turb = need;
-    }
-    return 0;
-}
-
 int turb_ice_impl(const char *calgo, double zt, double zu, int Ni, int Nj, const double *Ts_i, const double *t_zt,
                   const double *qs_i, const double *q_zt, const double *U_zu, const double *frice, const double *cxn,
                   double *Cd, double *Ch, double *Ce, double *t_zu, double *q_zu, double *Ubzu,
@@ -2027,45 +2000,26 @@ int turb_ice_impl(const char *calgo, double zt, double zu, int Ni, int Nj, const
     if (rc) return rc;
 
     double *optp[8] = {nullptr};
-    if (opt) {
-        optp[0] = opt->CdN; optp[1] = opt->ChN; optp[2] = opt->CeN; optp[3] = opt->xz0; optp[4] = opt->xu_star;
-        optp[5] = opt->xL; optp[6] = opt->xUN10; optp[7] = opt->CdN_frm;
-    }
-    const double *hin[6] = {Ts_i, t_zt, qs_i, q_zt, U_zu, need_frice ? frice : nullptr};
-    double *hout[14] = {Cd, Ch, Ce, t_zu, q_zu, Ubzu, optp[0], optp[1], optp[2], optp[3], optp[4], optp[5], optp[6], optp[7]};
-    const double *din[6];
-    double *dout[14];
-    if (on_device) {
-        for (int k = 0; k < 6; ++k) din[k] = hin[k];
-        for (int k = 0; k < 14; ++k) dout[k] = hout[k];
-    } else {
-        rc = ensure_turb_slab(n * 20);
-        if (rc) return rc;
-        double *p = g.d_turb;
-        for (int k = 0; k < 6; ++k) {
-            din[k] = hin[k] ? p : nullptr;
-            if (hin[k]) CUDA_TRY(cudaMemcpyAsync(p, hin[k], sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, cs_));
-            p += n;
-        }
-        for (int k = 0; k < 14; ++k) {
-            dout[k] = hout[k] ? p : nullptr;
-            p += n;
-        }
-    }
+    static_assert(sizeof(aerobulk_gpu_turb_ice_optional) == 8 * sizeof(double *), "8 optional outputs");
+    if (opt) memcpy(optp, opt, sizeof(*opt));
     abk::IceTurbArgs a;
     memset(&a, 0, sizeof(a));
-    a.Ts_i = din[0]; a.t_zt = din[1]; a.qs_i = din[2]; a.q_zt = din[3]; a.U_zu = din[4]; a.frice = din[5];
-    a.Cd = dout[0]; a.Ch = dout[1]; a.Ce = dout[2]; a.t_zu = dout[3]; a.q_zu = dout[4]; a.Ubzu = dout[5];
-    for (int k = 0; k < 8; ++k) a.opt[k] = dout[6 + k];
+    HostTransport t;
+    t.in(&a.Ts_i, Ts_i, n); t.in(&a.t_zt, t_zt, n); t.in(&a.qs_i, qs_i, n); t.in(&a.q_zt, q_zt, n); t.in(&a.U_zu, U_zu, n);
+    t.in(&a.frice, need_frice ? frice : nullptr, n);
+    t.out(&a.Cd, Cd, n); t.out(&a.Ch, Ch, n); t.out(&a.Ce, Ce, n); t.out(&a.t_zu, t_zu, n); t.out(&a.q_zu, q_zu, n);
+    t.out(&a.Ubzu, Ubzu, n);
+    for (int k = 0; k < 8; ++k) t.out(&a.opt[k], optp[k], n);
+    rc = t.open(on_device);
+    if (rc) return rc;
     a.n = n;
     a.form_index = g.ice_form_per_point ? -1 : n - 1;
     a.u = make_ice_uniform(zt, zu, cxn);
     a.bad_rough = g.d_bad + 1;
     CUDA_TRY(abk::launch_ice_turb(ialgo, fabs(zu - zt) < 0.01, a, cs_));
     g.launches += 1;
-    if (!on_device)
-        for (int k = 0; k < 14; ++k)
-            if (hout[k]) CUDA_TRY(cudaMemcpyAsync(hout[k], dout[k], sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, cs_));
+    rc = t.close();
+    if (rc) return rc;
     return finish_ice_call(cs_, "aerobulk_gpu_turb_ice");
 }
 
@@ -2096,46 +2050,20 @@ int oce_ice_impl(const char *calgo_ice, const char *calgo_oce, double zt, double
         out->u_star_i, out->L_i, out->UN10_i, out->rho_zu_i, out->Tau_i, out->QH_i, out->QL_i, out->Evap_i,
         out->Cd_w, out->Ch_w, out->Ce_w, out->theta_zu_w, out->q_zu_w, out->Ub_w, out->z0_w, out->u_star_w, out->L_w,
         out->UN10_w, out->Tau_w, out->QH_w, out->QL_w, out->Evap_w, out->Tau, out->QH, out->QL, out->Evap};
-    const double *hin[7] = {sit, oalgo ? sst : nullptr, t_zt, hum_zt, wind, slp, frice};
-    int nout = 0;
-    for (int k = 0; k < abk::NOCEICE_OUT; ++k) nout += hout[k] ? 1 : 0;
-    // scratch for the four ice fluxes the cell means need when the caller does not want them
-    int nscratch = 0;
-    if (oalgo)
-        for (int k = 0; k < 4; ++k) nscratch += hout[13 + k] ? 0 : 1;
-    rc = ensure_turb_slab(n * ((on_device ? 0 : 7 + nout) + nscratch));
-    if (rc) return rc;
-    double *p = g.d_turb;
-    const double *din[7];
-    double *dout[abk::NOCEICE_OUT];
-    if (on_device) {
-        for (int k = 0; k < 7; ++k) din[k] = hin[k];
-        for (int k = 0; k < abk::NOCEICE_OUT; ++k) dout[k] = hout[k];
-    } else {
-        for (int k = 0; k < 7; ++k) {
-            din[k] = hin[k] ? p : nullptr;
-            if (hin[k]) {
-                CUDA_TRY(cudaMemcpyAsync(p, hin[k], sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, cs_));
-                p += n;
-            }
-        }
-        for (int k = 0; k < abk::NOCEICE_OUT; ++k) {
-            dout[k] = hout[k] ? p : nullptr;
-            if (hout[k]) p += n;
-        }
-    }
     abk::OceIceArgs a;
     memset(&a, 0, sizeof(a));
-    a.sit = din[0]; a.sst = din[1]; a.t_zt = din[2]; a.hum_zt = din[3]; a.wnd = din[4]; a.slp = din[5]; a.frice = din[6];
-    for (int k = 0; k < abk::NOCEICE_OUT; ++k) a.out[k] = dout[k];
-    if (oalgo)
-        for (int k = 0; k < 4; ++k) {
-            a.ice_flux[k] = dout[13 + k];
-            if (!a.ice_flux[k]) {
-                a.ice_flux[k] = p;
-                p += n;
-            }
-        }
+    HostTransport t;
+    t.in(&a.sit, sit, n); t.in(&a.sst, oalgo ? sst : nullptr, n); t.in(&a.t_zt, t_zt, n); t.in(&a.hum_zt, hum_zt, n);
+    t.in(&a.wnd, wind, n); t.in(&a.slp, slp, n); t.in(&a.frice, frice, n);
+    // the leads kernel writes out[17..34]: without leads they stay as the caller passed them
+    for (int k = 0; k < abk::NOCEICE_OUT; ++k) t.out(&a.out[k], hout[k], n, oalgo || k < 17);
+    // scratch for the four ice fluxes the cell means need when the caller does not want them
+    for (int k = 0; k < 4 && oalgo; ++k)
+        if (!hout[13 + k]) t.scratch(&a.ice_flux[k], n);
+    rc = t.open(on_device);
+    if (rc) return rc;
+    for (int k = 0; k < 4 && oalgo; ++k)
+        if (hout[13 + k]) a.ice_flux[k] = a.out[13 + k];
     a.n = n;
     a.form_index = g.ice_form_per_point ? -1 : n - 1;
     a.hum_kind = hum_kind;
@@ -2150,10 +2078,8 @@ int oce_ice_impl(const char *calgo_ice, const char *calgo_oce, double zt, double
         CUDA_TRY(abk::launch_leads(oalgo, zteq, a, cs_));
         g.launches += 1;
     }
-    if (!on_device)
-        for (int k = 0; k < abk::NOCEICE_OUT; ++k)
-            if (hout[k] && (oalgo || k < 17))
-                CUDA_TRY(cudaMemcpyAsync(hout[k], dout[k], sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, cs_));
+    rc = t.close();
+    if (rc) return rc;
     return finish_ice_call(cs_, "aerobulk_gpu_oce_ice");
 }
 
@@ -2182,32 +2108,14 @@ int series_ice_impl(const char *calgo, double zt, double zu, long long n, const 
     static_assert(sizeof(aerobulk_gpu_series_ice_out) == abk::NICESERIES_OUT * sizeof(double *), "21 output pointers");
     double *hout[abk::NICESERIES_OUT];
     memcpy(hout, out, sizeof(hout));
-    const double *hin[8] = {sic, sit, t_zt, hum_zt, wind, slp, rad_sw, rad_lw};
-    const double *din[8];
-    double *dout[abk::NICESERIES_OUT];
-    if (on_device) {
-        for (int k = 0; k < 8; ++k) din[k] = hin[k];
-        for (int k = 0; k < abk::NICESERIES_OUT; ++k) dout[k] = hout[k];
-    } else {
-        int nout = 0;
-        for (int k = 0; k < abk::NICESERIES_OUT; ++k) nout += hout[k] ? 1 : 0;
-        rc = ensure_turb_slab(n * (8 + nout));
-        if (rc) return rc;
-        double *p = g.d_turb;
-        for (int k = 0; k < 8; ++k, p += n) {
-            din[k] = p;
-            CUDA_TRY(cudaMemcpyAsync(p, hin[k], sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, cs_));
-        }
-        for (int k = 0; k < abk::NICESERIES_OUT; ++k) {
-            dout[k] = hout[k] ? p : nullptr;
-            if (hout[k]) p += n;
-        }
-    }
     abk::IceSeriesArgs a;
     memset(&a, 0, sizeof(a));
-    a.sic = din[0]; a.sit = din[1]; a.t_zt = din[2]; a.hum_zt = din[3]; a.wnd = din[4]; a.slp = din[5];
-    a.rad_sw = din[6]; a.rad_lw = din[7];
-    for (int k = 0; k < abk::NICESERIES_OUT; ++k) a.out[k] = dout[k];
+    HostTransport t;
+    t.in(&a.sic, sic, n); t.in(&a.sit, sit, n); t.in(&a.t_zt, t_zt, n); t.in(&a.hum_zt, hum_zt, n); t.in(&a.wnd, wind, n);
+    t.in(&a.slp, slp, n); t.in(&a.rad_sw, rad_sw, n); t.in(&a.rad_lw, rad_lw, n);
+    for (int k = 0; k < abk::NICESERIES_OUT; ++k) t.out(&a.out[k], hout[k], n);
+    rc = t.open(on_device);
+    if (rc) return rc;
     a.n = n;
     a.hum_kind = hum_kind;
     a.ui = make_ice_uniform(zt, zu, nullptr);
@@ -2215,9 +2123,8 @@ int series_ice_impl(const char *calgo, double zt, double zu, long long n, const 
     a.bad_rough = g.d_bad + 1;
     CUDA_TRY(abk::launch_ice_series(ialgo, fabs(zu - zt) < 0.01, a, cs_));
     g.launches += 1;
-    if (!on_device)
-        for (int k = 0; k < abk::NICESERIES_OUT; ++k)
-            if (hout[k]) CUDA_TRY(cudaMemcpyAsync(hout[k], dout[k], sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, cs_));
+    rc = t.close();
+    if (rc) return rc;
     return finish_ice_call(cs_, "aerobulk_gpu_series_ice");
 }
 
@@ -2335,33 +2242,6 @@ int aerobulk_gpu_turb(const char *calgo, int kt, double zt, double zu, int Ni, i
                       const aerobulk_gpu_turb_optional *opt, int on_device)
 {
     std::lock_guard<std::mutex> lk(g_mu);
-    if (!on_device && T_s && q_s && ensure_device() == 0) {
-        // every array pinned: zero-copy (see zerocopy_mode); the device-pointer path is asynchronous, hence the wait
-        const double *h[25] = {T_s, q_s, t_zt, q_zt, U_zu, Qsw, rad_lw, slp, plong, Cd, Ch, Ce, t_zu, q_zu, Ubzu};
-        static_assert(sizeof(aerobulk_gpu_turb_optional) == 10 * sizeof(double *), "10 optional outputs");
-        if (opt) memcpy(h + 15, opt, sizeof(*opt));
-        else memset(h + 15, 0, 10 * sizeof(double *));
-        const double *d[25];
-        long long len[25];
-        unsigned char dir[25];
-        const unsigned char io = (l_use_cs || l_use_wl) ? 3 : 1;   // T_s, q_s come back only from the skin schemes
-        for (int k = 0; k < 25; ++k) {
-            len[k] = (long long)Ni * Nj;
-            dir[k] = k < 2 ? io : (k < 9 ? 1 : 2);
-        }
-        HostBounce hb;
-        if (alias_or_bounce(25, h, len, dir, d, hb)) {
-            aerobulk_gpu_turb_optional od;
-            memcpy(&od, d + 15, sizeof(od));
-            auto w = [](const double *p) { return const_cast<double *>(p); };
-            const int rc = turb_impl(calgo, kt, zt, zu, Ni, Nj, w(d[0]), d[2], w(d[1]), d[3], d[4], l_use_cs, l_use_wl, w(d[9]),
-                                     w(d[10]), w(d[11]), w(d[12]), w(d[13]), w(d[14]), d[5], d[6], d[7], isecday_utc, d[8],
-                                     opt ? &od : nullptr, 1);
-            if (rc) return rc;
-            CUDA_TRY(cudaStreamSynchronize(compute_stream()));
-            return bounce_finish(hb, 0);
-        }
-    }
     return turb_impl(calgo, kt, zt, zu, Ni, Nj, T_s, t_zt, q_s, q_zt, U_zu, l_use_cs, l_use_wl, Cd, Ch, Ce, t_zu, q_zu,
                      Ubzu, Qsw, rad_lw, slp, isecday_utc, plong, opt, on_device);
 }
@@ -2372,25 +2252,6 @@ int aerobulk_gpu_series(const char *calgo, int Nt, long long S, double zt, doubl
                         int l_use_skin, const aerobulk_gpu_series_out *out, int on_device)
 {
     std::lock_guard<std::mutex> lk(g_mu);
-    if (!on_device && out && lon && sst && t_zt && hum_zt && wind && slp && rad_sw && rad_lw && ensure_device() == 0) {
-        // every array pinned: the kernel works on the caller's memory directly (zero-copy, see zerocopy_mode)
-        const double *h[8 + AEROBULK_GPU_SERIES_NOUT] = {lon, sst, t_zt, hum_zt, wind, slp, rad_sw, rad_lw};
-        memcpy(h + 8, out, sizeof(double *) * AEROBULK_GPU_SERIES_NOUT);
-        const double *d[8 + AEROBULK_GPU_SERIES_NOUT];
-        long long len[8 + AEROBULK_GPU_SERIES_NOUT];
-        unsigned char dir[8 + AEROBULK_GPU_SERIES_NOUT];
-        for (int k = 0; k < 8 + AEROBULK_GPU_SERIES_NOUT; ++k) {
-            len[k] = k == 0 ? S : (long long)(Nt < 0 ? 0 : Nt) * (S < 0 ? 0 : S);   // lon is per station
-            dir[k] = k < 8 ? 1 : 2;
-        }
-        HostBounce hb;
-        if (alias_or_bounce(8 + AEROBULK_GPU_SERIES_NOUT, h, len, dir, d, hb)) {
-            aerobulk_gpu_series_out od;
-            memcpy(&od, d + 8, sizeof(od));
-            return bounce_finish(hb, series_impl(calgo, Nt, S, zt, zu, isecday_utc, d[0], d[1], d[2], d[3], hum_kind, d[4], d[5],
-                                                 d[6], d[7], l_use_skin, &od, 1));
-        }
-    }
     return series_impl(calgo, Nt, S, zt, zu, isecday_utc, lon, sst, t_zt, hum_zt, hum_kind, wind, slp, rad_sw, rad_lw,
                        l_use_skin, out, on_device);
 }
@@ -2408,27 +2269,6 @@ int aerobulk_gpu_turb_ice(const char *calgo, double zt, double zu, int Ni, int N
                           double *Ubzu, const aerobulk_gpu_turb_ice_optional *opt, int on_device)
 {
     std::lock_guard<std::mutex> lk(g_mu);
-    if (!on_device && Ts_i && ensure_device() == 0) {
-        const double *h[20] = {Ts_i, t_zt, qs_i, q_zt, U_zu, frice, Cd, Ch, Ce, t_zu, q_zu, Ubzu};
-        static_assert(sizeof(aerobulk_gpu_turb_ice_optional) == 8 * sizeof(double *), "8 optional outputs");
-        if (opt) memcpy(h + 12, opt, sizeof(*opt));
-        else memset(h + 12, 0, 8 * sizeof(double *));
-        const double *d[20];
-        long long len[20];
-        unsigned char dir[20];
-        for (int k = 0; k < 20; ++k) {
-            len[k] = (long long)Ni * Nj;
-            dir[k] = k < 6 ? 1 : 2;
-        }
-        HostBounce hb;
-        if (alias_or_bounce(20, h, len, dir, d, hb)) {
-            aerobulk_gpu_turb_ice_optional od;
-            memcpy(&od, d + 12, sizeof(od));
-            auto w = [](const double *p) { return const_cast<double *>(p); };
-            return bounce_finish(hb, turb_ice_impl(calgo, zt, zu, Ni, Nj, d[0], d[1], d[2], d[3], d[4], d[5], CxN_easy, w(d[6]),
-                                                   w(d[7]), w(d[8]), w(d[9]), w(d[10]), w(d[11]), opt ? &od : nullptr, 1));
-        }
-    }
     return turb_ice_impl(calgo, zt, zu, Ni, Nj, Ts_i, t_zt, qs_i, q_zt, U_zu, frice, CxN_easy, Cd, Ch, Ce, t_zu, q_zu, Ubzu,
                          opt, on_device);
 }
@@ -2439,25 +2279,6 @@ int aerobulk_gpu_oce_ice(const char *calgo_ice, const char *calgo_oce, double zt
                          const aerobulk_gpu_oce_ice_out *out, int on_device)
 {
     std::lock_guard<std::mutex> lk(g_mu);
-    if (!on_device && out && sit && t_zt && hum_zt && wind && slp && frice && ensure_device() == 0) {
-        const double *h[7 + 35] = {sit, sst, t_zt, hum_zt, wind, slp, frice};
-        static_assert(sizeof(aerobulk_gpu_oce_ice_out) == 35 * sizeof(double *), "35 output pointers");
-        memcpy(h + 7, out, sizeof(aerobulk_gpu_oce_ice_out));
-        const double *d[7 + 35];
-        long long len[7 + 35];
-        unsigned char dir[7 + 35];
-        for (int k = 0; k < 7 + 35; ++k) {
-            len[k] = n < 0 ? 0 : n;
-            dir[k] = k < 7 ? 1 : ((calgo_oce || k < 7 + 17) ? 2 : 0);   // the over-water outputs exist only with leads
-        }
-        HostBounce hb;
-        if (alias_or_bounce(7 + 35, h, len, dir, d, hb)) {
-            aerobulk_gpu_oce_ice_out od;
-            memcpy(&od, d + 7, sizeof(od));
-            return bounce_finish(hb, oce_ice_impl(calgo_ice, calgo_oce, zt, zu, n, d[0], d[1], d[2], d[3], hum_kind, d[4], d[5],
-                                                  d[6], CxN_easy, &od, 1));
-        }
-    }
     return oce_ice_impl(calgo_ice, calgo_oce, zt, zu, n, sit, sst, t_zt, hum_zt, hum_kind, wind, slp, frice, CxN_easy, out,
                         on_device);
 }
@@ -2467,25 +2288,6 @@ int aerobulk_gpu_series_ice(const char *calgo, double zt, double zu, long long n
                             const double *rad_sw, const double *rad_lw, const aerobulk_gpu_series_ice_out *out, int on_device)
 {
     std::lock_guard<std::mutex> lk(g_mu);
-    if (!on_device && out && sic && sit && t_zt && hum_zt && wind && slp && rad_sw && rad_lw && ensure_device() == 0) {
-        constexpr int NO = abk::NICESERIES_OUT;
-        const double *h[8 + NO] = {sic, sit, t_zt, hum_zt, wind, slp, rad_sw, rad_lw};
-        memcpy(h + 8, out, sizeof(double *) * NO);
-        const double *d[8 + NO];
-        long long len[8 + NO];
-        unsigned char dir[8 + NO];
-        for (int k = 0; k < 8 + NO; ++k) {
-            len[k] = n < 0 ? 0 : n;
-            dir[k] = k < 8 ? 1 : 2;
-        }
-        HostBounce hb;
-        if (alias_or_bounce(8 + NO, h, len, dir, d, hb)) {
-            aerobulk_gpu_series_ice_out od;
-            memcpy(&od, d + 8, sizeof(od));
-            return bounce_finish(hb, series_ice_impl(calgo, zt, zu, n, d[0], d[1], d[2], d[3], hum_kind, d[4], d[5], d[6], d[7],
-                                                     &od, 1));
-        }
-    }
     return series_ice_impl(calgo, zt, zu, n, sic, sit, t_zt, hum_zt, hum_kind, wind, slp, rad_sw, rad_lw, out, on_device);
 }
 
@@ -2512,16 +2314,12 @@ int aerobulk_gpu_selftest_host_copy(long long n, int rounds)
     // no device needed: exercises the copy threads of the pageable-array path on host memory alone
     if (n < 1 || rounds < 1) return -1;
     std::vector<double> src((size_t)n), mid((size_t)n), dst((size_t)n);
-    const long long step = (long long)(COPY_PIECE_BYTES / sizeof(double));
     int bad = 0;
     for (int r = 0; r < rounds; ++r) {
         for (long long i = 0; i < n; ++i) src[(size_t)i] = (double)(i * 31 + r);
         std::vector<CopyPiece> there, back;
-        for (long long o = 0; o < n; o += step) {
-            const size_t m = (size_t)(n - o < step ? n - o : step);
-            there.push_back(CopyPiece{mid.data() + o, src.data() + o, sizeof(double) * m});
-            back.push_back(CopyPiece{dst.data() + o, mid.data() + o, sizeof(double) * m});
-        }
+        add_pieces(there, mid.data(), src.data(), n);
+        add_pieces(back, dst.data(), mid.data(), n);
         copy_pool().run(there.data(), (int)there.size());
         copy_pool().run(back.data(), (int)back.size());
         bad += memcmp(src.data(), dst.data(), sizeof(double) * (size_t)n) != 0;
