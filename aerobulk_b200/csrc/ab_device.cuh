@@ -134,7 +134,7 @@ constexpr double INV_GRAV = 1. / GRAV;
 ABD double virt_temp(double T, double q) { return T * (1. + KC(RCTV0) * q); }           // :247-269
 
 // Goff (1957) saturation vapour pressure [Pa], :777-800 (rt0, not the triple point)
-ABD_HEAVY double e_sat(double T)
+ABD_HEAVY double e_sat_goff(double T)
 {
     const double zta = abm::dmax(T, 180.);
     const double ztmp = fdiv(KC(RT0), zta);
@@ -144,6 +144,9 @@ ABD_HEAVY double e_sat(double T)
                      + KC(0.42873 * 1.e-3) * (abm::dexp10_b(KC(4.76955) * (1. - ztmp)) - 1.) + KC(0.78614);
     return 100. * abm::dexp10_b(a);   // T is floored at 180 K: every exponent of this function is inside [-4, 4]
 }
+// On [230, 330) K, every temperature of the ocean path, the same function from a piecewise polynomial
+// (abm::esat_table, within 2 ulp of the formula; ~25 instructions instead of ~115); elsewhere, and for NaN, the formula.
+ABD double e_sat(double T) { return (T >= 230. && T < 330.) ? abm::esat_table(T) : e_sat_goff(T); }
 ABD double q_sat_from_e(double es, double p) { return fdiv(KC(REPS0) * es, p - KC(1. - REPS0) * es); }  // :903
 ABD double q_sat(double T, double p) { return q_sat_from_e(e_sat(T), p); }                   // :881-904
 

@@ -1,4 +1,4 @@
-// ab_math.cuh -- the kernels' own FP64 exp / exp10 / log / log10 / atan / pow.
+// ab_math.cuh -- the kernels' own FP64 exp / exp10 / log / log10 / atan / pow, and Goff's e_sat as a piecewise polynomial.
 //
 // Why not libdevice: ptxas builds every FP64 literal of CUDA's math functions with two 32-bit moves
 // (UMOV / IMAD.MOV), which made ~35 % of the issued instructions of the flux kernels and a 188 KB
@@ -26,6 +26,7 @@
 #define ABM_TABLE static const
 #define ABM_GTABLE static const
 #define ABM_LDG(p) (*(p))
+struct double2 { double x, y; };
 namespace abm {
 static inline int hi_word(double x) { int64_t b; std::memcpy(&b, &x, 8); return (int)(b >> 32); }
 static inline int lo_word(double x) { int64_t b; std::memcpy(&b, &x, 8); return (int)(b & 0xffffffff); }
@@ -222,22 +223,27 @@ ABM_BIG double dlog_poly(double x)
 #define ABM_SMEM_TABLES 1   // measured 3 % faster than __ldg of the global tables (64-bit address arithmetic)
 #endif
 #if ABM_SMEM_TABLES && !defined(ABM_HOST_TEST)
-// block-local copies of the tables in shared memory (4.5 KB; 32-bit addressing, LDS instead of LDG);
-// every kernel must call abm::load_tables() (all threads) before the first exp/log
+// block-local copies of the tables in shared memory (4.5 KB, and 3.2 KB of e_sat coefficients; 32-bit addressing, LDS
+// instead of LDG); every kernel must call abm::load_tables() (all threads) before the first exp/log/esat_table
 __shared__ double S_EXP_T[64];
 __shared__ double S_LOG_T[512];
+__shared__ __align__(16) double S_ESAT_T[8 * ESAT_ROWS];
 ABM_FN void load_tables()
 {
     for (int i = threadIdx.x; i < 64; i += blockDim.x) S_EXP_T[i] = EXP_T[i];
     for (int i = threadIdx.x; i < 512; i += blockDim.x) S_LOG_T[i] = LOG_T[i];
+    for (int i = threadIdx.x; i < 4 * ESAT_ROWS; i += blockDim.x)
+        reinterpret_cast<double2 *>(S_ESAT_T)[i] = reinterpret_cast<const double2 *>(ESAT_T)[i];
     __syncthreads();
 }
 #define ABM_EXP_T(i) S_EXP_T[i]
 #define ABM_LOG_T(i) S_LOG_T[i]
+#define ABM_ESAT_T2(i) reinterpret_cast<const double2 *>(S_ESAT_T)[i]
 #else
 ABM_FN void load_tables() {}
 #define ABM_EXP_T(i) ABM_LDG(&EXP_T[i])
 #define ABM_LOG_T(i) ABM_LDG(&LOG_T[i])
+#define ABM_ESAT_T2(i) ABM_LDG(reinterpret_cast<const double2 *>(ESAT_T) + (i))
 #endif
 
 // exp(r) for |r| <= ln2/128 times 2^(k/64), k = 64 m + j
@@ -330,6 +336,24 @@ ABM_FN double dlog(double x) { return dlog_table(x); }
 #endif
 
 ABM_FN double dlog10(double x) { return dlog(x) * MATH_K[K_LOG10E]; }
+
+// Goff's saturation vapour pressure over water [Pa] for 229 <= T < 331 (the caller checks the range) from the
+// piecewise polynomial ESAT_T: ~25 instructions instead of the quotient, log10 and three exp10 of the formula (~115),
+// within 2 ulp of it.  Row m = rint(T / h) is centred on T_c = h m; T - T_c is exact (|T - T_c| <= h / 2 and h is a
+// power of two), so the only rounding is the evaluation's.  Estrin form: e_sat sits on the dependent chain of the
+// skin loops.  The four coefficient pairs of a row are ESAT_ROWS apart (tools/gen_math_tables.py: bank spread).
+ABM_FN double esat_table(double T)
+{
+    const double MAGIC = 6755399441055744.0;   // 1.5 * 2^52: adding it rounds to nearest integer
+    const double t = fma(T, 1. / ESAT_H, MAGIC);
+    const double x = fma(t - MAGIC, -ESAT_H, T) * (2. / ESAT_H);
+    const int i = lo_word(t) - ESAT_M0;
+    const double2 c01 = ABM_ESAT_T2(i), c23 = ABM_ESAT_T2(i + ESAT_ROWS), c45 = ABM_ESAT_T2(i + 2 * ESAT_ROWS),
+                  c67 = ABM_ESAT_T2(i + 3 * ESAT_ROWS);
+    const double x2 = x * x;
+    const double a0 = fma(c01.y, x, c01.x), a1 = fma(c23.y, x, c23.x), a2 = fma(c45.y, x, c45.x), a3 = fma(c67.y, x, c67.x);
+    return fma(fma(a3, x2, a2), x2 * x2, fma(a1, x2, a0));
+}
 
 // atan(t) for |t| <= tan(pi/8) (Estrin)
 ABM_FN double atan_core(double t)

@@ -1,21 +1,23 @@
 """Regenerates the measured tables of DESIGN.md (the blocks between <!-- BEGIN:x --> / <!-- END:x --> markers) from the
 committed evidence files, so that the document always quotes the files it names.
 
-    python tools/design_numbers.py [<tag> [--bench-tag <tag2>]] [--check]        (no tag: profiles/CURRENT.json)
+    python tools/design_numbers.py [<tag> [--bench-tag <tag2>] [--kbench-tag <tag3>]] [--check]   (no tag: profiles/CURRENT.json)
 
 reads profiles/bench_<tag>.json, profiles/launches_<tag>_summary.txt, profiles/traffic.json,
-profiles/kbench_1440x720_<tag>.txt, profiles/kbench_4320x2160_<tag>.txt; --check only reports whether DESIGN.md is current."""
+profiles/kbench_1440x720_<tag>.txt, profiles/kbench_4320x2160_<tag>.txt; --check only reports whether DESIGN.md is current.
+The bench line and the kbench files may come from a later checkpoint than the ncu captures (--bench-tag, --kbench-tag)."""
 import json, os, re, sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 P = lambda *a: os.path.join(ROOT, "profiles", *a)
-pos = [a for i, a in enumerate(sys.argv[1:], 1) if not a.startswith("--") and sys.argv[i - 1] != "--bench-tag"]
+pos = [a for i, a in enumerate(sys.argv[1:], 1) if not a.startswith("--") and sys.argv[i - 1] not in ("--bench-tag", "--kbench-tag")]
 if pos:
     tag = pos[0]
     btag = sys.argv[sys.argv.index("--bench-tag") + 1] if "--bench-tag" in sys.argv else tag   # bench line of a later checkpoint
+    ktag = sys.argv[sys.argv.index("--kbench-tag") + 1] if "--kbench-tag" in sys.argv else tag
 else:                                    # the checkpoint DESIGN.md currently quotes
     cur = json.load(open(P("CURRENT.json")))
-    tag, btag = cur["tag"], cur["bench_tag"]
+    tag, btag, ktag = cur["tag"], cur["bench_tag"], cur.get("kbench_tag", cur["tag"])
 bench = json.loads(open(P(f"bench_{btag}.json")).read().strip().splitlines()[-1])
 traffic = json.load(open(P("traffic.json")))
 NAMES = {"ncar": "NCAR", "andreas": "ANDREAS", "coare3p0": "COARE 3.0", "coare3p6": "COARE 3.6", "ecmwf": "ECMWF",
@@ -101,7 +103,7 @@ def kb(path):
     return out
 
 
-small, large = kb(P(f"kbench_1440x720_{tag}.txt")), kb(P(f"kbench_4320x2160_{tag}.txt"))
+small, large = kb(P(f"kbench_1440x720_{ktag}.txt")), kb(P(f"kbench_4320x2160_{ktag}.txt"))
 rows = ["| algorithm | 1440×720 (C2 size) | 4320×2160 (C3/C4 size) |", "|---|---|---|"]
 one = lambda d, k: f"{d[k][0]:.3f} ms · {d[k][1]:.1f} Gpt/s"
 two = lambda d, a, b: f"{d[a][0]:.3f} / {d[b][0]:.3f} ms · {d[a][1]:.1f} / {d[b][1]:.1f} Gpt/s"
