@@ -3,15 +3,13 @@
 import numpy as np
 import pytest
 
+import parity_util as pu
 from aerobulk_b200 import synth
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-10   # scaled metric of tests/test_gpu_parity.py: |gpu-ref| / (|ref| + S_f)
 OPT = ("CdN", "ChN", "CeN", "xz0", "xu_star", "xL", "xUN10", "CdN_frm")
-SCALE = {"Cd": 1e-3, "Ch": 1e-3, "Ce": 1e-3, "t_zu": 1.0, "q_zu": 1e-3, "Ubzu": 1e-2, "CdN": 1e-3, "ChN": 1e-3, "CeN": 1e-3,
-         "xz0": 1e-5, "xu_star": 1e-2, "xL": 1e-2, "xUN10": 1e-2, "CdN_frm": 1e-3,
-         "theta_zu": 1.0, "Ub": 1e-2, "RiB": 1e-2, "z0": 1e-5, "u_star": 1e-2, "L": 1e-2, "UN10": 1e-2, "rho_zu": 1.0,
-         "Tau": 1e-2, "QH": 10.0, "QL": 10.0, "Evap": 1e-5}
+SCALE = pu.ICE_SCALE
 
 
 @pytest.fixture(scope="module")
@@ -21,10 +19,23 @@ def ab():
     return ab
 
 
-def _compare(tag, got, ref, keys, flux_of=None):
-    """At most 2e-5 of the points above TOL (near-calm / vanishing-difference points amplify rounding noise), none
-    above 1e-6.  Ch and Ce are 0/0 at a vanishing air-surface difference: only compared where |dtheta|, |dq| is sizeable."""
+def _prove(tag, worst_pt, inputs, run_oracle, scale):
+    """Every point above TOL must sit where the oracle itself moves under ulp-level input nudges, or where such a nudge
+    trips the reference's rough_leng_tq fail-stop (parity_util.prove_flips)."""
+    bad = np.flatnonzero(worst_pt > TOL)
+    print(f"[parity] {tag}: n={worst_pt.size} max {worst_pt.max():.3e} points>1e-10: {bad.size}")
+    if bad.size:
+        proven = pu.prove_flips(bad, worst_pt[bad], inputs, run_oracle, tag, scale=scale, failstop=10)
+        assert proven.all(), (tag, "points above 1e-10 where the oracle is NOT sensitive to ulp-level input nudges",
+                              bad[~proven].tolist(), worst_pt[bad][~proven].tolist())
+
+
+def _compare(tag, got, ref, keys, flux_of, inputs, run_oracle):
+    """At most 2e-5 of the points above TOL (near-calm / vanishing-difference points amplify rounding noise), and each
+    of them proven by _prove.  Ch and Ce are 0/0 at a vanishing air-surface difference: only compared where |dtheta|,
+    |dq| is sizeable."""
     worst = 0.0
+    worst_pt = np.zeros(np.size(got[keys[0]]))
     for k in keys:
         g, r = np.ravel(got[k]), np.ravel(ref[k])
         base = k[:-2] if k.endswith(("_i", "_w")) else k
@@ -36,8 +47,9 @@ def _compare(tag, got, ref, keys, flux_of=None):
         assert np.all(np.isfinite(g)), (tag, k)
         bad = int((e > TOL).sum())
         assert bad <= max(1, int(2e-5 * e.size)), (tag, k, bad, float(e.max()))
-        assert float(e.max()) <= 1e-6, (tag, k, float(e.max()))
         worst = max(worst, float(np.sort(e)[-2]))
+        worst_pt = np.maximum(worst_pt, e)
+    _prove(tag, worst_pt, inputs, run_oracle, pu.ice_scale(keys))
     return worst
 
 
@@ -86,7 +98,10 @@ def test_turb_ice_matches_oracle(ab, algo, zt, nb_iter):
                         f, ab.AerobulkError, OracleError)
     siq = f["siq"]
     dth, dq = np.abs(ref["t_zu"] - f["sit"]) > 0.05, np.abs(ref["q_zu"] - siq) > 2e-5
-    worst = _compare(f"turb_ice {algo}", got, ref, ("Cd", "Ch", "Ce", "t_zu", "q_zu", "Ubzu") + OPT, {"Ch": dth, "Ce": dq})
+    inputs = dict(Ts_i=f["sit"], t_zt=f["tha"], qs_i=siq, q_zt=f["hum_zt"], U_zu=f["wind"], frice=f["frice"])
+    last = {k: v[-1] for k, v in inputs.items()} if algo.startswith("lg15") else None
+    worst = _compare(f"turb_ice {algo}", got, ref, ("Cd", "Ch", "Ce", "t_zu", "q_zu", "Ubzu") + OPT, {"Ch": dth, "Ce": dq},
+                     inputs, pu.turb_ice_runner(OracleSession, algo, zt, 10.0, nb_iter, cxn, last))
     assert worst <= TOL
     if algo.startswith("lg15"):   # reference behaviour: one form drag for all, from the last point
         assert np.all(got["CdN_frm"] == got["CdN_frm"][0])
@@ -103,7 +118,9 @@ def test_lg15_per_point_form_drag(ab):
     o = OracleSession(threads=8)
     ref = o.turb_ice("lg15", 2.0, 10.0, f["sit"], tha, siq, f["hum_zt"], f["wind"], frice=f["frice"], per_point_form_drag=True, want=OPT)
     dth, dq = np.abs(ref["t_zu"] - f["sit"]) > 0.05, np.abs(ref["q_zu"] - siq) > 2e-5
-    assert _compare("lg15 per point", got, ref, ("Cd", "Ch", "Ce", "t_zu", "q_zu") + OPT, {"Ch": dth, "Ce": dq}) <= TOL
+    inputs = dict(Ts_i=f["sit"], t_zt=tha, qs_i=siq, q_zt=f["hum_zt"], U_zu=f["wind"], frice=f["frice"])
+    assert _compare("lg15 per point", got, ref, ("Cd", "Ch", "Ce", "t_zu", "q_zu") + OPT, {"Ch": dth, "Ce": dq}, inputs,
+                    pu.turb_ice_runner(OracleSession, "lg15", 2.0, 10.0, o.nb_iter, per_point_form_drag=True)) <= TOL
     assert len(np.unique(got["CdN_frm"])) > 100
 
 
@@ -127,7 +144,10 @@ def test_oce_ice_matches_oracle(ab, ice, oce, hum):
     keys = [k for k in ab.OCE_ICE_OUT if oce is not None or k.endswith("_i")]
     sizeable = {"Ch_i": np.abs(ref["QH_i"]) > 1.0, "Ce_i": np.abs(ref["QL_i"]) > 1.0,
                 "Ch_w": np.abs(ref["QH_w"]) > 1.0, "Ce_w": np.abs(ref["QL_w"]) > 1.0}
-    assert _compare(f"oce_ice {ice}+{oce}", got, ref, keys, sizeable) <= TOL
+    inputs = {k: f[k] for k in ("sit", "sst", "t_zt", "hum_zt", "wind", "slp", "frice")}
+    last = {k: v[-1] for k, v in inputs.items()} if ice.startswith("lg15") else None
+    run = pu.oce_ice_runner(OracleSession, ice, oce, 2.0, 10.0, 20, {"q": 0, "dp": 1, "rh": 2}[hum], cxn, last)
+    assert _compare(f"oce_ice {ice}+{oce}", got, ref, keys, sizeable, inputs, run) <= TOL
     if oce is None:
         assert np.all(got["QH_w"] == 0.0) and np.all(got["Tau"] == 0.0)
     else:
@@ -203,6 +223,7 @@ def test_series_ice_matches_oracle(ab, algo, zt, hum):
     ren = {"Cd_i": "Cd", "Ch_i": "Ch", "Ce_i": "Ce", "TAU": "Tau", "SBLM": "Evap", "Ublk": "Ub", "RiB_zt": "RiB", "RiB_zu": "RiB",
            "Qlw": "QH", "QNS": "QH", "Qsw": "QH"}
     worst = 0.0
+    worst_pt = np.zeros(n)
     for k in ab.SERIES_ICE_OUT:
         g, r = got[k], ref[k]
         assert np.all(np.isfinite(g)), k
@@ -218,8 +239,10 @@ def test_series_ice_matches_oracle(ab, algo, zt, hum):
             e = np.where(np.abs(ref["QL"]) > 1.0, e, 0.0)
         bad = int((e > TOL).sum())
         assert bad <= max(1, int(2e-5 * n)), (algo, k, bad, float(e.max()))
-        assert float(e.max()) <= 1e-6, (algo, k, float(e.max()))
         worst = max(worst, float(np.sort(e)[-2]))
+        worst_pt = np.maximum(worst_pt, e)
+    _prove(f"series_ice {algo} zt={zt} {hum}", worst_pt, f, pu.series_ice_runner(OracleSession, algo, zt, 10.0, 20, hk),
+           pu.ice_scale(ab.SERIES_ICE_OUT))
     assert worst <= TOL
     # a subset of outputs gives the same bits
     part = ab.series_ice(algo, zt, 10.0, **f, hum_kind=hum, want=("QNS", "TAU"))

@@ -4,6 +4,7 @@ independently, optional outputs (CdN, ChN, CeN, z0, u*, L, UN10, dT_cs, dT_wl, H
 import numpy as np
 import pytest
 
+import parity_util as pu
 from aerobulk_b200 import synth
 
 pytestmark = pytest.mark.gpu
@@ -29,18 +30,23 @@ def _inputs(Ni, Nj):
     return f, np.asfortranarray(ssq), np.asfortranarray(theta), np.asfortranarray(wnd), lon
 
 
-def _cmp(tag, got, ref, keys, n):
+def _cmp(tag, got, ref, keys, n, inputs, run_oracle):
+    """Scaled error per output (S_f: parity_util.TURB_SCALE; L compared as 1/L).  A non-finite output fails; at most
+    max(1, 2e-5 n) points of an output above TOL, and every point above TOL must be proven to sit where the oracle
+    itself is sensitive to ulp-level input nudges (parity_util.prove_flips with run_oracle)."""
+    g, r = pu.metric_view({k: got[k] for k in keys}), pu.metric_view({k: ref[k] for k in keys})
+    worst = np.zeros(n)
     for k in keys:
-        g, r = np.ravel(got[k], order="F"), np.ravel(ref[k], order="F")
-        scale = {"xL": 1.0, "T_s": 1.0, "t_zu": 1.0, "xUN10": 1e-2, "Ubzu": 1e-2, "pHz_wl": 1e-2}.get(k, 0.0)
-        # L = 1/(1/L) blows up at neutrality: compare 1/L instead
-        if k == "xL":
-            g, r = 1.0 / g, 1.0 / r
-            scale = 1e-3
-        e = np.abs(g - r) / (np.abs(r) + scale + 1e-300)
+        assert np.all(np.isfinite(g[k])), (tag, k, "non-finite output")
+        e = pu.scaled_error(g[k], r[k], pu.TURB_SCALE[k])
         bad = int((e > TOL).sum())
         assert bad <= max(1, int(2e-5 * n)), (tag, k, bad, float(e.max()))
-        assert float(np.sort(e)[-2] if e.size > 1 else e.max()) <= 1e-9, (tag, k, float(e.max()))
+        worst = np.maximum(worst, e)
+    bad = np.flatnonzero(worst > TOL)
+    if bad.size:
+        proven = pu.prove_flips(bad, worst[bad], inputs, run_oracle, tag, scale={k: pu.TURB_SCALE[k] for k in keys})
+        assert proven.all(), (tag, "points above 1e-10 where the oracle is NOT sensitive to ulp-level input nudges",
+                              bad[~proven].tolist(), worst[bad][~proven].tolist())
 
 
 @pytest.mark.parametrize("algo", ["ncar", "andreas", "coare3p0", "coare3p6", "ecmwf"])
@@ -55,7 +61,9 @@ def test_turb_noskin_with_optional_outputs(ab, algo):
     o.set_nb_iter(8)
     ref = o.turb(algo, 1, 2.0, 10.0, f["sst"], theta, ssq, f["hum_zt"], wnd, want=WANT)
     assert np.array_equal(got["T_s"], f["sst"]) and np.array_equal(got["q_s"], ssq)   # untouched without skin
-    _cmp(f"turb {algo}", got, ref, ("Cd", "Ch", "Ce", "t_zu", "q_zu", "Ubzu") + WANT, Ni * Nj)
+    inputs = dict(T_s=f["sst"], t_zt=theta, q_s=ssq, q_zt=f["hum_zt"], U_zu=wnd)
+    _cmp(f"turb {algo}", got, ref, ("Cd", "Ch", "Ce", "t_zu", "q_zu", "Ubzu") + WANT, Ni * Nj, inputs,
+         pu.turb_runner(OracleSession, algo, 2.0, 10.0, 8))
 
 
 @pytest.mark.parametrize("algo,cs,wl", [("coare3p6", True, False), ("coare3p6", False, True), ("coare3p6", True, True),
@@ -75,15 +83,22 @@ def test_turb_skin_day_cycle_with_real_solar_time(ab, algo, cs, wl):
     want = ("xu_star",) + (("pdT_cs",) if cs else ()) + (("pdT_wl", "pHz_wl") if wl else ())
     resets = 0
     prev_dT = None
+    qsw_all = []
     for kt in range(1, Nt + 1):
         isd = 3600 * (kt - 1)
         # net solar flux following the LOCAL solar hour of each longitude
         hr = (isd / 3600.0 + lon / 15.0) % 24.0
         qsw = np.asfortranarray(np.maximum(0.0, 800.0 * np.sin(np.pi * (hr - 6.0) / 12.0)))
+        qsw_all.append(qsw)
         kw = dict(l_use_cs=cs, l_use_wl=wl, Qsw=qsw, rad_lw=f["rad_lw"], slp=f["slp"], isecday_utc=isd, plong=lon, want=want)
         got = ab.turb(algo, kt, 2.0, 10.0, f["sst"], theta, ssq, f["hum_zt"], wnd, **kw)
         ref = o.turb(algo, kt, 2.0, 10.0, f["sst"], theta, ssq, f["hum_zt"], wnd, **kw)
-        _cmp(f"turb {algo} cs={cs} wl={wl} kt={kt}", got, ref, ("Cd", "Ch", "Ce", "t_zu", "q_zu", "Ubzu", "T_s", "q_s") + want, Ni * Nj)
+        inputs = dict(T_s=f["sst"], t_zt=theta, q_s=ssq, q_zt=f["hum_zt"], U_zu=wnd, Qsw=list(qsw_all), rad_lw=f["rad_lw"],
+                      slp=f["slp"], plong=lon)
+        run = pu.turb_runner(OracleSession, algo, 2.0, 10.0, 5, cs, wl, isecday=[3600 * (j - 1) for j in range(1, kt + 1)],
+                             nitend=Nt)
+        _cmp(f"turb {algo} cs={cs} wl={wl} kt={kt}", got, ref, ("Cd", "Ch", "Ce", "t_zu", "q_zu", "Ubzu", "T_s", "q_s") + want,
+             Ni * Nj, inputs, lambda pi: run(pi)[-1:])
         if wl and algo != "ecmwf":
             dT = np.ravel(got["pdT_wl"], order="F")
             if prev_dT is not None:
