@@ -41,12 +41,6 @@ namespace {
 
 constexpr int MAX_CHUNKS = 16;          // capacity; the number used is chunk_limit() (default 6, measured best)
 constexpr long long MIN_CHUNK_POINTS = 200000;
-#ifndef AEROBULK_GPU_COPY_STREAMING_DEFAULT
-#define AEROBULK_GPU_COPY_STREAMING_DEFAULT 1
-#endif
-#ifndef AEROBULK_GPU_ZEROCOPY_DEFAULT
-#define AEROBULK_GPU_ZEROCOPY_DEFAULT 3
-#endif
 
 // tuning knobs of the host-array pipeline (experiments: tools/diag_e2e.py)
 int chunk_limit()
@@ -58,39 +52,17 @@ int chunk_limit()
     }();
     return v;
 }
-// AEROBULK_GPU_TRACE=1: GPU timeline of every host-array call (H2D / kernel / D2H end of each chunk) on stderr
-bool trace_env()
-{
-    static bool v = [] { const char *e = getenv("AEROBULK_GPU_TRACE"); return e && atoi(e) != 0; }();
-    return v;
-}
-bool trace_on();   // + "the calling thread drives session 0" (the trace events live on its device), defined below
-cudaEvent_t tr_t0 = nullptr, tr_in[MAX_CHUNKS] = {}, tr_k[MAX_CHUNKS] = {}, tr_out[MAX_CHUNKS] = {};
-void trace_init()
-{
-    if (tr_t0) return;
-    cudaEventCreate(&tr_t0);
-    for (int i = 0; i < MAX_CHUNKS; ++i) {
-        cudaEventCreate(&tr_in[i]);
-        cudaEventCreate(&tr_k[i]);
-        cudaEventCreate(&tr_out[i]);
-    }
-}
-int chunk_shape()   // 0: sizes decrease linearly (K..1), 1: equal, 2: small first chunk then equal
-{
-    static int v = [] { const char *e = getenv("AEROBULK_GPU_CHUNK_SHAPE"); return e ? atoi(e) : 0; }();
-    return v;
-}
 // Zero-copy host-array calls.  When EVERY array of a call is pinned host memory (cudaHostAlloc / cudaHostRegister: it has a
 // device alias under unified virtual addressing) the flux kernel loads its inputs from and stores its outputs to the
 // caller's arrays directly: each byte crosses PCIe once, both directions busy for the whole launch, no staging, no
 // copy-engine granularity.  Measured 1.54 ms per 1 M-point skin call against 1.75-1.85 ms for the staged pipeline
-// (tools/e2e_probe.py).  AEROBULK_GPU_ZEROCOPY=0 disables it; 1 / 2 select one direction only (experiments: outputs
-// alone 1.77 ms, inputs alone 2.27 ms).  Not used at jt == 1 when AEROBULK_INIT needs the field statistics (the inputs
-// would cross PCIe twice), nor together with the stability sort (a gather / scatter across PCIe: 4.7 ms).
-int zerocopy_mode()
+// (tools/e2e_probe.py); one direction alone measured slower (outputs 1.77 ms, inputs 2.27 ms).  Not used at jt == 1 when
+// AEROBULK_INIT needs the field statistics (the inputs would cross PCIe twice), nor together with the stability sort (a
+// gather / scatter across PCIe: 4.7 ms).  AEROBULK_GPU_ZEROCOPY=0 turns it off, and with it the pinned slab of pageable
+// arrays, which the kernel reads zero-copy too.
+bool zerocopy_on()
 {
-    static int v = [] { const char *e = getenv("AEROBULK_GPU_ZEROCOPY"); return e ? atoi(e) : AEROBULK_GPU_ZEROCOPY_DEFAULT; }();
+    static bool v = [] { const char *e = getenv("AEROBULK_GPU_ZEROCOPY"); return e ? atoi(e) != 0 : true; }();
     return v;
 }
 // device alias of a pinned (page-locked, device-mapped) host pointer, or nullptr
@@ -151,7 +123,7 @@ int host_threads()
 }
 CopyPool &copy_pool()
 {
-    static CopyPool *p = new CopyPool(host_threads(), [] { const char *e = getenv("AEROBULK_GPU_COPY_STREAMING"); return e ? atoi(e) != 0 : AEROBULK_GPU_COPY_STREAMING_DEFAULT != 0; }());   // never destroyed: its threads outlive static destructors
+    static CopyPool *p = new CopyPool(host_threads(), [] { const char *e = getenv("AEROBULK_GPU_COPY_STREAMING"); return e ? atoi(e) != 0 : true; }());   // never destroyed: its threads outlive static destructors
     return *p;
 }
 // CopyPool::run has ONE caller at a time; the device threads of a split call take turns (the copies are bound by the
@@ -174,16 +146,6 @@ long long bounce_chunk_points()
         long long k = e ? atoll(e) : 180224;
         return k < 2048 ? 2048 : k;
     }();
-    return v;
-}
-int bounce_shape()   // 0: equal chunks; 1 (default, measured 2.26-2.34 vs 2.45 ms): small first and last chunks (weights 1,2,3,..,3,2,1): shorter fill and drain
-{
-    static int v = [] { const char *e = getenv("AEROBULK_GPU_BOUNCE_SHAPE"); return e ? atoi(e) : 1; }();
-    return v;
-}
-int bounce_lag()   // chunks the GPU keeps queued before the host turns to copying results home
-{
-    static int v = [] { const char *e = getenv("AEROBULK_GPU_BOUNCE_LAG"); int k = e ? atoi(e) : 2; return k < 1 ? 1 : k; }();
     return v;
 }
 size_t bounce_max_bytes()   // larger slabs are not worth pinning: the driver-staged copies take over
@@ -283,7 +245,6 @@ thread_local Session *cur = &sess[0];
 #define g (*cur)
 int n_devices = 1;
 std::mutex g_mu;
-bool trace_on() { return trace_env() && cur == &sess[0]; }
 
 const char *HUM_NAMES[3] = {"sh", "dp", "rh"};
 
@@ -441,6 +402,28 @@ int alloc_ecmwf_state(long long n)
     }
     g.n_ecmwf = n;
     return 0;
+}
+// kt == nit000 -> *_INIT allocates the warm-layer state (mod_blk_coare3p6.f90:250,68-95; mod_blk_ecmwf.f90:189); the
+// state is shared by aerobulk_model and TURB_*, like the module arrays of the reference
+int init_wl_state(int ialgo, long long n)
+{
+    if (ialgo == abd::ECMWF) {
+        if (g.n_ecmwf) return fail(AEROBULK_GPU_ERR_STATE, " ECMWF_INIT => allocation of dT_wl & Hz_wl failed!");
+        return alloc_ecmwf_state(n);
+    }
+    if (g.n_coare) return fail(AEROBULK_GPU_ERR_STATE, " COARE_INIT => allocation of Tau_ac, Qnt_ac, dT_wl & Hz_wl failed!");
+    return alloc_coare_state(n);
+}
+// points the warm-layer state of a FluxArgs / TurbArgs at the row block that starts at point s0
+template <class Args>
+void bind_wl_state(Args &a, int ialgo, long long s0)
+{
+    if (ialgo == abd::ECMWF) {
+        a.dT_wl = g.e_dT_wl + s0;
+    } else {
+        a.dT_wl = g.c_state[0] + s0; a.Hz_wl = g.c_state[1] + s0;
+        a.Qnt_ac = g.c_state[2] + s0; a.Tau_ac = g.c_state[3] + s0;
+    }
 }
 
 // Moves elements [s0, s0+len) of `nf` fields between host and device staging.  Consecutive fields whose HOST arrays are
@@ -811,10 +794,16 @@ int spec_chunk_limit()
     return v;
 }
 // Row-block chunk plan of a host-array call: cstart[0..nchunks], boundaries on multiples of 2048 points (whole sort
-// windows / thread blocks).  kind 0: one chunk (device arrays, zero-copy on pinned arrays); 1: staged H2D | kernel | D2H
-// pipeline whose kernels wait for the LAST input byte (sizes decrease linearly by default: short exposed tail); 2: pageable
-// arrays through the pinned slab (small first and last chunks by default: short fill and drain); 3: staged pipeline with
-// the speculative AEROBULK_INIT (jt == 1): H2D and D2H overlap, up to 12 equal pieces with half-size first and last ones.
+// windows / thread blocks).
+//   kind 0: one chunk (device arrays, zero-copy on pinned arrays);
+//   kind 1: staged H2D | kernel | D2H pipeline.  It is H2D-bound (PCIe ~50 GB/s per direction measured, vs. >150 GB/s
+//           consumed by the kernel), so its length is H2D(all) + kernel(last chunk) + D2H(last chunk): sizes decrease
+//           linearly (weights K..1) to keep the exposed tail short while the early pieces stay large enough for full
+//           PCIe efficiency.  (Two copy-in streams were measured slower: 2.3 vs 2.0 ms per 1M-point call.)
+//   kind 2: pageable arrays through the pinned slab: small first and last chunks (weights 1,2,3,..,3,2,1) for a short
+//           fill and drain, 2.26-2.34 ms per 1 M-point skin call against 2.45 ms with equal chunks;
+//   kind 3: staged pipeline with the speculative AEROBULK_INIT (jt == 1): H2D and D2H overlap, up to 12 equal pieces
+//           with half-size first and last ones.
 int plan_chunks(long long n, int kind, long long *cstart)
 {
     int nchunks = 1;
@@ -830,9 +819,9 @@ int plan_chunks(long long n, int kind, long long *cstart)
     }
     double w[MAX_CHUNKS], wsum = 0.;
     for (int c = 0; c < nchunks; ++c) {
-        if (kind == 2) w[c] = bounce_shape() == 1 ? (double)((c + 1 < nchunks - c) ? c + 1 : nchunks - c) : 1.;
+        if (kind == 2) w[c] = (double)((c + 1 < nchunks - c) ? c + 1 : nchunks - c);
         else if (kind == 3) w[c] = (c == 0 || c == nchunks - 1) ? 0.5 : 1.;   // both directions busy: equal pieces, short fill and drain
-        else w[c] = chunk_shape() == 0 ? (double)(nchunks - c) : (chunk_shape() == 2 && c == 0 ? 0.5 : 1.);
+        else w[c] = (double)(nchunks - c);
         wsum += w[c];
     }
     double acc = 0.;
@@ -850,24 +839,33 @@ int plan_chunks(long long n, int kind, long long *cstart)
 // ---------------------------------------------------------------------------
 // AEROBULK_MODEL (mod_aerobulk.f90:176-269) + aerobulk_compute dispatch
 // ---------------------------------------------------------------------------
-int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj,
-               const double *sst, const double *t_zt, const double *hum_zt, const double *U_zu,
-               const double *V_zu, const double *slp, double *QL, double *QH, double *Tau_x, double *Tau_y,
-               double *Evap, const int *Niter, const int *l_use_skin, const double *rad_sw,
-               const double *rad_lw, double *T_s)
+// the argument checks that come before any device work (:244), for one device and for a split call alike
+int check_model_args(int jt, const char *calgo, int Ni, int Nj, const double *sst, const double *t_zt, const double *hum_zt,
+                     const double *U_zu, const double *V_zu, const double *slp, const double *QL, const double *QH,
+                     const double *Tau_x, const double *Tau_y, const double *Evap)
 {
     g.errcode = 0;
     g.errmsg[0] = 0;
     if (!calgo || !sst || !t_zt || !hum_zt || !U_zu || !V_zu || !slp || !QL || !QH || !Tau_x || !Tau_y || !Evap)
         return fail(AEROBULK_GPU_ERR_ARG, "aerobulk_gpu_model: NULL mandatory argument");
     if (Ni < 0 || Nj < 0) return fail(AEROBULK_GPU_ERR_ARG, "aerobulk_gpu_model: negative shape %d x %d", Ni, Nj);
+    if (jt < 1) return fail(AEROBULK_GPU_ERR_JT, "AEROBULK_MODEL => jt < 1 !??\n we are in a Fortran world here...");
+    return 0;
+}
 
+int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj,
+               const double *sst, const double *t_zt, const double *hum_zt, const double *U_zu,
+               const double *V_zu, const double *slp, double *QL, double *QH, double *Tau_x, double *Tau_y,
+               double *Evap, const int *Niter, const int *l_use_skin, const double *rad_sw,
+               const double *rad_lw, double *T_s)
+{
+    int rc = check_model_args(jt, calgo, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap);
+    if (rc) return rc;
     if (Niter) g.nb_iter = *Niter;   // :236 sticky
     const bool lskin = l_use_skin ? (*l_use_skin != 0) : false;
     const bool lsrad = (rad_sw != nullptr) && (rad_lw != nullptr);
-    if (jt < 1) return fail(AEROBULK_GPU_ERR_JT, "AEROBULK_MODEL => jt < 1 !??\n we are in a Fortran world here...");
 
-    int rc = ensure_device();
+    rc = ensure_device();
     if (rc) return rc;
     const long long n = (long long)Ni * (long long)Nj;
     cudaStream_t cs = compute_stream();
@@ -885,62 +883,41 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
 
     // rad_lw before rad_sw: a caller slab [sst .. slp, rad_lw] with a per-step rad_sw elsewhere is one run + one array
     const double *in_h[8] = {sst, t_zt, hum_zt, U_zu, V_zu, slp, lsrad ? rad_lw : nullptr, lsrad ? rad_sw : nullptr};
-    const double *in_d[8];
     double *out_h[6] = {QL, QH, Tau_x, Tau_y, Evap, lsrad ? T_s : nullptr};
-    double *out_d[6];
+    const double *in_d[8] = {};   // what the kernels read and write
+    double *out_d[6] = {};
 
-    // jt == 1 with PAGEABLE arrays: the staged pipeline (with its speculative AEROBULK_INIT) runs from / to the library's
-    // pinned slab, and the copy threads feed it chunk by chunk -- chunk c+1 of the 8 inputs goes into the slab while the
-    // GPU receives / computes chunk c, and the results of the chunks whose D2H has landed go home meanwhile.  (Round 1
-    // copied the whole inputs in first and the whole outputs out last: three phases one after the other.)
-    double *user_out[6] = {};
-    const double *user_in[8] = {};
-    bool bounce_first = false;
-    if (!device_ptrs && jt == 1 && !g.preinit_done && bounce_on() && zerocopy_mode() == 3 && n >= BOUNCE_MIN_POINTS) {
-        bool pinned = true;
-        for (int k = 0; k < 8 && pinned; ++k) pinned = !in_h[k] || device_alias(in_h[k]);
-        for (int k = 0; k < 6 && pinned; ++k) pinned = !out_h[k] || device_alias(out_h[k]);
-        if (!pinned && ensure_bounce(n)) {
-            for (int k = 0; k < 8; ++k) user_in[k] = in_h[k];
-            for (int k = 0; k < 8; ++k) in_h[k] = in_h[k] ? g.hb + (long long)k * g.cap_hb : nullptr;
-            for (int k = 0; k < 6; ++k) {
-                user_out[k] = out_h[k];
-                out_h[k] = out_h[k] ? g.hb + (long long)(8 + k) * g.cap_hb : nullptr;
-            }
-            bounce_first = true;
-        }
-    }
-
-    // Chunk plan of the host-array pipeline: contiguous row blocks of the flattened fields.  The pipeline is
-    // H2D-bound (PCIe ~50 GB/s per direction measured, vs. >150 GB/s consumed by the kernel), so its length
-    // is H2D(all) + kernel(last chunk) + D2H(last chunk): chunk sizes DEcrease linearly (weights K..1) to
-    // keep the exposed tail short while the early pieces stay large enough for full PCIe efficiency.
-    // (Two copy-in streams were measured slower: 2.3 vs 2.0 ms per 1M-point call.)
-    // zero-copy legs (host-array calls whose arrays are ALL pinned): see zerocopy_mode()
-    bool zc_in = false, zc_out = false;
-    const double *in_alias[8] = {};
-    double *out_alias[6] = {};
-    if (!device_ptrs && n > 0 && zerocopy_mode() != 0 && !(jt == 1 && !g.preinit_done)) {
-        zc_in = (zerocopy_mode() & 2) != 0;
-        zc_out = (zerocopy_mode() & 1) != 0;
-        for (int k = 0; k < 8 && zc_in; ++k)
-            if (in_h[k] && !(in_alias[k] = device_alias(in_h[k]))) zc_in = false;
-        for (int k = 0; k < 6 && zc_out; ++k)
-            if (out_h[k] && !(out_alias[k] = const_cast<double *>(device_alias(out_h[k])))) zc_out = false;
-        if (zerocopy_mode() == 3 && !(zc_in && zc_out)) zc_in = zc_out = false;   // all arrays pinned, or the staged pipeline
-    }
-    // pageable caller arrays: bounce through the library's pinned slab on the copy threads (see CopyPool)
-    const bool bounce = !device_ptrs && !zc_in && !zc_out && bounce_on() && zerocopy_mode() == 3 && n >= BOUNCE_MIN_POINTS &&
-                        !(jt == 1 && !g.preinit_done) && ensure_bounce(n);
-    if (bounce) {
-        for (int k = 0; k < 8; ++k) in_alias[k] = in_h[k] ? g.hb_dev + (long long)k * g.cap_hb : nullptr;
-        for (int k = 0; k < 6; ++k) out_alias[k] = out_h[k] ? g.hb_dev + (long long)(8 + k) * g.cap_hb : nullptr;
-        zc_in = zc_out = true;
+    // How the arrays reach the kernel, chosen once per call, in this order:
+    //   DEVICE  device pointers (aerobulk_gpu_model_device): one launch on them;
+    //   ALIAS   jt > 1 or AEROBULK_INIT already done, every array pinned: one launch on their device aliases, no sort;
+    //   BOUNCE  jt > 1, pageable arrays of BOUNCE_MIN_POINTS or more, and the pinned slab fits: the copy threads move kind-2
+    //           chunks between the caller's arrays and the slab, the kernel works on the slab zero-copy, no sort, and the
+    //           outputs go home two chunks behind the GPU;
+    //   STAGED  anything else: H2D | kernel | D2H through the device staging arrays, kind-1 chunks.
+    // At jt == 1 with AEROBULK_INIT still to run the path is STAGED whatever the arrays, with kind-3 chunks; `spec_init`:
+    // there are two or more of them and AEROBULK_INIT runs speculatively chunk by chunk (below), otherwise the statistics
+    // are taken once all inputs are in.  `slab_first`: the arrays are pageable, BOUNCE_MIN_POINTS or more, and the pinned
+    // slab fits, so the pipeline copies from / to the slab and the copy threads feed it -- chunk by chunk under
+    // spec_init, otherwise whole.
+    enum Path { DEVICE, ALIAS, BOUNCE, STAGED } path = device_ptrs ? DEVICE : STAGED;
+    const bool init_stats = jt == 1 && !g.preinit_done;   // this call takes AEROBULK_INIT's field statistics
+    const bool slab_ok = bounce_on() && zerocopy_on() && n >= BOUNCE_MIN_POINTS;   // the kernel reads the slab zero-copy
+    auto alias_all = [&] {   // device aliases of every array into in_d / out_d; false at the first array without one
+        for (int k = 0; k < 8; ++k)
+            if (in_h[k] && !(in_d[k] = device_alias(in_h[k]))) return false;
+        for (int k = 0; k < 6; ++k)
+            if (out_h[k] && !(out_d[k] = const_cast<double *>(device_alias(out_h[k])))) return false;
+        return true;
+    };
+    bool slab_first = false;
+    if (!device_ptrs && init_stats) {
+        slab_first = slab_ok && !alias_all() && ensure_bounce(n);
+    } else if (!device_ptrs) {
+        if (n > 0 && zerocopy_on() && alias_all()) path = ALIAS;
+        else if (slab_ok && ensure_bounce(n)) path = BOUNCE;
     }
     long long cstart[MAX_CHUNKS + 1];
-    static const bool spec_env = [] { const char *e = getenv("AEROBULK_GPU_SPEC_INIT"); return e ? atoi(e) != 0 : true; }();
-    const bool want_spec = spec_env && jt == 1 && !g.preinit_done && !device_ptrs && !zc_in && !bounce;
-    const int nchunks = plan_chunks(n, bounce ? 2 : ((!device_ptrs && !zc_in) ? (want_spec ? 3 : 1) : 0), cstart);
+    const int nchunks = plan_chunks(n, path == BOUNCE ? 2 : path == STAGED ? (init_stats ? 3 : 1) : 0, cstart);
     // Speculative AEROBULK_INIT (jt == 1 of a staged host-array call with >= 2 chunks).  The reference judges the WHOLE
     // fields before it computes anything, which would hold the first flux launch -- and every byte of D2H -- back until the
     // last input byte has arrived: H2D and D2H one after the other.  Instead each chunk's statistics are taken as it lands,
@@ -949,42 +926,51 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     // reference's; the few chunks (normally none) whose running verdict differed from it are recomputed from the staged
     // inputs, and an AEROBULK_INIT error is raised exactly as before -- the arrays the reference would never have
     // written are then undefined.  Same results, H2D and D2H overlapped: C5 end to end 0.54 -> ~1 Gpt/s.
-    const bool spec_init = want_spec && nchunks >= 2;
+    const bool spec_init = path == STAGED && init_stats && nchunks >= 2;
 
-    if (device_ptrs) {
-        for (int k = 0; k < 8; ++k) in_d[k] = in_h[k];
-        for (int k = 0; k < 6; ++k) out_d[k] = out_h[k];
-    } else {
-        if (!(zc_in && zc_out)) {
-            rc = ensure_staging(n);
-            if (rc) return rc;
+    // through the slab: the caller's arrays move to user_in / user_out, in_h / out_h name the slab rows
+    double *user_in[8] = {}, *user_out[6] = {};
+    if (slab_first || path == BOUNCE) {
+        for (int k = 0; k < 8; ++k) {
+            user_in[k] = const_cast<double *>(in_h[k]);
+            in_h[k] = in_h[k] ? g.hb + (long long)k * g.cap_hb : nullptr;
         }
-        for (int k = 0; k < 8; ++k) in_d[k] = in_h[k] ? (zc_in ? in_alias[k] : g.d_in[k]) : nullptr;
-        for (int k = 0; k < 6; ++k) out_d[k] = out_h[k] ? (zc_out ? out_alias[k] : g.d_out[k]) : nullptr;
-        if (trace_on()) {
-            trace_init();
-            cudaEventRecord(tr_t0, g.in_stream);
+        for (int k = 0; k < 6; ++k) {
+            user_out[k] = out_h[k];
+            out_h[k] = out_h[k] ? g.hb + (long long)(8 + k) * g.cap_hb : nullptr;
         }
     }
-    // pageable arrays at jt == 1: chunk-wise through the slab if the pipeline is chunk-wise (speculative init), else whole
-    const bool pipe_bounce = bounce_first && spec_init;
-    if (bounce_first && !pipe_bounce) bounce_copy(8, const_cast<double *const *>(user_in), 0, 0, n, true);
+    if (path == STAGED) {
+        rc = ensure_staging(n);
+        if (rc) return rc;
+    }
+    for (int k = 0; k < 8; ++k) {
+        if (!in_h[k] || path == DEVICE) in_d[k] = in_h[k];
+        else if (path == BOUNCE) in_d[k] = g.hb_dev + (long long)k * g.cap_hb;
+        else if (path == STAGED) in_d[k] = g.d_in[k];
+    }
+    for (int k = 0; k < 6; ++k) {
+        if (!out_h[k] || path == DEVICE) out_d[k] = out_h[k];
+        else if (path == BOUNCE) out_d[k] = g.hb_dev + (long long)(8 + k) * g.cap_hb;
+        else if (path == STAGED) out_d[k] = g.d_out[k];
+    }
+
+    if (slab_first && !spec_init) bounce_copy(8, user_in, 0, 0, n, true);
     // H2D of chunk c on the copy-in stream (preceded by its way into the slab on the copy threads where that applies)
     auto enqueue_h2d = [&](int c) -> int {
         const long long s0 = cstart[c], len = cstart[c + 1] - s0;
-        if (len > 0 && !zc_in) {
-            if (pipe_bounce) bounce_copy(8, const_cast<double *const *>(user_in), 0, s0, len, true);
+        if (len > 0 && path == STAGED) {
+            if (slab_first && spec_init) bounce_copy(8, user_in, 0, s0, len, true);
             const int r = copy_fields(8, g.d_in, const_cast<double *const *>(in_h), g.cap, s0, len, true, g.in_stream);
             if (r) return r;
         }
         CUDA_TRY(cudaEventRecord(g.ev_in[c], g.in_stream));
-        if (trace_on()) cudaEventRecord(tr_in[c], g.in_stream);
         return 0;
     };
     int h2d_next = 0;   // first chunk whose H2D is not enqueued yet
     if (!device_ptrs) {
         // all of them up front, except where the copy threads feed the slab: there chunk c + 1 follows the launch of chunk c
-        for (; h2d_next < (pipe_bounce ? 1 : nchunks); ++h2d_next) {
+        for (; h2d_next < (slab_first && spec_init ? 1 : nchunks); ++h2d_next) {
             rc = enqueue_h2d(h2d_next);
             if (rc) return rc;
         }
@@ -1037,18 +1023,9 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
         return fail(AEROBULK_GPU_ERR_SKIN_NORAD,
                     "skin schemes are active (l_use_skin_schemes is sticky, mod_aerobulk.f90:74) but rad_sw/rad_lw are absent");
 
-    // kt == nit000 -> *_INIT allocates the warm-layer state (mod_blk_coare3p6.f90:250,68-95; mod_blk_ecmwf.f90:189)
     if (use_skin && jt == 1) {
-        if (ialgo == abd::ECMWF) {
-            if (g.n_ecmwf) return fail(AEROBULK_GPU_ERR_STATE, " ECMWF_INIT => allocation of dT_wl & Hz_wl failed!");
-            rc = alloc_ecmwf_state(n);
-            if (rc) return rc;
-        } else {
-            if (g.n_coare)
-                return fail(AEROBULK_GPU_ERR_STATE, " COARE_INIT => allocation of Tau_ac, Qnt_ac, dT_wl & Hz_wl failed!");
-            rc = alloc_coare_state(n);
-            if (rc) return rc;
-        }
+        rc = init_wl_state(ialgo, n);
+        if (rc) return rc;
     }
     if (use_skin) {
         const long long have = (ialgo == abd::ECMWF) ? g.n_ecmwf : g.n_coare;
@@ -1062,7 +1039,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     // the doubtful points to themselves, ECMWF + skin gains the most (5.01 -> 4.54 ms by day, 4.46 -> 3.88 ms by night;
     // with the round-1 proxy it lost 1 %).
     // (never with zero-copy inputs: the gather through the permutation would cross PCIe at sector granularity)
-    const bool do_sort = !zc_in && !zc_out && (g.sort_points == 2 || (g.sort_points == 1 && ialgo != abd::NCAR));
+    const bool do_sort = (path == DEVICE || path == STAGED) && (g.sort_points == 2 || (g.sort_points == 1 && ialgo != abd::NCAR));
     if (do_sort) {
         // every chunk is padded to whole sort windows
         const long long need = n + (long long)(nchunks + 1) * abk::sort_window();
@@ -1084,44 +1061,20 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     a.bad_index = g.d_bad;
     const bool zteq = fabs(zu - zt) < 0.01;
 
-    int launched[MAX_CHUNKS], n_launched = 0, n_home = 0;
-    bool home[MAX_CHUNKS] = {};   // pageable jt == 1: chunk already copied back to the caller's arrays
-    for (int c = 0; c < nchunks; ++c) {
-        const long long s0 = cstart[c], len = cstart[c + 1] - s0;
-        if (len <= 0) continue;
+    // the kernels of chunk c on the compute stream: classify (when sorting) and flux, on the chunk's row block of every
+    // array and of the warm-layer state; `timed`: the flux launch between a pair of aerobulk_gpu_set_kernel_timing events
+    auto launch_chunk = [&](int c, bool timed) -> int {
+        const long long s0 = cstart[c];
         a.sst = in_d[0] + s0; a.t_zt = in_d[1] + s0; a.hum_zt = in_d[2] + s0;
         a.U_zu = in_d[3] + s0; a.V_zu = in_d[4] + s0; a.slp = in_d[5] + s0;
         a.rad_lw = in_d[6] ? in_d[6] + s0 : nullptr;
         a.rad_sw = in_d[7] ? in_d[7] + s0 : nullptr;
-        a.lon = nullptr;
         a.QL = out_d[0] + s0; a.QH = out_d[1] + s0; a.Tau_x = out_d[2] + s0; a.Tau_y = out_d[3] + s0;
         a.Evap = out_d[4] + s0;
         a.T_s = out_d[5] ? out_d[5] + s0 : nullptr;
-        if (use_skin) {
-            if (ialgo == abd::ECMWF) {
-                a.dT_wl = g.e_dT_wl + s0;
-            } else {
-                a.dT_wl = g.c_state[0] + s0; a.Hz_wl = g.c_state[1] + s0;
-                a.Qnt_ac = g.c_state[2] + s0; a.Tau_ac = g.c_state[3] + s0;
-            }
-        }
-        a.n = len;
+        if (use_skin) bind_wl_state(a, ialgo, s0);
+        a.n = cstart[c + 1] - s0;
         a.index_offset = s0;
-        if (bounce) bounce_copy(8, const_cast<double *const *>(in_h), 0, s0, len, true);
-        while (pipe_bounce && h2d_next <= c) {   // (normally enqueued one iteration ahead, below)
-            rc = enqueue_h2d(h2d_next++);
-            if (rc) return rc;
-        }
-        if (!device_ptrs) CUDA_TRY(cudaStreamWaitEvent(cs, g.ev_in[c], 0));
-        if (spec_init) {
-            rc = launch_local_stats(len, a.sst, a.t_zt, a.hum_zt, a.U_zu, a.V_zu, a.slp, lsrad ? a.rad_lw : nullptr, cs,
-                                    g.d_cstats + (long long)c * abk::NSTATS);
-            if (rc) return rc;
-            CUDA_TRY(abk::launch_init_decide(g.d_cstats, c + 1, lsrad ? 1 : 0, g.d_cgstats + (long long)c * abk::NSTATS,
-                                             g.d_cinit + 2 * c, cs));
-            g.launches += 1;
-            a.init_dev = g.d_cinit + 2 * c;
-        }
         a.perm = nullptr;
         if (do_sort) {
             unsigned short *perm = g.d_perm + s0 + (long long)c * abk::sort_window();
@@ -1130,7 +1083,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
             a.perm = perm;
         }
         cudaEvent_t kt0 = nullptr, kt1 = nullptr;
-        if (g.time_kernels) {
+        if (timed && g.time_kernels) {
             if (g.kt_used + 2 > g.kt_ev.size()) {
                 cudaEvent_t e0, e1;
                 CUDA_TRY(cudaEventCreate(&e0));
@@ -1146,37 +1099,62 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
         CUDA_TRY(abk::launch_flux(ialgo, use_skin, zteq, a, cs));
         g.launches += 1;
         if (kt1) CUDA_TRY(cudaEventRecord(kt1, cs));
-        if (!device_ptrs) {
-            CUDA_TRY(cudaEventRecord(g.ev_k[c], cs));
-            if (trace_on()) cudaEventRecord(tr_k[c], cs);
-            CUDA_TRY(cudaStreamWaitEvent(g.out_stream, g.ev_k[c], 0));
-            if (!zc_out) {
-                rc = copy_fields(6, g.d_out, out_h, g.cap, s0, len, false, g.out_stream);
+        return 0;
+    };
+    // D2H of chunk c on the copy-out stream once its kernel is done (the zero-copy kernels have written the host already)
+    auto enqueue_d2h = [&](int c) -> int {
+        CUDA_TRY(cudaEventRecord(g.ev_k[c], cs));
+        CUDA_TRY(cudaStreamWaitEvent(g.out_stream, g.ev_k[c], 0));
+        if (path != STAGED) return 0;
+        return copy_fields(6, g.d_out, out_h, g.cap, cstart[c], cstart[c + 1] - cstart[c], false, g.out_stream);
+    };
+
+    int launched[MAX_CHUNKS], n_launched = 0, n_home = 0;
+    bool home[MAX_CHUNKS] = {};   // pageable jt == 1: chunk already copied back to the caller's arrays
+    for (int c = 0; c < nchunks; ++c) {
+        const long long s0 = cstart[c], len = cstart[c + 1] - s0;
+        if (len <= 0) continue;
+        if (path == BOUNCE) bounce_copy(8, user_in, 0, s0, len, true);
+        while (slab_first && spec_init && h2d_next <= c) {   // (normally enqueued one iteration ahead, below)
+            rc = enqueue_h2d(h2d_next++);
+            if (rc) return rc;
+        }
+        if (!device_ptrs) CUDA_TRY(cudaStreamWaitEvent(cs, g.ev_in[c], 0));
+        if (spec_init) {
+            rc = launch_local_stats(len, in_d[0] + s0, in_d[1] + s0, in_d[2] + s0, in_d[3] + s0, in_d[4] + s0, in_d[5] + s0,
+                                    lsrad ? in_d[6] + s0 : nullptr, cs, g.d_cstats + (long long)c * abk::NSTATS);
+            if (rc) return rc;
+            CUDA_TRY(abk::launch_init_decide(g.d_cstats, c + 1, lsrad ? 1 : 0, g.d_cgstats + (long long)c * abk::NSTATS,
+                                             g.d_cinit + 2 * c, cs));
+            g.launches += 1;
+            a.init_dev = g.d_cinit + 2 * c;
+        }
+        rc = launch_chunk(c, true);
+        if (rc) return rc;
+        if (device_ptrs) continue;
+        rc = enqueue_d2h(c);
+        if (rc) return rc;
+        if (slab_first && spec_init) {
+            CUDA_TRY(cudaEventRecord(g.ev_out[c], g.out_stream));
+            launched[n_launched++] = c;
+            // the next chunk goes into the slab (and on to the device) while the GPU works on this one ...
+            while (h2d_next < nchunks && h2d_next <= c + 1) {
+                rc = enqueue_h2d(h2d_next++);
                 if (rc) return rc;
             }
-            if (trace_on()) cudaEventRecord(tr_out[c], g.out_stream);
-            if (pipe_bounce) {
-                CUDA_TRY(cudaEventRecord(g.ev_out[c], g.out_stream));
-                launched[n_launched++] = c;
-                // the next chunk goes into the slab (and on to the device) while the GPU works on this one ...
-                while (h2d_next < nchunks && h2d_next <= c + 1) {
-                    rc = enqueue_h2d(h2d_next++);
-                    if (rc) return rc;
-                }
-                // ... and the chunks whose results have landed in the slab go home
-                while (n_home < n_launched && cudaEventQuery(g.ev_out[launched[n_home]]) == cudaSuccess) {
-                    const int h = launched[n_home++];
-                    bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], false);
-                    home[h] = true;
-                }
+            // ... and the chunks whose results have landed in the slab go home
+            while (n_home < n_launched && cudaEventQuery(g.ev_out[launched[n_home]]) == cudaSuccess) {
+                const int h = launched[n_home++];
+                bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], false);
+                home[h] = true;
             }
-            if (bounce) {   // results of an earlier chunk go home while the GPU has bounce_lag() chunks queued
-                launched[n_launched++] = c;
-                if (n_launched - n_home > bounce_lag()) {
-                    const int h = launched[n_home++];
-                    CUDA_TRY(cudaEventSynchronize(g.ev_k[h]));
-                    bounce_copy(6, out_h, 8, cstart[h], cstart[h + 1] - cstart[h], false);
-                }
+        }
+        if (path == BOUNCE) {   // results of an earlier chunk go home while the GPU has two chunks queued
+            launched[n_launched++] = c;
+            if (n_launched - n_home > 2) {
+                const int h = launched[n_home++];
+                CUDA_TRY(cudaEventSynchronize(g.ev_k[h]));
+                bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], false);
             }
         }
     }
@@ -1201,47 +1179,17 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
         a.init_dev = nullptr;
         a.ihum = g.ihum;
         for (int c = 0; c < nchunks; ++c) {
-            const long long s0 = cstart[c], len = cstart[c + 1] - s0;
-            if (len <= 0 || (cinit[2 * c] == g.ihum && cinit[2 * c + 1] == 0)) continue;
-            a.sst = in_d[0] + s0; a.t_zt = in_d[1] + s0; a.hum_zt = in_d[2] + s0;
-            a.U_zu = in_d[3] + s0; a.V_zu = in_d[4] + s0; a.slp = in_d[5] + s0;
-            a.rad_lw = in_d[6] ? in_d[6] + s0 : nullptr;
-            a.rad_sw = in_d[7] ? in_d[7] + s0 : nullptr;
-            a.QL = out_d[0] + s0; a.QH = out_d[1] + s0; a.Tau_x = out_d[2] + s0; a.Tau_y = out_d[3] + s0;
-            a.Evap = out_d[4] + s0;
-            a.T_s = out_d[5] ? out_d[5] + s0 : nullptr;
-            if (use_skin) {
-                if (ialgo == abd::ECMWF) {
-                    a.dT_wl = g.e_dT_wl + s0;
-                } else {
-                    a.dT_wl = g.c_state[0] + s0; a.Hz_wl = g.c_state[1] + s0;
-                    a.Qnt_ac = g.c_state[2] + s0; a.Tau_ac = g.c_state[3] + s0;
-                }
-            }
-            a.n = len;
-            a.index_offset = s0;
-            a.perm = nullptr;
-            if (do_sort) {
-                unsigned short *perm = g.d_perm + s0 + (long long)c * abk::sort_window();
-                CUDA_TRY(abk::launch_classify(a, perm, use_skin, cs));
-                g.launches += 1;
-                a.perm = perm;
-            }
-            CUDA_TRY(abk::launch_flux(ialgo, use_skin, zteq, a, cs));
-            g.launches += 1;
-            CUDA_TRY(cudaEventRecord(g.ev_k[c], cs));
-            CUDA_TRY(cudaStreamWaitEvent(g.out_stream, g.ev_k[c], 0));
-            if (!zc_out) {
-                rc = copy_fields(6, g.d_out, out_h, g.cap, s0, len, false, g.out_stream);
-                if (rc) return rc;
-            }
+            if (cstart[c + 1] <= cstart[c] || (cinit[2 * c] == g.ihum && cinit[2 * c + 1] == 0)) continue;
+            rc = launch_chunk(c, false);
+            if (!rc) rc = enqueue_d2h(c);
+            if (rc) return rc;
             home[c] = false;   // recomputed: what went home earlier is stale
         }
     }
-    while (bounce && n_home < n_launched) {
+    while (path == BOUNCE && n_home < n_launched) {
         const int h = launched[n_home++];
         CUDA_TRY(cudaEventSynchronize(g.ev_k[h]));
-        bounce_copy(6, out_h, 8, cstart[h], cstart[h + 1] - cstart[h], false);
+        bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], false);
     }
     CUDA_TRY(cudaMemcpyAsync(g.h_bad, g.d_bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, cs));
     CUDA_TRY(cudaEventRecord(g.ev_bad, cs));
@@ -1256,24 +1204,14 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     if (!never_sync && (!device_ptrs || last || (jt == 1 && !g.init_pending))) {
         CUDA_TRY(cudaStreamSynchronize(cs));
         if (!device_ptrs) CUDA_TRY(cudaStreamSynchronize(g.out_stream));
-        if (bounce_first) {   // what is not home yet (everything, without the chunk-wise feed)
+        if (slab_first) {   // what is not home yet (everything, without the chunk-wise feed)
             for (int c = 0; c < nchunks; ++c) {
                 const long long s0 = cstart[c], len = cstart[c + 1] - s0;
-                if (len > 0 && !(pipe_bounce && home[c])) bounce_copy(6, user_out, 8, s0, len, false);
+                if (len > 0 && !home[c]) bounce_copy(6, user_out, 8, s0, len, false);
             }
         }
         rc = resolve_init();   // an asynchronous AEROBULK_INIT of this session reports first, as in the reference
         if (!rc) rc = check_bad_flag(device_ptrs ? nullptr : Tau_x, device_ptrs ? nullptr : Tau_y);
-        if (!device_ptrs && trace_on()) {
-            fprintf(stderr, "[aerobulk_gpu trace] jt=%d chunks=%d  (ms since the first H2D: in | kernel | out)\n", jt, nchunks);
-            for (int c = 0; c < nchunks; ++c) {
-                float a = 0.f, b = 0.f, d = 0.f;
-                cudaEventElapsedTime(&a, tr_t0, tr_in[c]);
-                cudaEventElapsedTime(&b, tr_t0, tr_k[c]);
-                cudaEventElapsedTime(&d, tr_t0, tr_out[c]);
-                fprintf(stderr, "   chunk %d  %7lld pts  %6.3f | %6.3f | %6.3f\n", c, cstart[c + 1] - cstart[c], a, b, d);
-            }
-        }
     }
 
     // kt == nitend -> *_EXIT frees the state (mod_blk_coare3p6.f90:411); jt == Nt -> AEROBULK_BYE (:267)
@@ -1384,13 +1322,9 @@ int model_multi(int jt, int Nt, const char *calgo, double zt, double zu, int Ni,
                 const int *l_use_skin, const double *rad_sw, const double *rad_lw, double *T_s)
 {
     Session &s0 = sess[0];
-    s0.errcode = 0;
-    s0.errmsg[0] = 0;
-    if (!calgo || !sst || !t_zt || !hum_zt || !U_zu || !V_zu || !slp || !QL || !QH || !Tau_x || !Tau_y || !Evap)
-        return fail(AEROBULK_GPU_ERR_ARG, "aerobulk_gpu_model: NULL mandatory argument");
-    if (Ni < 0 || Nj < 0) return fail(AEROBULK_GPU_ERR_ARG, "aerobulk_gpu_model: negative shape %d x %d", Ni, Nj);
-    if (jt < 1) return fail(AEROBULK_GPU_ERR_JT, "AEROBULK_MODEL => jt < 1 !??\n we are in a Fortran world here...");
-    int rc = ensure_device();   // session 0: resolves its device id
+    int rc = check_model_args(jt, calgo, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap);
+    if (rc) return rc;
+    rc = ensure_device();   // session 0: resolves its device id
     if (rc) return rc;
     int count = 0;
     CUDA_TRY(cudaGetDeviceCount(&count));
@@ -1506,7 +1440,7 @@ int ensure_turb_slab(long long need)
 // entry point registers each array with its length and role and asks for device-only scratch; open() stores a device
 // pointer in every registered slot, close() brings the outputs home.  open() picks the first mode that applies:
 //   DEVICE  the caller passed device pointers: they pass through, nothing moves, close() does nothing;
-//   ALIAS   every array is pinned (cudaHostAlloc / cudaHostRegister) and zerocopy_mode() == 3: the kernel works on the
+//   ALIAS   every array is pinned (cudaHostAlloc / cudaHostRegister) and zerocopy_on(): the kernel works on the
 //           caller's memory through its device aliases;
 //   BOUNCE  from BOUNCE_MIN_POINTS elements up, the copy threads pack the inputs into the pinned slab g.hx, the kernel
 //           works on the slab zero-copy and the copy threads bring the outputs home (pageable cudaMemcpy is staged by
@@ -1536,7 +1470,7 @@ struct HostTransport {
 
     Mode pick(long long total, long long longest)
     {
-        if (zerocopy_mode() != 3) return STAGED;
+        if (!zerocopy_on()) return STAGED;
         bool pinned = true;
         for (Array &a : arrays)
             if (a.host && !(a.dev = const_cast<double *>(device_alias(a.host)))) {
@@ -1634,15 +1568,8 @@ int turb_impl(const char *calgo, int kt, double zt, double zu, int Ni, int Nj, d
     const long long n = (long long)Ni * Nj;
     cudaStream_t cs_ = compute_stream();
 
-    // kt == nit000 -> *_INIT ; state shared with the aerobulk_model path, like the module arrays of the reference
     if (wl && kt == 1) {
-        if (ialgo == abd::ECMWF) {
-            if (g.n_ecmwf) return fail(AEROBULK_GPU_ERR_STATE, " ECMWF_INIT => allocation of dT_wl & Hz_wl failed!");
-            rc = alloc_ecmwf_state(n);
-        } else {
-            if (g.n_coare) return fail(AEROBULK_GPU_ERR_STATE, " COARE_INIT => allocation of Tau_ac, Qnt_ac, dT_wl & Hz_wl failed!");
-            rc = alloc_coare_state(n);
-        }
+        rc = init_wl_state(ialgo, n);
         if (rc) return rc;
     }
     if (wl) {
@@ -1670,13 +1597,7 @@ int turb_impl(const char *calgo, int kt, double zt, double zu, int Ni, int Nj, d
     for (int k = 0; k < 10; ++k) t.out(&a.opt[k], optp[k], n);
     rc = t.open(on_device);
     if (rc) return rc;
-    if (wl) {
-        if (ialgo == abd::ECMWF) {
-            a.dT_wl = g.e_dT_wl;
-        } else {
-            a.dT_wl = g.c_state[0]; a.Hz_wl = g.c_state[1]; a.Qnt_ac = g.c_state[2]; a.Tau_ac = g.c_state[3];
-        }
-    }
+    if (wl) bind_wl_state(a, ialgo, 0);
     CUDA_TRY(abk::launch_turb(ialgo, cs, wl, fabs(zu - zt) < 0.01, a, cs_));
     g.launches += 1;
     rc = t.close();

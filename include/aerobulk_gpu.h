@@ -29,8 +29,8 @@
  * (cudaHostAlloc / cudaHostRegister) the kernels read and write the caller's memory directly over PCIe ("zero-copy":
  * same results, ~20 % faster end to end, no staging memory).
  * Environment: AEROBULK_GPU_DEVICE (or LOCAL_RANK) device ordinal; AEROBULK_GPU_ZEROCOPY=0 staged copies even for pinned
- * arrays; AEROBULK_GPU_MAX_CHUNKS / AEROBULK_GPU_MIN_CHUNK_POINTS / AEROBULK_GPU_CHUNK_SHAPE pipeline tuning;
- * AEROBULK_GPU_TRACE=1 GPU timeline of every staged call on stderr; pageable arrays: AEROBULK_GPU_BOUNCE=0 driver-staged
+ * arrays (and no pinned slab for pageable ones); AEROBULK_GPU_MAX_CHUNKS / AEROBULK_GPU_MIN_CHUNK_POINTS pipeline
+ * tuning; pageable arrays: AEROBULK_GPU_BOUNCE=0 driver-staged
  * copies, AEROBULK_GPU_HOST_THREADS copy threads (default: 3/4 of the CPUs the process may run on, at most 12),
  * AEROBULK_GPU_BOUNCE_CHUNK_POINTS, AEROBULK_GPU_COPY_STREAMING=0 plain instead of non-temporal stores,
  * AEROBULK_GPU_BOUNCE_MAX_MB largest pinned slab the library may allocate for them (default 12288; beyond it, or when the
