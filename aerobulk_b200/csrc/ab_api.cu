@@ -552,6 +552,12 @@ int algo_id(const char *calgo)
     return 0;
 }
 
+// COARE 3.0, COARE 3.6 and ECMWF have cool-skin / warm-layer schemes; NCAR and ANDREAS have none
+bool has_skin_schemes(int ialgo) { return ialgo == abd::COARE3P0 || ialgo == abd::COARE3P6 || ialgo == abd::ECMWF; }
+
+// l_zt_equal_zu of the TURB_* routines: the ZTEQ kernels when the two heights are less than 1 cm apart
+bool zt_eq_zu(double zt, double zu) { return fabs(zu - zt) < 0.01; }
+
 // ---------------------------------------------------------------------------
 // AEROBULK_INIT from field statistics (mod_aerobulk.f90:24-160)
 // ---------------------------------------------------------------------------
@@ -1017,8 +1023,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     const int ialgo = algo_id(calgo);
     if (!ialgo)
         return fail(AEROBULK_GPU_ERR_ALGO, "ERROR: mod_aerobulk_compute.f90 => bulk algorithm %s is unknown!!!", calgo);
-    const bool skin_algo = (ialgo == abd::COARE3P0 || ialgo == abd::COARE3P6 || ialgo == abd::ECMWF);
-    const bool use_skin = g.l_use_skin_schemes && skin_algo;
+    const bool use_skin = g.l_use_skin_schemes && has_skin_schemes(ialgo);
     if (use_skin && !lsrad)
         return fail(AEROBULK_GPU_ERR_SKIN_NORAD,
                     "skin schemes are active (l_use_skin_schemes is sticky, mod_aerobulk.f90:74) but rad_sw/rad_lw are absent");
@@ -1059,7 +1064,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     a.init_dev = g.init_pending ? g.d_init : nullptr;
     a.first_step = (jt == 1);
     a.bad_index = g.d_bad;
-    const bool zteq = fabs(zu - zt) < 0.01;
+    const bool zteq = zt_eq_zu(zt, zu);
 
     // the kernels of chunk c on the compute stream: classify (when sorting) and flux, on the chunk's row block of every
     // array and of the warm-layer state; `timed`: the flux launch between a pair of aerobulk_gpu_set_kernel_timing events
@@ -1551,8 +1556,7 @@ int turb_impl(const char *calgo, int kt, double zt, double zu, int Ni, int Nj, d
         return fail(AEROBULK_GPU_ERR_ARG, "aerobulk_gpu_turb: NULL mandatory argument");
     const int ialgo = algo_id(calgo);
     if (!ialgo) return fail(AEROBULK_GPU_ERR_ALGO, "aerobulk_gpu_turb: bulk algorithm %s is unknown!!!", calgo);
-    const bool skin_algo = (ialgo == abd::COARE3P0 || ialgo == abd::COARE3P6 || ialgo == abd::ECMWF);
-    if (!skin_algo && (l_use_cs || l_use_wl))
+    if (!has_skin_schemes(ialgo) && (l_use_cs || l_use_wl))
         return fail(AEROBULK_GPU_ERR_SKIN_ALGO, "aerobulk_gpu_turb: TURB_%s has no cool-skin / warm-layer option", calgo);
     const bool cs = l_use_cs != 0, wl = l_use_wl != 0;
     // mod_blk_coare3p6.f90:263-269, mod_blk_ecmwf.f90:202-206
@@ -1598,7 +1602,7 @@ int turb_impl(const char *calgo, int kt, double zt, double zu, int Ni, int Nj, d
     rc = t.open(on_device);
     if (rc) return rc;
     if (wl) bind_wl_state(a, ialgo, 0);
-    CUDA_TRY(abk::launch_turb(ialgo, cs, wl, fabs(zu - zt) < 0.01, a, cs_));
+    CUDA_TRY(abk::launch_turb(ialgo, cs, wl, zt_eq_zu(zt, zu), a, cs_));
     g.launches += 1;
     rc = t.close();
     if (rc) return rc;
@@ -1627,7 +1631,7 @@ int series_impl(const char *calgo, int Nt, long long S, double zt, double zu, co
         return fail(AEROBULK_GPU_ERR_ARG, "aerobulk_gpu_series: bad Nt=%d, S=%lld or hum_kind=%d", Nt, S, hum_kind);
     const int ialgo = algo_id(calgo);
     if (!ialgo) return fail(AEROBULK_GPU_ERR_ALGO, "aerobulk_gpu_series: bulk algorithm %s is unknown!!!", calgo);
-    const bool skin = l_use_skin && (ialgo == abd::COARE3P0 || ialgo == abd::COARE3P6 || ialgo == abd::ECMWF);
+    const bool skin = l_use_skin && has_skin_schemes(ialgo);
     int rc = ensure_device();
     if (rc) return rc;
     const long long n = (long long)Nt * S;
@@ -1660,7 +1664,7 @@ int series_impl(const char *calgo, int Nt, long long S, double zt, double zu, co
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(d_isd, isd, sizeof(int) * (size_t)Nt, cudaMemcpyHostToDevice, cs_));
     a.isd = reinterpret_cast<const int *>(d_isd);
-    CUDA_TRY(abk::launch_series(ialgo, skin, fabs(zu - zt) < 0.01, a, cs_));
+    CUDA_TRY(abk::launch_series(ialgo, skin, zt_eq_zu(zt, zu), a, cs_));
     g.launches += 1;
     CUDA_TRY(cudaMemcpyAsync(g.h_bad, g.d_bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, cs_));
     rc = t.close();
@@ -1937,7 +1941,7 @@ int turb_ice_impl(const char *calgo, double zt, double zu, int Ni, int Nj, const
     a.form_index = g.ice_form_per_point ? -1 : n - 1;
     a.u = make_ice_uniform(zt, zu, cxn);
     a.bad_rough = g.d_bad + 1;
-    CUDA_TRY(abk::launch_ice_turb(ialgo, fabs(zu - zt) < 0.01, a, cs_));
+    CUDA_TRY(abk::launch_ice_turb(ialgo, zt_eq_zu(zt, zu), a, cs_));
     g.launches += 1;
     rc = t.close();
     if (rc) return rc;
@@ -1992,7 +1996,7 @@ int oce_ice_impl(const char *calgo_ice, const char *calgo_oce, double zt, double
     a.uo = make_uniform(zt, zu);
     a.bad_tau = g.d_bad;
     a.bad_rough = g.d_bad + 1;
-    const bool zteq = fabs(zu - zt) < 0.01;
+    const bool zteq = zt_eq_zu(zt, zu);
     CUDA_TRY(abk::launch_ice_flux(ialgo, zteq, a, cs_));
     g.launches += 1;
     if (oalgo) {
@@ -2042,7 +2046,7 @@ int series_ice_impl(const char *calgo, double zt, double zu, long long n, const 
     a.ui = make_ice_uniform(zt, zu, nullptr);
     a.bad_tau = g.d_bad;
     a.bad_rough = g.d_bad + 1;
-    CUDA_TRY(abk::launch_ice_series(ialgo, fabs(zu - zt) < 0.01, a, cs_));
+    CUDA_TRY(abk::launch_ice_series(ialgo, zt_eq_zu(zt, zu), a, cs_));
     g.launches += 1;
     rc = t.close();
     if (rc) return rc;
@@ -2719,7 +2723,7 @@ double aerobulk_gpu_bytes_per_point(const char *calgo, int skin)
 {
     const int a = calgo ? algo_id(calgo) : 0;
     if (!a) return 0.;
-    if (!skin || a == abd::NCAR || a == abd::ANDREAS) return 88.;
+    if (!skin || !has_skin_schemes(a)) return 88.;
     return a == abd::ECMWF ? 128. : 176.;
 }
 
@@ -2732,10 +2736,9 @@ int aerobulk_gpu_kernel_info(const char *calgo, int skin, int zt_eq_zu, int *reg
     if (!a) return fail(AEROBULK_GPU_ERR_ALGO, "aerobulk_gpu_kernel_info: bulk algorithm %s is unknown!!!", calgo ? calgo : "(null)");
     int rc = ensure_device();
     if (rc) return rc;
-    const bool sk = skin && (a == abd::COARE3P0 || a == abd::COARE3P6 || a == abd::ECMWF);
     cudaFuncAttributes at;
     int blocks = 0;
-    CUDA_TRY(abk::flux_kernel_attributes(a, sk, zt_eq_zu != 0, &at, &blocks));
+    CUDA_TRY(abk::flux_kernel_attributes(a, skin && has_skin_schemes(a), zt_eq_zu != 0, &at, &blocks));
     if (registers) *registers = at.numRegs;
     if (local_bytes) *local_bytes = (int)at.localSizeBytes;
     if (blocks_per_sm) *blocks_per_sm = blocks;

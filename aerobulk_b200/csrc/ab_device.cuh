@@ -1200,5 +1200,17 @@ ABD Coeffs solve_andreas(const Uniform &u, const PointIn &p, Diag &dg)
     return c;
 }
 
+// ---------------------------------------------------------------------------
+// one TURB_<ALGO> call: the solver of the algorithm, with cool-skin (CS) / warm-layer (WL) where it has them
+// ---------------------------------------------------------------------------
+template <int ALGO, bool CS, bool WL, bool ZTEQ>
+ABD Coeffs solve_ocean(const Uniform &u, const PointIn &p, WarmLayer &wl, Diag &dg)
+{
+    if (ALGO == NCAR) return solve_ncar<ZTEQ>(u, p, dg);
+    else if (ALGO == ANDREAS) return solve_andreas<ZTEQ>(u, p, dg);
+    else if (ALGO == ECMWF) return solve_ecmwf<CS, WL, ZTEQ>(u, p, wl, dg);
+    else return solve_coare<ALGO == COARE3P6, CS, WL, ZTEQ>(u, p, wl, dg);
+}
+
 #undef ABD
 }  // namespace abd

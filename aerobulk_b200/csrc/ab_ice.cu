@@ -144,12 +144,8 @@ __global__ void __launch_bounds__(ICE_BLOCK, ICE_MIN_BLOCKS) leads_kernel(const 
     p.slp = slp;
     p.Qsw = 0.; p.rlw = 0.; p.lon = 0.; p.has_lon = false;
     WarmLayer wl = {0., 0., 0., 0.};
-    Coeffs c;
     Diag dg;
-    if (OALGO == NCAR) c = solve_ncar<ZTEQ>(a.uo, p, dg);
-    else if (OALGO == ANDREAS) c = solve_andreas<ZTEQ>(a.uo, p, dg);
-    else if (OALGO == ECMWF) c = solve_ecmwf<false, false, ZTEQ>(a.uo, p, wl, dg);
-    else c = solve_coare<OALGO == COARE3P6, false, false, ZTEQ>(a.uo, p, wl, dg);
+    const Coeffs c = solve_ocean<OALGO, false, false, ZTEQ>(a.uo, p, wl, dg);
     const AirZu air = air_at_zu(a.uo.zu, c.t_zu, c.q_zu, slp);
     const Flux f = bulk_formula(air, sst, p.ssq, c.t_zu, c.q_zu, c.Cd, c.Ch, c.Ce, wnd, c.Ub);
     if (f.tau > 10.) atomicMin(a.bad_tau, (unsigned long long)i);
@@ -162,85 +158,55 @@ __global__ void __launch_bounds__(ICE_BLOCK, ICE_MIN_BLOCKS) leads_kernel(const 
         if (a.out[17 + k]) a.out[17 + k][i] = v[k];
 }
 
-static unsigned nblocks(long long n) { return (unsigned)((n + ICE_BLOCK - 1) / ICE_BLOCK); }
-
-template <int IALGO>
-static cudaError_t ice_turb_zt(bool zteq, const IceTurbArgs &a, cudaStream_t s)
+// The instantiation a sea-ice launch runs: f(IALGO, ZTEQ) with std::integral_constant arguments, nullptr for an unknown
+// algorithm.
+template <class F>
+static auto pick_ice(int ialgo, bool zteq, F f) -> decltype(f(IntC<ICE_NEMO>{}, BoolC<false>{}))
 {
-    if (zteq) ice_turb_kernel<IALGO, true><<<nblocks(a.n), ICE_BLOCK, 0, s>>>(a);
-    else ice_turb_kernel<IALGO, false><<<nblocks(a.n), ICE_BLOCK, 0, s>>>(a);
+    const auto z = [&](auto I) { return zteq ? f(I, BoolC<true>{}) : f(I, BoolC<false>{}); };
+    switch (ialgo) {
+    case ICE_NEMO: return z(IntC<ICE_NEMO>{});
+    case ICE_EASY: return z(IntC<ICE_EASY>{});
+    case ICE_AN05: return z(IntC<ICE_AN05>{});
+    case ICE_LU12: return z(IntC<ICE_LU12>{});
+    case ICE_LG15: return z(IntC<ICE_LG15>{});
+    default: return nullptr;
+    }
+}
+
+// every launch of this file: nothing to do for n <= 0 (whatever the algorithm), else one thread per point
+template <class Args>
+static cudaError_t launch_ice(void (*k)(Args), const Args &a, cudaStream_t s)
+{
+    if (a.n <= 0) return cudaSuccess;
+    if (!k) return cudaErrorInvalidValue;
+    k<<<(unsigned)((a.n + ICE_BLOCK - 1) / ICE_BLOCK), ICE_BLOCK, 0, s>>>(a);
     return cudaGetLastError();
 }
+
 cudaError_t launch_ice_turb(int ialgo, bool zteq, const IceTurbArgs &a, cudaStream_t s)
 {
-    if (a.n <= 0) return cudaSuccess;
-    switch (ialgo) {
-    case ICE_NEMO: return ice_turb_zt<ICE_NEMO>(zteq, a, s);
-    case ICE_EASY: return ice_turb_zt<ICE_EASY>(zteq, a, s);
-    case ICE_AN05: return ice_turb_zt<ICE_AN05>(zteq, a, s);
-    case ICE_LU12: return ice_turb_zt<ICE_LU12>(zteq, a, s);
-    case ICE_LG15: return ice_turb_zt<ICE_LG15>(zteq, a, s);
-    default: return cudaErrorInvalidValue;
-    }
-}
-
-template <int IALGO>
-static cudaError_t ice_flux_zt(bool zteq, const OceIceArgs &a, cudaStream_t s)
-{
-    if (zteq) ice_flux_kernel<IALGO, true><<<nblocks(a.n), ICE_BLOCK, 0, s>>>(a);
-    else ice_flux_kernel<IALGO, false><<<nblocks(a.n), ICE_BLOCK, 0, s>>>(a);
-    return cudaGetLastError();
-}
-template <int IALGO>
-static cudaError_t ice_series_zt(bool zteq, const IceSeriesArgs &a, cudaStream_t s)
-{
-    if (zteq) ice_series_kernel<IALGO, true><<<nblocks(a.n), ICE_BLOCK, 0, s>>>(a);
-    else ice_series_kernel<IALGO, false><<<nblocks(a.n), ICE_BLOCK, 0, s>>>(a);
-    return cudaGetLastError();
-}
-cudaError_t launch_ice_series(int ialgo, bool zteq, const IceSeriesArgs &a, cudaStream_t s)
-{
-    if (a.n <= 0) return cudaSuccess;
-    switch (ialgo) {
-    case ICE_NEMO: return ice_series_zt<ICE_NEMO>(zteq, a, s);
-    case ICE_AN05: return ice_series_zt<ICE_AN05>(zteq, a, s);
-    case ICE_LU12: return ice_series_zt<ICE_LU12>(zteq, a, s);
-    case ICE_LG15: return ice_series_zt<ICE_LG15>(zteq, a, s);
-    default: return cudaErrorInvalidValue;
-    }
+    return launch_ice(pick_ice(ialgo, zteq, [](auto I, auto Z) { return ice_turb_kernel<I(), Z()>; }), a, s);
 }
 
 cudaError_t launch_ice_flux(int ialgo, bool zteq, const OceIceArgs &a, cudaStream_t s)
 {
-    if (a.n <= 0) return cudaSuccess;
-    switch (ialgo) {
-    case ICE_NEMO: return ice_flux_zt<ICE_NEMO>(zteq, a, s);
-    case ICE_EASY: return ice_flux_zt<ICE_EASY>(zteq, a, s);
-    case ICE_AN05: return ice_flux_zt<ICE_AN05>(zteq, a, s);
-    case ICE_LU12: return ice_flux_zt<ICE_LU12>(zteq, a, s);
-    case ICE_LG15: return ice_flux_zt<ICE_LG15>(zteq, a, s);
-    default: return cudaErrorInvalidValue;
-    }
+    return launch_ice(pick_ice(ialgo, zteq, [](auto I, auto Z) { return ice_flux_kernel<I(), Z()>; }), a, s);
 }
 
-template <int OALGO>
-static cudaError_t leads_zt(bool zteq, const OceIceArgs &a, cudaStream_t s)
+// the sea-ice station series has no EASY: ice_series_kernel<ICE_EASY, *> is never built
+cudaError_t launch_ice_series(int ialgo, bool zteq, const IceSeriesArgs &a, cudaStream_t s)
 {
-    if (zteq) leads_kernel<OALGO, true><<<nblocks(a.n), ICE_BLOCK, 0, s>>>(a);
-    else leads_kernel<OALGO, false><<<nblocks(a.n), ICE_BLOCK, 0, s>>>(a);
-    return cudaGetLastError();
+    return launch_ice(pick_ice(ialgo, zteq, [](auto I, auto Z) -> void (*)(IceSeriesArgs) {
+                          if constexpr (I() == ICE_EASY) return nullptr;
+                          else return ice_series_kernel<I(), Z()>;
+                      }), a, s);
 }
+
+// the leads run the ocean algorithm without skin
 cudaError_t launch_leads(int oalgo, bool zteq, const OceIceArgs &a, cudaStream_t s)
 {
-    if (a.n <= 0) return cudaSuccess;
-    switch (oalgo) {
-    case COARE3P0: return leads_zt<COARE3P0>(zteq, a, s);
-    case COARE3P6: return leads_zt<COARE3P6>(zteq, a, s);
-    case NCAR: return leads_zt<NCAR>(zteq, a, s);
-    case ECMWF: return leads_zt<ECMWF>(zteq, a, s);
-    case ANDREAS: return leads_zt<ANDREAS>(zteq, a, s);
-    default: return cudaErrorInvalidValue;
-    }
+    return launch_ice(pick_ocean(oalgo, false, zteq, [](auto A, auto, auto Z) { return leads_kernel<A(), Z()>; }), a, s);
 }
 
 }  // namespace abk

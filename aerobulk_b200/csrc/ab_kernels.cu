@@ -159,6 +159,33 @@ __global__ void __launch_bounds__(SORT_BLOCK) classify_kernel(const FluxArgs a, 
     }
 }
 
+// warm-layer state of point i at the start of a step (*_INIT values at kt == nit000), and its write-back
+template <int ALGO, class Args>
+__device__ __forceinline__ void load_warm_layer(const Args &a, long long i, WarmLayer &wl)
+{
+    if (ALGO == ECMWF) {
+        wl.Hz = 3.;                                            // rd0, mod_skin_ecmwf.f90:57 (constant)
+        wl.dT = a.first_step ? 0. : a.dT_wl[i];
+    } else if (a.first_step) {
+        wl.Hz = 20.;                                           // Hwl_max, mod_blk_coare3p6.f90:84-87
+    } else {
+        wl.dT = a.dT_wl[i];
+        wl.Hz = a.Hz_wl[i];
+        wl.Qac = a.Qnt_ac[i];
+        wl.Tac = a.Tau_ac[i];
+    }
+}
+template <int ALGO, class Args>
+__device__ __forceinline__ void store_warm_layer(const Args &a, long long i, const WarmLayer &wl)
+{
+    a.dT_wl[i] = wl.dT;
+    if (ALGO != ECMWF) {
+        a.Hz_wl[i] = wl.Hz;
+        a.Qnt_ac[i] = wl.Qac;
+        a.Tau_ac[i] = wl.Tac;
+    }
+}
+
 template <int ALGO, bool SKIN, bool ZTEQ>
 __global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOCKS_NOSKIN) flux_kernel(const FluxArgs a)
 {
@@ -204,34 +231,12 @@ __global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOC
             p.lon = __ldg(a.lon + i);
             p.has_lon = true;
         }
-        if (ALGO == ECMWF) {
-            wl.Hz = 3.;                                            // rd0, mod_skin_ecmwf.f90:57 (constant)
-            wl.dT = a.first_step ? 0. : a.dT_wl[i];
-        } else if (a.first_step) {
-            wl.Hz = 20.;                                           // Hwl_max, mod_blk_coare3p6.f90:84-87
-        } else {
-            wl.dT = a.dT_wl[i];
-            wl.Hz = a.Hz_wl[i];
-            wl.Qac = a.Qnt_ac[i];
-            wl.Tac = a.Tau_ac[i];
-        }
+        load_warm_layer<ALGO>(a, i, wl);
     }
 
-    Coeffs c;
     Diag dg;   // optional TURB_* outputs: unused here, eliminated by the compiler
-    if (ALGO == NCAR) c = solve_ncar<ZTEQ>(a.u, p, dg);
-    else if (ALGO == ANDREAS) c = solve_andreas<ZTEQ>(a.u, p, dg);
-    else if (ALGO == ECMWF) c = solve_ecmwf<SKIN, SKIN, ZTEQ>(a.u, p, wl, dg);
-    else c = solve_coare<ALGO == COARE3P6, SKIN, SKIN, ZTEQ>(a.u, p, wl, dg);
-
-    if (SKIN) {
-        a.dT_wl[i] = wl.dT;
-        if (ALGO != ECMWF) {
-            a.Hz_wl[i] = wl.Hz;
-            a.Qnt_ac[i] = wl.Qac;
-            a.Tau_ac[i] = wl.Tac;
-        }
-    }
+    const Coeffs c = solve_ocean<ALGO, SKIN, SKIN, ZTEQ>(a.u, p, wl, dg);
+    if (SKIN) store_warm_layer<ALGO>(a, i, wl);
 
     // ---- flux assembly (BULK_FORMULA, :184-185) and stress vector (:189-194)
     const Flux f = bulk_formula(air_at_zu(a.u.zu, c.t_zu, c.q_zu, slp), c.Ts, c.qs, c.t_zu, c.q_zu, c.Cd, c.Ch, c.Ce, p.wnd, c.Ub);
@@ -251,34 +256,20 @@ __global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOC
     if (a.T_s) a.T_s[i] = c.Ts;
 }
 
-template <int ALGO, bool SKIN, bool ZTEQ>
-static cudaError_t launch_one(const FluxArgs &a, cudaStream_t s)
+static auto flux_kernel_for(int algo, bool skin, bool zteq)
 {
-    if (a.n <= 0) return cudaSuccess;
-    const long long span = a.perm ? (a.n + SORT_WIN - 1) / SORT_WIN * SORT_WIN : a.n;   // whole windows of slots
-    const long long blocks = (span + FLUX_BLOCK - 1) / FLUX_BLOCK;
-    flux_kernel<ALGO, SKIN, ZTEQ><<<(unsigned)blocks, FLUX_BLOCK, 0, s>>>(a);
-    return cudaGetLastError();
-}
-
-template <int ALGO, bool SKIN>
-static cudaError_t launch_zt(bool zteq, const FluxArgs &a, cudaStream_t s)
-{
-    return zteq ? launch_one<ALGO, SKIN, true>(a, s) : launch_one<ALGO, SKIN, false>(a, s);
+    return pick_ocean(algo, skin, zteq, [](auto A, auto S, auto Z) { return flux_kernel<A(), S(), Z()>; });
 }
 
 cudaError_t launch_flux(int algo, bool skin, bool zteq, const FluxArgs &a, cudaStream_t s)
 {
-    switch (algo) {
-    case COARE3P0: return skin ? launch_zt<COARE3P0, true>(zteq, a, s) : launch_zt<COARE3P0, false>(zteq, a, s);
-    case COARE3P6: return skin ? launch_zt<COARE3P6, true>(zteq, a, s) : launch_zt<COARE3P6, false>(zteq, a, s);
-    case ECMWF: return skin ? launch_zt<ECMWF, true>(zteq, a, s) : launch_zt<ECMWF, false>(zteq, a, s);
-    case NCAR: return launch_zt<NCAR, false>(zteq, a, s);
-    case ANDREAS: return launch_zt<ANDREAS, false>(zteq, a, s);
-    default: return cudaErrorInvalidValue;
-    }
+    const auto k = flux_kernel_for(algo, skin, zteq);
+    if (!k) return cudaErrorInvalidValue;
+    if (a.n <= 0) return cudaSuccess;
+    const long long span = a.perm ? (a.n + SORT_WIN - 1) / SORT_WIN * SORT_WIN : a.n;   // whole windows of slots
+    k<<<(unsigned)((span + FLUX_BLOCK - 1) / FLUX_BLOCK), FLUX_BLOCK, 0, s>>>(a);
+    return cudaGetLastError();
 }
-
 
 // ---------------------------------------------------------------------------
 // turb_kernel<ALGO,CS,WL,ZTEQ>: the direct TURB_* entry (SURVEY.md 8f row 1) on the same solvers
@@ -311,33 +302,10 @@ __global__ void __launch_bounds__(FLUX_BLOCK, (CS || WL) ? AB_MIN_BLOCKS : AB_MI
             p.has_lon = true;
         }
     }
-    if (WL) {
-        if (ALGO == ECMWF) {
-            wl.Hz = 3.;
-            wl.dT = a.first_step ? 0. : a.dT_wl[i];
-        } else if (a.first_step) {
-            wl.Hz = 20.;
-        } else {
-            wl.dT = a.dT_wl[i];
-            wl.Hz = a.Hz_wl[i];
-            wl.Qac = a.Qnt_ac[i];
-            wl.Tac = a.Tau_ac[i];
-        }
-    }
-    Coeffs c;
+    if (WL) load_warm_layer<ALGO>(a, i, wl);
     Diag dg;
-    if (ALGO == NCAR) c = solve_ncar<ZTEQ>(a.u, p, dg);
-    else if (ALGO == ANDREAS) c = solve_andreas<ZTEQ>(a.u, p, dg);
-    else if (ALGO == ECMWF) c = solve_ecmwf<CS, WL, ZTEQ>(a.u, p, wl, dg);
-    else c = solve_coare<ALGO == COARE3P6, CS, WL, ZTEQ>(a.u, p, wl, dg);
-    if (WL) {
-        a.dT_wl[i] = wl.dT;
-        if (ALGO != ECMWF) {
-            a.Hz_wl[i] = wl.Hz;
-            a.Qnt_ac[i] = wl.Qac;
-            a.Tau_ac[i] = wl.Tac;
-        }
-    }
+    const Coeffs c = solve_ocean<ALGO, CS, WL, ZTEQ>(a.u, p, wl, dg);
+    if (WL) store_warm_layer<ALGO>(a, i, wl);
     if (SKIN) {
         a.T_s[i] = c.Ts;
         a.q_s[i] = c.qs;
@@ -356,33 +324,18 @@ __global__ void __launch_bounds__(FLUX_BLOCK, (CS || WL) ? AB_MIN_BLOCKS : AB_MI
     if (WL && a.opt[9]) a.opt[9][i] = wl.Hz;
 }
 
-template <int ALGO, bool CS, bool WL>
-static cudaError_t turb_zt(bool zteq, const TurbArgs &a, cudaStream_t s)
-{
-    if (a.n <= 0) return cudaSuccess;
-    const unsigned blocks = (unsigned)((a.n + FLUX_BLOCK - 1) / FLUX_BLOCK);
-    if (zteq) turb_kernel<ALGO, CS, WL, true><<<blocks, FLUX_BLOCK, 0, s>>>(a);
-    else turb_kernel<ALGO, CS, WL, false><<<blocks, FLUX_BLOCK, 0, s>>>(a);
-    return cudaGetLastError();
-}
-template <int ALGO>
-static cudaError_t turb_skin(bool cs, bool wl, bool zteq, const TurbArgs &a, cudaStream_t s)
-{
-    if (cs && wl) return turb_zt<ALGO, true, true>(zteq, a, s);
-    if (cs) return turb_zt<ALGO, true, false>(zteq, a, s);
-    if (wl) return turb_zt<ALGO, false, true>(zteq, a, s);
-    return turb_zt<ALGO, false, false>(zteq, a, s);
-}
+// cool skin and warm layer are separate options here; NCAR and ANDREAS take neither
 cudaError_t launch_turb(int algo, bool cs, bool wl, bool zteq, const TurbArgs &a, cudaStream_t s)
 {
-    switch (algo) {
-    case COARE3P0: return turb_skin<COARE3P0>(cs, wl, zteq, a, s);
-    case COARE3P6: return turb_skin<COARE3P6>(cs, wl, zteq, a, s);
-    case ECMWF: return turb_skin<ECMWF>(cs, wl, zteq, a, s);
-    case NCAR: return turb_zt<NCAR, false, false>(zteq, a, s);
-    case ANDREAS: return turb_zt<ANDREAS, false, false>(zteq, a, s);
-    default: return cudaErrorInvalidValue;
-    }
+    const auto k = pick_ocean(algo, cs || wl, zteq, [cs, wl](auto A, auto S, auto Z) {
+        if constexpr (!S()) return turb_kernel<A(), false, false, Z()>;
+        else return cs ? (wl ? turb_kernel<A(), true, true, Z()> : turb_kernel<A(), true, false, Z()>)
+                       : turb_kernel<A(), false, true, Z()>;
+    });
+    if (!k) return cudaErrorInvalidValue;
+    if (a.n <= 0) return cudaSuccess;
+    k<<<(unsigned)((a.n + FLUX_BLOCK - 1) / FLUX_BLOCK), FLUX_BLOCK, 0, s>>>(a);
+    return cudaGetLastError();
 }
 
 int flux_block_size() { return FLUX_BLOCK; }
@@ -397,28 +350,13 @@ cudaError_t launch_classify(const FluxArgs &a, unsigned short *perm, bool skin, 
     return cudaGetLastError();
 }
 
-template <int ALGO, bool SKIN, bool ZTEQ>
-static cudaError_t attr_one(cudaFuncAttributes *attr, int *blocks_per_sm)
-{
-    cudaError_t e = cudaFuncGetAttributes(attr, flux_kernel<ALGO, SKIN, ZTEQ>);
-    if (e != cudaSuccess || !blocks_per_sm) return e;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, flux_kernel<ALGO, SKIN, ZTEQ>, FLUX_BLOCK, 0);
-}
-template <int ALGO, bool SKIN>
-static cudaError_t attr_zt(bool zteq, cudaFuncAttributes *attr, int *blocks_per_sm)
-{
-    return zteq ? attr_one<ALGO, SKIN, true>(attr, blocks_per_sm) : attr_one<ALGO, SKIN, false>(attr, blocks_per_sm);
-}
 cudaError_t flux_kernel_attributes(int algo, bool skin, bool zteq, cudaFuncAttributes *attr, int *blocks_per_sm)
 {
-    switch (algo) {
-    case COARE3P0: return skin ? attr_zt<COARE3P0, true>(zteq, attr, blocks_per_sm) : attr_zt<COARE3P0, false>(zteq, attr, blocks_per_sm);
-    case COARE3P6: return skin ? attr_zt<COARE3P6, true>(zteq, attr, blocks_per_sm) : attr_zt<COARE3P6, false>(zteq, attr, blocks_per_sm);
-    case ECMWF: return skin ? attr_zt<ECMWF, true>(zteq, attr, blocks_per_sm) : attr_zt<ECMWF, false>(zteq, attr, blocks_per_sm);
-    case NCAR: return attr_zt<NCAR, false>(zteq, attr, blocks_per_sm);
-    case ANDREAS: return attr_zt<ANDREAS, false>(zteq, attr, blocks_per_sm);
-    default: return cudaErrorInvalidValue;
-    }
+    const auto k = flux_kernel_for(algo, skin, zteq);
+    if (!k) return cudaErrorInvalidValue;
+    cudaError_t e = cudaFuncGetAttributes(attr, k);
+    if (e != cudaSuccess || !blocks_per_sm) return e;
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k, FLUX_BLOCK, 0);
 }
 
 // ---------------------------------------------------------------------------

@@ -3,10 +3,32 @@
 
 #include <cuda_runtime.h>
 
+#include <type_traits>
+
 #include "ab_device.cuh"
 #include "ab_ice.cuh"
 
 namespace abk {
+
+template <int V> using IntC = std::integral_constant<int, V>;
+template <bool V> using BoolC = std::bool_constant<V>;
+
+// The instantiation an ocean launch runs: f(ALGO, SKIN, ZTEQ) with std::integral_constant arguments, nullptr for an
+// unknown algorithm.  Skin schemes exist for COARE 3.x and ECMWF only: NCAR and ANDREAS ignore `skin`.
+template <class F>
+auto pick_ocean(int algo, bool skin, bool zteq, F f) -> decltype(f(IntC<abd::NCAR>{}, BoolC<false>{}, BoolC<false>{}))
+{
+    const auto z = [&](auto A, auto S) { return zteq ? f(A, S, BoolC<true>{}) : f(A, S, BoolC<false>{}); };
+    const auto sz = [&](auto A) { return skin ? z(A, BoolC<true>{}) : z(A, BoolC<false>{}); };
+    switch (algo) {
+    case abd::COARE3P0: return sz(IntC<abd::COARE3P0>{});
+    case abd::COARE3P6: return sz(IntC<abd::COARE3P6>{});
+    case abd::ECMWF: return sz(IntC<abd::ECMWF>{});
+    case abd::NCAR: return z(IntC<abd::NCAR>{}, BoolC<false>{});
+    case abd::ANDREAS: return z(IntC<abd::ANDREAS>{}, BoolC<false>{});
+    default: return nullptr;
+    }
+}
 
 // One fused launch = reference aerobulk_compute (src/mod_aerobulk_compute.f90:22-213)
 // steps 1-9 for `n` consecutive grid points.

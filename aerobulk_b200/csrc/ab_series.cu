@@ -60,13 +60,9 @@ __global__ void __launch_bounds__(SERIES_BLOCK, SERIES_MIN_BLOCKS) series_kernel
         p.lon = lon;
         p.has_lon = true;
 
-        Coeffs c;
         Diag dg;
         dg.dT_cs = 0.;
-        if (ALGO == NCAR) c = solve_ncar<ZTEQ>(u, p, dg);
-        else if (ALGO == ANDREAS) c = solve_andreas<ZTEQ>(u, p, dg);
-        else if (ALGO == ECMWF) c = solve_ecmwf<SKIN, SKIN, ZTEQ>(u, p, wl, dg);
-        else c = solve_coare<ALGO == COARE3P6, SKIN, SKIN, ZTEQ>(u, p, wl, dg);
+        const Coeffs c = solve_ocean<ALGO, SKIN, SKIN, ZTEQ>(u, p, wl, dg);
         const double Ts = SKIN ? c.Ts : sst;
         const double qs = SKIN ? c.qs : p.ssq;
 
@@ -90,26 +86,13 @@ __global__ void __launch_bounds__(SERIES_BLOCK, SERIES_MIN_BLOCKS) series_kernel
     }
 }
 
-template <int ALGO, bool SKIN>
-static cudaError_t series_zt(bool zteq, const SeriesArgs &a, cudaStream_t s)
-{
-    if (a.S <= 0 || a.Nt <= 0) return cudaSuccess;
-    const unsigned blocks = (unsigned)((a.S + SERIES_BLOCK - 1) / SERIES_BLOCK);
-    if (zteq) series_kernel<ALGO, SKIN, true><<<blocks, SERIES_BLOCK, 0, s>>>(a);
-    else series_kernel<ALGO, SKIN, false><<<blocks, SERIES_BLOCK, 0, s>>>(a);
-    return cudaGetLastError();
-}
-
 cudaError_t launch_series(int algo, bool skin, bool zteq, const SeriesArgs &a, cudaStream_t s)
 {
-    switch (algo) {
-    case COARE3P0: return skin ? series_zt<COARE3P0, true>(zteq, a, s) : series_zt<COARE3P0, false>(zteq, a, s);
-    case COARE3P6: return skin ? series_zt<COARE3P6, true>(zteq, a, s) : series_zt<COARE3P6, false>(zteq, a, s);
-    case ECMWF: return skin ? series_zt<ECMWF, true>(zteq, a, s) : series_zt<ECMWF, false>(zteq, a, s);
-    case NCAR: return series_zt<NCAR, false>(zteq, a, s);
-    case ANDREAS: return series_zt<ANDREAS, false>(zteq, a, s);
-    default: return cudaErrorInvalidValue;
-    }
+    const auto k = pick_ocean(algo, skin, zteq, [](auto A, auto S, auto Z) { return series_kernel<A(), S(), Z()>; });
+    if (!k) return cudaErrorInvalidValue;
+    if (a.S <= 0 || a.Nt <= 0) return cudaSuccess;
+    k<<<(unsigned)((a.S + SERIES_BLOCK - 1) / SERIES_BLOCK), SERIES_BLOCK, 0, s>>>(a);
+    return cudaGetLastError();
 }
 
 }  // namespace abk

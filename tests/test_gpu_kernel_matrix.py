@@ -6,7 +6,8 @@ holds, one call that launches it.  The CPU census test reads the instantiations 
 (`cuobjdump -symbols`) and fails when one has no entry, so a new template parameter or algorithm cannot ship without a
 parity case.  The GPU tests run each entry at two point counts and gate it like the model path (parity_util).
 
-Which instantiation a call launches (aerobulk_b200/csrc/ab_api.cu, ab_kernels.cu, ab_series.cu, ab_ice.cu):
+Which instantiation a call launches: each launch_* function picks it through pick_ocean (ab_kernels.cuh) or pick_ice
+(ab_ice.cu), from the flags ab_api.cu derives with zt_eq_zu and has_skin_schemes:
   - ZTEQ = |zu - zt| < 0.01, for every kernel;
   - flux_kernel<ALGO, SKIN, ZTEQ> (aerobulk_model): SKIN = l_use_skin for COARE 3.0 / 3.6 and ECMWF, false otherwise;
   - turb_kernel<ALGO, CS, WL, ZTEQ> (TURB_*): CS = l_use_cs, WL = l_use_wl (NCAR and ANDREAS take neither);
