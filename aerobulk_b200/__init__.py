@@ -7,7 +7,8 @@ reference's ``aerobulk_model`` interface used by the tests and by ``bench.py``.
 There is no CPU fallback: importing :mod:`aerobulk_b200.model` without the built
 library raises, and every compute call fails without a CUDA device.
 """
-from .model import (AerobulkError, aerobulk_model, aerobulk_model_device, get_state, set_state, humidity_type,
+from .model import (AerobulkError, aerobulk_model, aerobulk_model_device, aerobulk_model_f32, aerobulk_model_device_f32,
+                    get_state, set_state, humidity_type,
                     last_error, launch_count, lib, measure_fp64_peak, nb_iter, reset, set_gdept, set_nb_iter,
                     set_rdt, set_stream, set_verbose, synchronize, use_skin, work_per_point, bytes_per_point, kernel_info,
                     set_nitend, turb, series, series_csv, series_device, SERIES_OUT, turb_ice, oce_ice,
@@ -17,7 +18,8 @@ from .model import (AerobulkError, aerobulk_model, aerobulk_model_device, get_st
                     aerobulk_bye)
 
 ALGORITHMS = ("coare3p0", "coare3p6", "ncar", "ecmwf", "andreas")
-__all__ = ["ALGORITHMS", "AerobulkError", "aerobulk_model", "aerobulk_model_device", "get_state", "set_state", "humidity_type",
+__all__ = ["ALGORITHMS", "AerobulkError", "aerobulk_model", "aerobulk_model_device", "aerobulk_model_f32",
+           "aerobulk_model_device_f32", "get_state", "set_state", "humidity_type",
            "last_error", "launch_count", "lib", "measure_fp64_peak", "nb_iter", "reset", "set_gdept", "set_nb_iter",
            "set_rdt", "set_stream", "set_verbose", "synchronize", "use_skin", "work_per_point", "bytes_per_point", "kernel_info",
            "set_nitend", "turb", "series", "series_csv", "series_device", "SERIES_OUT", "turb_ice", "oce_ice",

@@ -3,9 +3,10 @@
 // and the warm-layer module arrays of src/mod_skin_coare.f90:31-36 /
 // src/mod_skin_ecmwf.f90:52-55) and the C ABI declared in include/aerobulk_gpu.h.
 //
-// Data layout in HBM: every field is one contiguous FP64 array of Ni*Nj points in the
-// caller's (Fortran, column-major) order; a row block j0..j1 is the byte range
-// [j0*Ni*8, j1*Ni*8) of each field, so chunks and shards are plain pointer offsets.
+// Data layout in HBM: every field is one contiguous array of Ni*Nj points in the caller's
+// (Fortran, column-major) order, FP64 -- or FP32 for the whole of an aerobulk_gpu_model*_f32
+// call; a row block j0..j1 is the byte range [j0*Ni*es, j1*Ni*es) of each field (es = 8 or
+// 4 bytes per element), so chunks and shards are plain pointer offsets.
 // Host-array calls stage through 8 input + 6 output device arrays (grow-only) and are
 // pipelined in row-block chunks over three streams (H2D | kernel | D2H).
 // Warm-layer state never leaves the device between jt==1 and jt==nitend.
@@ -66,7 +67,8 @@ bool zerocopy_on()
     return v;
 }
 // device alias of a pinned (page-locked, device-mapped) host pointer, or nullptr
-const double *device_alias(const double *p)
+template <class T>
+T *device_alias(T *p)
 {
     if (!p) return nullptr;
     cudaPointerAttributes a;
@@ -74,7 +76,13 @@ const double *device_alias(const double *p)
         cudaGetLastError();
         return nullptr;
     }
-    return (a.type == cudaMemoryTypeHost && a.devicePointer) ? static_cast<const double *>(a.devicePointer) : nullptr;
+    return (a.type == cudaMemoryTypeHost && a.devicePointer) ? static_cast<T *>(a.devicePointer) : nullptr;
+}
+// element i of an array of es-byte elements (aerobulk_model arrays are FP64 or FP32, see model_impl); NULL stays NULL
+template <class T>
+T *elem_at(T *p, long long i, size_t es)
+{
+    return p ? p + i * (long long)es : nullptr;
 }
 long long min_chunk_points()
 {
@@ -184,11 +192,11 @@ struct Session {
     long long n_coare = 0, n_ecmwf = 0, cap_coare = 0, cap_ecmwf = 0;
     double *c_state[4] = {nullptr, nullptr, nullptr, nullptr};   // dT_wl, Hz_wl, Qnt_ac, Tau_ac
     double *e_dT_wl = nullptr;
-    // ---- staging for host-array calls
+    // ---- staging for host-array calls: 14 rows of `cap` bytes (a multiple of ROW_ALIGN), for FP64 and FP32 calls alike
     long long cap = 0;
-    double *d_in[8] = {}, *d_out[6] = {};
-    // ---- pinned bounce slab for pageable caller arrays (14 fields, pitch cap_hb) and its device alias
-    double *hb = nullptr, *hb_dev = nullptr;
+    char *d_in[8] = {}, *d_out[6] = {};
+    // ---- pinned bounce slab for pageable caller arrays (14 rows, pitch cap_hb bytes: a multiple of ROW_ALIGN) and its device alias
+    char *hb = nullptr, *hb_dev = nullptr;
     long long cap_hb = 0;
     // ---- the same for the other host-array entry points (turb, series, ice): arrays packed back to back
     double *hx = nullptr, *hx_dev = nullptr;
@@ -220,7 +228,8 @@ struct Session {
     bool bad_pending = false;
     int pend_launches = 0;        // model calls whose flag has not been looked at yet
     int last_Ni = 0;
-    const double *last_taux = nullptr, *last_tauy = nullptr;   // device pointers of the last launch
+    const void *last_taux = nullptr, *last_tauy = nullptr;   // device pointers of the last launch
+    size_t last_es = sizeof(double);                         // and the size of their elements
     long launches = 0;
     // ---- opt-in: device-pointer calls never synchronise, not even at jt == Nt (aerobulk_gpu_set_async)
     bool async_device = false;
@@ -426,28 +435,30 @@ void bind_wl_state(Args &a, int ialgo, long long s0)
     }
 }
 
-// Moves elements [s0, s0+len) of `nf` fields between host and device staging.  Consecutive fields whose HOST arrays are
-// equally spaced in memory (a caller that keeps its fields in one slab) go in ONE pitched copy: with H2D and D2H running
-// concurrently in 0.4-3 MB pieces the DMA engines reach 62 GB/s aggregate, with one pitched copy per chunk 72 GB/s
-// (tools/probes/duplex_probe.cu on this pool's B200: 1.86 -> 1.62 ms per 1 M-point skin call).
-int copy_fields(int nf, double *const *dev, double *const *host, long long dev_pitch, long long s0, long long len, bool h2d,
-                cudaStream_t st)
+// Moves elements [s0, s0+len) of `nf` fields of es-byte elements between host and device staging (dev_pitch: bytes
+// between device rows).  Consecutive fields whose HOST arrays are equally spaced in memory (a caller that keeps its
+// fields in one slab) go in ONE pitched copy: with H2D and D2H running concurrently in 0.4-3 MB pieces the DMA engines
+// reach 62 GB/s aggregate, with one pitched copy per chunk 72 GB/s (tools/probes/duplex_probe.cu on this pool's B200:
+// 1.86 -> 1.62 ms per 1 M-point skin call).
+int copy_fields(int nf, char *const *dev, char *const *host, long long dev_pitch, long long s0, long long len, size_t es,
+                bool h2d, cudaStream_t st)
 {
     const long long MAX_PITCH_BYTES = 0x7fffffffLL;   // cudaDevAttrMaxPitch
+    const long long o = s0 * (long long)es, bytes = len * (long long)es;
     int k = 0;
     while (k < nf) {
         if (!host[k]) { ++k; continue; }
         int run = 1;
         if (k + 1 < nf && host[k + 1]) {
-            const long long d = host[k + 1] - host[k];
-            if (d >= len && d * 8 <= MAX_PITCH_BYTES && dev_pitch * 8 <= MAX_PITCH_BYTES)
+            const long long d = host[k + 1] - host[k];   // bytes
+            if (d >= bytes && d <= MAX_PITCH_BYTES && dev_pitch <= MAX_PITCH_BYTES)
                 while (k + run < nf && host[k + run] && host[k + run] - host[k + run - 1] == d) ++run;
         }
         if (run > 1 && g.pitched_ok) {
-            const size_t hp = (size_t)(host[k + 1] - host[k]) * 8, dp = (size_t)dev_pitch * 8, w = (size_t)len * 8;
+            const size_t hp = (size_t)(host[k + 1] - host[k]), dp = (size_t)dev_pitch, w = (size_t)bytes;
             const cudaError_t e =
-                h2d ? cudaMemcpy2DAsync(dev[k] + s0, dp, host[k] + s0, hp, w, (size_t)run, cudaMemcpyHostToDevice, st)
-                    : cudaMemcpy2DAsync(host[k] + s0, hp, dev[k] + s0, dp, w, (size_t)run, cudaMemcpyDeviceToHost, st);
+                h2d ? cudaMemcpy2DAsync(dev[k] + o, dp, host[k] + o, hp, w, (size_t)run, cudaMemcpyHostToDevice, st)
+                    : cudaMemcpy2DAsync(host[k] + o, hp, dev[k] + o, dp, w, (size_t)run, cudaMemcpyDeviceToHost, st);
             if (e == cudaErrorInvalidValue) {
                 // equally spaced but SEPARATE pinned allocations: the driver refuses a pitched copy that spans them.
                 // Nothing was enqueued; use plain copies from now on.
@@ -458,32 +469,41 @@ int copy_fields(int nf, double *const *dev, double *const *host, long long dev_p
             CUDA_TRY(e);
         } else if (run > 1) {
             for (int j = k; j < k + run; ++j) {
-                if (h2d) CUDA_TRY(cudaMemcpyAsync(dev[j] + s0, host[j] + s0, sizeof(double) * (size_t)len, cudaMemcpyHostToDevice, st));
-                else CUDA_TRY(cudaMemcpyAsync(host[j] + s0, dev[j] + s0, sizeof(double) * (size_t)len, cudaMemcpyDeviceToHost, st));
+                if (h2d) CUDA_TRY(cudaMemcpyAsync(dev[j] + o, host[j] + o, (size_t)bytes, cudaMemcpyHostToDevice, st));
+                else CUDA_TRY(cudaMemcpyAsync(host[j] + o, dev[j] + o, (size_t)bytes, cudaMemcpyDeviceToHost, st));
             }
         } else {
-            if (h2d) CUDA_TRY(cudaMemcpyAsync(dev[k] + s0, host[k] + s0, sizeof(double) * (size_t)len, cudaMemcpyHostToDevice, st));
-            else CUDA_TRY(cudaMemcpyAsync(host[k] + s0, dev[k] + s0, sizeof(double) * (size_t)len, cudaMemcpyDeviceToHost, st));
+            if (h2d) CUDA_TRY(cudaMemcpyAsync(dev[k] + o, host[k] + o, (size_t)bytes, cudaMemcpyHostToDevice, st));
+            else CUDA_TRY(cudaMemcpyAsync(host[k] + o, dev[k] + o, (size_t)bytes, cudaMemcpyDeviceToHost, st));
         }
         k += run;
     }
     return 0;
 }
 
-int ensure_staging(long long n)
+// Row pitch of the staging arrays and of the pinned slab: the bytes of one field (points x element size) rounded up to
+// ROW_ALIGN.  Both are grow-only and shared by FP64 and FP32 calls, so a row sized for an odd number of floats must not
+// leave a later, smaller FP64 call with rows that are not 8-byte aligned; 256 bytes also keeps every row on a whole
+// number of 128-byte lines for coalesced access.
+constexpr long long ROW_ALIGN = 256;
+long long aligned_row(long long bytes) { return (bytes + ROW_ALIGN - 1) / ROW_ALIGN * ROW_ALIGN; }
+
+// `row`: bytes per field (points x element size)
+int ensure_staging(long long row)
 {
-    if (n <= g.cap) return 0;
-    // one slab, fields equally spaced (pitch = cap doubles): a run of equally spaced caller arrays then moves with ONE
+    row = aligned_row(row);
+    if (row <= g.cap) return 0;
+    // one slab, fields equally spaced (pitch = cap bytes): a run of equally spaced caller arrays then moves with ONE
     // pitched copy per chunk (see copy_fields)
     if (g.d_in[0]) cudaFree(g.d_in[0]);
     for (int k = 0; k < 8; ++k) g.d_in[k] = nullptr;
     for (int k = 0; k < 6; ++k) g.d_out[k] = nullptr;
     g.cap = 0;
-    double *slab = nullptr;
-    CUDA_TRY(cudaMalloc(&slab, sizeof(double) * (size_t)n * 14));
-    for (int k = 0; k < 8; ++k) g.d_in[k] = slab + (long long)k * n;
-    for (int k = 0; k < 6; ++k) g.d_out[k] = slab + (long long)(8 + k) * n;
-    g.cap = n;
+    char *slab = nullptr;
+    CUDA_TRY(cudaMalloc(&slab, (size_t)row * 14));
+    for (int k = 0; k < 8; ++k) g.d_in[k] = slab + (long long)k * row;
+    for (int k = 0; k < 6; ++k) g.d_out[k] = slab + (long long)(8 + k) * row;
+    g.cap = row;
     return 0;
 }
 
@@ -496,15 +516,16 @@ void free_bounce()
     g.hx = g.hx_dev = nullptr;
     g.cap_hx = 0;
 }
-// Grows a mapped pinned slab to n rows of `rows` doubles (cap counts n).  False, with the slab released, when the host
-// has no pinned memory to spare: the session stays usable and the caller keeps the driver-staged copies.
-bool grow_mapped(double *&h, double *&d, long long &cap, long long n, int rows)
+// Grows a mapped pinned slab to `rows` rows of n elements of type T (cap counts n).  False, with the slab released, when
+// the host has no pinned memory to spare: the session stays usable and the caller keeps the driver-staged copies.
+template <class T>
+bool grow_mapped(T *&h, T *&d, long long &cap, long long n, int rows)
 {
     if (n <= cap) return true;
     if (h) cudaFreeHost(h);
     h = d = nullptr;
     cap = 0;
-    if (cudaHostAlloc(&h, sizeof(double) * (size_t)n * rows, cudaHostAllocPortable | cudaHostAllocMapped) != cudaSuccess ||
+    if (cudaHostAlloc(&h, sizeof(T) * (size_t)n * rows, cudaHostAllocPortable | cudaHostAllocMapped) != cudaSuccess ||
         cudaHostGetDevicePointer(&d, h, 0) != cudaSuccess) {
         cudaGetLastError();
         if (h) cudaFreeHost(h);
@@ -514,30 +535,36 @@ bool grow_mapped(double *&h, double *&d, long long &cap, long long n, int rows)
     cap = n;
     return true;
 }
-bool ensure_bounce(long long n)
+// `row`: bytes per field (points x element size)
+bool ensure_bounce(long long row)
 {
-    if (n <= g.cap_hb) return true;
-    if (sizeof(double) * (size_t)n * 14 > bounce_max_bytes()) return false;
+    row = aligned_row(row);
+    if (row <= g.cap_hb) return true;
+    if ((size_t)row * 14 > bounce_max_bytes()) return false;
     free_bounce();
-    return grow_mapped(g.hb, g.hb_dev, g.cap_hb, n, 14);
+    return grow_mapped(g.hb, g.hb_dev, g.cap_hb, row, 14);
 }
-// appends the copy of len doubles from src to dst, cut into COPY_PIECE_BYTES pieces for the copy threads
-void add_pieces(std::vector<CopyPiece> &pieces, double *dst, const double *src, long long len)
+// appends the copy of `bytes` bytes from src to dst, cut into COPY_PIECE_BYTES pieces for the copy threads
+void add_pieces(std::vector<CopyPiece> &pieces, void *dst, const void *src, size_t bytes)
 {
-    const long long step = (long long)(COPY_PIECE_BYTES / sizeof(double));
-    for (long long o = 0; o < len; o += step)
-        pieces.push_back(CopyPiece{dst + o, src + o, sizeof(double) * (size_t)(len - o < step ? len - o : step)});
+    char *d = static_cast<char *>(dst);
+    const char *s = static_cast<const char *>(src);
+    for (size_t o = 0; o < bytes; o += COPY_PIECE_BYTES)
+        pieces.push_back(CopyPiece{d + o, s + o, bytes - o < COPY_PIECE_BYTES ? bytes - o : COPY_PIECE_BYTES});
 }
-// copy points [s0, s0+len) of nf fields between the caller's arrays and the bounce slab rows row0.., on the copy threads
-void bounce_copy(int nf, double *const *user, int row0, long long s0, long long len, bool to_slab)
+// copy points [s0, s0+len) of nf fields of es-byte elements between the caller's arrays and the bounce slab rows
+// row0.., on the copy threads
+void bounce_copy(int nf, char *const *user, int row0, long long s0, long long len, size_t es, bool to_slab)
 {
     static thread_local std::vector<CopyPiece> pieces;
     pieces.clear();
+    const long long o = s0 * (long long)es;
+    const size_t bytes = (size_t)len * es;
     for (int k = 0; k < nf; ++k) {
         if (!user[k]) continue;
-        double *u = user[k] + s0, *b = g.hb + (long long)(row0 + k) * g.cap_hb + s0;
-        if (to_slab) add_pieces(pieces, b, u, len);
-        else add_pieces(pieces, u, b, len);
+        char *u = user[k] + o, *b = g.hb + (long long)(row0 + k) * g.cap_hb + o;
+        if (to_slab) add_pieces(pieces, b, u, bytes);
+        else add_pieces(pieces, u, b, bytes);
     }
     pool_run(pieces.data(), (int)pieces.size());
 }
@@ -694,9 +721,10 @@ int resolve_init()
     return init_checks(g.pend_lsrad, st, g.pend_Ni, g.pend_Nj);
 }
 
-// stats_fast_kernel + stats_fix_kernel + stats_final on stream s; the 64-double vector lands in `d_out` (device memory)
-int launch_local_stats(long long n, const double *sst, const double *t_zt, const double *hum, const double *U,
-                       const double *V, const double *slp, const double *rad_lw, cudaStream_t s, double *d_out)
+// stats_fast_kernel + stats_fix_kernel + stats_final (their *_io_kernel<float> twins for es == sizeof(float)) on stream
+// s; the 64-double vector lands in `d_out` (device memory)
+int launch_local_stats(long long n, size_t es, const void *sst, const void *t_zt, const void *hum, const void *U,
+                       const void *V, const void *slp, const void *rad_lw, cudaStream_t s, double *d_out)
 {
     abk::StatsArgs a;
     a.sst = sst; a.t_zt = t_zt; a.hum_zt = hum; a.U_zu = U; a.V_zu = V; a.slp = slp; a.rad_lw = rad_lw;
@@ -705,14 +733,14 @@ int launch_local_stats(long long n, const double *sst, const double *t_zt, const
     a.out = d_out;
     long long want = (n + 255) / 256;
     int nblocks = (int)(want < 1 ? 1 : (want > abk::stats_max_blocks() ? abk::stats_max_blocks() : want));
-    CUDA_TRY(abk::launch_stats(a, nblocks, s));
+    CUDA_TRY(abk::launch_stats(es, a, nblocks, s));
     g.launches += 3;   // stats_fast_kernel, stats_fix_kernel, stats_final
     return 0;
 }
-int local_stats(long long n, const double *sst, const double *t_zt, const double *hum, const double *U,
-                const double *V, const double *slp, const double *rad_lw, cudaStream_t s, double *host_stats)
+int local_stats(long long n, size_t es, const void *sst, const void *t_zt, const void *hum, const void *U,
+                const void *V, const void *slp, const void *rad_lw, cudaStream_t s, double *host_stats)
 {
-    const int rc = launch_local_stats(n, sst, t_zt, hum, U, V, slp, rad_lw, s, g.d_stats);
+    const int rc = launch_local_stats(n, es, sst, t_zt, hum, U, V, slp, rad_lw, s, g.d_stats);
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(host_stats, g.d_stats, sizeof(double) * abk::NSTATS, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
@@ -744,8 +772,24 @@ abd::Uniform make_uniform(double zt, double zu)
     return u;
 }
 
-// reports a wind stress > 10 N/m^2 found by earlier launches (mod_phymbl.f90:1250-1253)
-int check_bad_flag(const double *h_taux, const double *h_tauy)
+// element i of an array of es-byte elements, widened to double; `on_device`: p is device memory (false on a failed copy)
+bool read_elem(const void *p, long long i, size_t es, bool on_device, double *v)
+{
+    const char *q = static_cast<const char *>(p) + i * (long long)es;
+    float f = 0.f;
+    void *dst = es == sizeof(float) ? static_cast<void *>(&f) : static_cast<void *>(v);
+    if (on_device) {
+        if (cudaMemcpy(dst, q, es, cudaMemcpyDeviceToHost) != cudaSuccess) return false;
+    } else {
+        memcpy(dst, q, es);
+    }
+    if (es == sizeof(float)) *v = f;
+    return true;
+}
+
+// reports a wind stress > 10 N/m^2 found by earlier launches (mod_phymbl.f90:1250-1253); h_taux / h_tauy: the host
+// output arrays of the last call (elements of g.last_es bytes), or NULL
+int check_bad_flag(const void *h_taux, const void *h_tauy)
 {
     if (!g.bad_pending) return 0;
     // the flag copy of an asynchronous device-pointer call may still be in flight (entry points that did not wait)
@@ -764,14 +808,11 @@ int check_bad_flag(const double *h_taux, const double *h_tauy)
     double tx = 0., ty = 0.;
     bool have_tau = false;
     if (h_taux && h_tauy) {
-        tx = h_taux[bad];
-        ty = h_tauy[bad];
-        have_tau = true;
+        have_tau = read_elem(h_taux, (long long)bad, g.last_es, false, &tx) && read_elem(h_tauy, (long long)bad, g.last_es, false, &ty);
     } else if (g.last_taux && g.last_tauy && flagged_launches == 1) {
         // the buffers of the ONE call the flag can come from; with several asynchronous calls behind the flag the
         // offending call (and its output arrays and shape) is not known any more and only the index is reported
-        have_tau = cudaMemcpy(&tx, g.last_taux + bad, sizeof(double), cudaMemcpyDeviceToHost) == cudaSuccess &&
-                   cudaMemcpy(&ty, g.last_tauy + bad, sizeof(double), cudaMemcpyDeviceToHost) == cudaSuccess;
+        have_tau = read_elem(g.last_taux, (long long)bad, g.last_es, true, &tx) && read_elem(g.last_tauy, (long long)bad, g.last_es, true, &ty);
     }
     if (have_tau)
         return fail(AEROBULK_GPU_ERR_TAU,
@@ -846,9 +887,9 @@ int plan_chunks(long long n, int kind, long long *cstart)
 // AEROBULK_MODEL (mod_aerobulk.f90:176-269) + aerobulk_compute dispatch
 // ---------------------------------------------------------------------------
 // the argument checks that come before any device work (:244), for one device and for a split call alike
-int check_model_args(int jt, const char *calgo, int Ni, int Nj, const double *sst, const double *t_zt, const double *hum_zt,
-                     const double *U_zu, const double *V_zu, const double *slp, const double *QL, const double *QH,
-                     const double *Tau_x, const double *Tau_y, const double *Evap)
+int check_model_args(int jt, const char *calgo, int Ni, int Nj, const void *sst, const void *t_zt, const void *hum_zt,
+                     const void *U_zu, const void *V_zu, const void *slp, const void *QL, const void *QH,
+                     const void *Tau_x, const void *Tau_y, const void *Evap)
 {
     g.errcode = 0;
     g.errmsg[0] = 0;
@@ -859,11 +900,14 @@ int check_model_args(int jt, const char *calgo, int Ni, int Nj, const double *ss
     return 0;
 }
 
-int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj,
-               const double *sst, const double *t_zt, const double *hum_zt, const double *U_zu,
-               const double *V_zu, const double *slp, double *QL, double *QH, double *Tau_x, double *Tau_y,
-               double *Evap, const int *Niter, const int *l_use_skin, const double *rad_sw,
-               const double *rad_lw, double *T_s)
+// `es`: bytes per element of every array of the call, sizeof(double) (aerobulk_gpu_model*) or sizeof(float)
+// (aerobulk_gpu_model*_f32).  Only the kernels (abk::ELEM_F64 / ELEM_F32) and the byte counts of the copies depend on it:
+// the transport path, the chunk plan, AEROBULK_INIT and the warm-layer state (always FP64) do not.
+int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj,
+               const void *sst, const void *t_zt, const void *hum_zt, const void *U_zu,
+               const void *V_zu, const void *slp, void *QL, void *QH, void *Tau_x, void *Tau_y,
+               void *Evap, const int *Niter, const int *l_use_skin, const void *rad_sw,
+               const void *rad_lw, void *T_s)
 {
     int rc = check_model_args(jt, calgo, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap);
     if (rc) return rc;
@@ -888,10 +932,14 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     }
 
     // rad_lw before rad_sw: a caller slab [sst .. slp, rad_lw] with a per-step rad_sw elsewhere is one run + one array
-    const double *in_h[8] = {sst, t_zt, hum_zt, U_zu, V_zu, slp, lsrad ? rad_lw : nullptr, lsrad ? rad_sw : nullptr};
-    double *out_h[6] = {QL, QH, Tau_x, Tau_y, Evap, lsrad ? T_s : nullptr};
-    const double *in_d[8] = {};   // what the kernels read and write
-    double *out_d[6] = {};
+    auto in_p = [](const void *p) { return static_cast<const char *>(p); };
+    auto out_p = [](void *p) { return static_cast<char *>(p); };
+    const char *in_h[8] = {in_p(sst), in_p(t_zt), in_p(hum_zt), in_p(U_zu), in_p(V_zu), in_p(slp),
+                           lsrad ? in_p(rad_lw) : nullptr, lsrad ? in_p(rad_sw) : nullptr};
+    char *out_h[6] = {out_p(QL), out_p(QH), out_p(Tau_x), out_p(Tau_y), out_p(Evap), lsrad ? out_p(T_s) : nullptr};
+    const char *in_d[8] = {};   // what the kernels read and write
+    char *out_d[6] = {};
+    const long long row = n * (long long)es;   // bytes per field
 
     // How the arrays reach the kernel, chosen once per call, in this order:
     //   DEVICE  device pointers (aerobulk_gpu_model_device): one launch on them;
@@ -912,15 +960,15 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
         for (int k = 0; k < 8; ++k)
             if (in_h[k] && !(in_d[k] = device_alias(in_h[k]))) return false;
         for (int k = 0; k < 6; ++k)
-            if (out_h[k] && !(out_d[k] = const_cast<double *>(device_alias(out_h[k])))) return false;
+            if (out_h[k] && !(out_d[k] = device_alias(out_h[k]))) return false;
         return true;
     };
     bool slab_first = false;
     if (!device_ptrs && init_stats) {
-        slab_first = slab_ok && !alias_all() && ensure_bounce(n);
+        slab_first = slab_ok && !alias_all() && ensure_bounce(row);
     } else if (!device_ptrs) {
         if (n > 0 && zerocopy_on() && alias_all()) path = ALIAS;
-        else if (slab_ok && ensure_bounce(n)) path = BOUNCE;
+        else if (slab_ok && ensure_bounce(row)) path = BOUNCE;
     }
     long long cstart[MAX_CHUNKS + 1];
     const int nchunks = plan_chunks(n, path == BOUNCE ? 2 : path == STAGED ? (init_stats ? 3 : 1) : 0, cstart);
@@ -935,10 +983,10 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     const bool spec_init = path == STAGED && init_stats && nchunks >= 2;
 
     // through the slab: the caller's arrays move to user_in / user_out, in_h / out_h name the slab rows
-    double *user_in[8] = {}, *user_out[6] = {};
+    char *user_in[8] = {}, *user_out[6] = {};
     if (slab_first || path == BOUNCE) {
         for (int k = 0; k < 8; ++k) {
-            user_in[k] = const_cast<double *>(in_h[k]);
+            user_in[k] = const_cast<char *>(in_h[k]);
             in_h[k] = in_h[k] ? g.hb + (long long)k * g.cap_hb : nullptr;
         }
         for (int k = 0; k < 6; ++k) {
@@ -947,7 +995,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
         }
     }
     if (path == STAGED) {
-        rc = ensure_staging(n);
+        rc = ensure_staging(row);
         if (rc) return rc;
     }
     for (int k = 0; k < 8; ++k) {
@@ -961,13 +1009,13 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
         else if (path == STAGED) out_d[k] = g.d_out[k];
     }
 
-    if (slab_first && !spec_init) bounce_copy(8, user_in, 0, 0, n, true);
+    if (slab_first && !spec_init) bounce_copy(8, user_in, 0, 0, n, es, true);
     // H2D of chunk c on the copy-in stream (preceded by its way into the slab on the copy threads where that applies)
     auto enqueue_h2d = [&](int c) -> int {
         const long long s0 = cstart[c], len = cstart[c + 1] - s0;
         if (len > 0 && path == STAGED) {
-            if (slab_first && spec_init) bounce_copy(8, user_in, 0, s0, len, true);
-            const int r = copy_fields(8, g.d_in, const_cast<double *const *>(in_h), g.cap, s0, len, true, g.in_stream);
+            if (slab_first && spec_init) bounce_copy(8, user_in, 0, s0, len, es, true);
+            const int r = copy_fields(8, g.d_in, const_cast<char *const *>(in_h), g.cap, s0, len, es, true, g.in_stream);
             if (r) return r;
         }
         CUDA_TRY(cudaEventRecord(g.ev_in[c], g.in_stream));
@@ -997,14 +1045,14 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
             if (device_ptrs && !g.verbose && !g.stats_hook && n > 0) {
                 // device-resident session, banners off: no host round trip -- the statistics stay on the device, are judged
                 // there, and the flux kernel reads the verdict from device memory (init_async / resolve_init)
-                rc = launch_local_stats(n, in_d[0], in_d[1], in_d[2], in_d[3], in_d[4], in_d[5], lsrad ? in_d[6] : nullptr, cs, g.d_stats);
+                rc = launch_local_stats(n, es, in_d[0], in_d[1], in_d[2], in_d[3], in_d[4], in_d[5], lsrad ? in_d[6] : nullptr, cs, g.d_stats);
                 if (rc) return rc;
                 rc = init_async(Nt, calgo, lskin, lsrad, g.d_stats, 1, Ni, Nj, cs);
                 if (rc) return rc;
             } else {
             if (n > 0) {
                 // :248 -- prsw=rad_lw: rad_lw is checked against both radiation ranges, rad_sw never
-                rc = local_stats(n, in_d[0], in_d[1], in_d[2], in_d[3], in_d[4], in_d[5], lsrad ? in_d[6] : nullptr, cs, st);
+                rc = local_stats(n, es, in_d[0], in_d[1], in_d[2], in_d[3], in_d[4], in_d[5], lsrad ? in_d[6] : nullptr, cs, st);
                 if (rc) return rc;
             } else {
                 memset(st, 0, sizeof(st));
@@ -1070,20 +1118,20 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     // array and of the warm-layer state; `timed`: the flux launch between a pair of aerobulk_gpu_set_kernel_timing events
     auto launch_chunk = [&](int c, bool timed) -> int {
         const long long s0 = cstart[c];
-        a.sst = in_d[0] + s0; a.t_zt = in_d[1] + s0; a.hum_zt = in_d[2] + s0;
-        a.U_zu = in_d[3] + s0; a.V_zu = in_d[4] + s0; a.slp = in_d[5] + s0;
-        a.rad_lw = in_d[6] ? in_d[6] + s0 : nullptr;
-        a.rad_sw = in_d[7] ? in_d[7] + s0 : nullptr;
-        a.QL = out_d[0] + s0; a.QH = out_d[1] + s0; a.Tau_x = out_d[2] + s0; a.Tau_y = out_d[3] + s0;
-        a.Evap = out_d[4] + s0;
-        a.T_s = out_d[5] ? out_d[5] + s0 : nullptr;
+        a.sst = elem_at(in_d[0], s0, es); a.t_zt = elem_at(in_d[1], s0, es); a.hum_zt = elem_at(in_d[2], s0, es);
+        a.U_zu = elem_at(in_d[3], s0, es); a.V_zu = elem_at(in_d[4], s0, es); a.slp = elem_at(in_d[5], s0, es);
+        a.rad_lw = elem_at(in_d[6], s0, es);
+        a.rad_sw = elem_at(in_d[7], s0, es);
+        a.QL = elem_at(out_d[0], s0, es); a.QH = elem_at(out_d[1], s0, es); a.Tau_x = elem_at(out_d[2], s0, es);
+        a.Tau_y = elem_at(out_d[3], s0, es); a.Evap = elem_at(out_d[4], s0, es);
+        a.T_s = elem_at(out_d[5], s0, es);
         if (use_skin) bind_wl_state(a, ialgo, s0);
         a.n = cstart[c + 1] - s0;
         a.index_offset = s0;
         a.perm = nullptr;
         if (do_sort) {
             unsigned short *perm = g.d_perm + s0 + (long long)c * abk::sort_window();
-            CUDA_TRY(abk::launch_classify(a, perm, use_skin, cs));
+            CUDA_TRY(abk::launch_classify(es, a, perm, use_skin, cs));
             g.launches += 1;
             a.perm = perm;
         }
@@ -1101,7 +1149,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
             g.kt_used += 2;
             CUDA_TRY(cudaEventRecord(kt0, cs));
         }
-        CUDA_TRY(abk::launch_flux(ialgo, use_skin, zteq, a, cs));
+        CUDA_TRY(abk::launch_flux(ialgo, use_skin, zteq, es, a, cs));
         g.launches += 1;
         if (kt1) CUDA_TRY(cudaEventRecord(kt1, cs));
         return 0;
@@ -1111,7 +1159,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
         CUDA_TRY(cudaEventRecord(g.ev_k[c], cs));
         CUDA_TRY(cudaStreamWaitEvent(g.out_stream, g.ev_k[c], 0));
         if (path != STAGED) return 0;
-        return copy_fields(6, g.d_out, out_h, g.cap, cstart[c], cstart[c + 1] - cstart[c], false, g.out_stream);
+        return copy_fields(6, g.d_out, out_h, g.cap, cstart[c], cstart[c + 1] - cstart[c], es, false, g.out_stream);
     };
 
     int launched[MAX_CHUNKS], n_launched = 0, n_home = 0;
@@ -1119,15 +1167,16 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     for (int c = 0; c < nchunks; ++c) {
         const long long s0 = cstart[c], len = cstart[c + 1] - s0;
         if (len <= 0) continue;
-        if (path == BOUNCE) bounce_copy(8, user_in, 0, s0, len, true);
+        if (path == BOUNCE) bounce_copy(8, user_in, 0, s0, len, es, true);
         while (slab_first && spec_init && h2d_next <= c) {   // (normally enqueued one iteration ahead, below)
             rc = enqueue_h2d(h2d_next++);
             if (rc) return rc;
         }
         if (!device_ptrs) CUDA_TRY(cudaStreamWaitEvent(cs, g.ev_in[c], 0));
         if (spec_init) {
-            rc = launch_local_stats(len, in_d[0] + s0, in_d[1] + s0, in_d[2] + s0, in_d[3] + s0, in_d[4] + s0, in_d[5] + s0,
-                                    lsrad ? in_d[6] + s0 : nullptr, cs, g.d_cstats + (long long)c * abk::NSTATS);
+            rc = launch_local_stats(len, es, elem_at(in_d[0], s0, es), elem_at(in_d[1], s0, es), elem_at(in_d[2], s0, es),
+                                    elem_at(in_d[3], s0, es), elem_at(in_d[4], s0, es), elem_at(in_d[5], s0, es),
+                                    lsrad ? elem_at(in_d[6], s0, es) : nullptr, cs, g.d_cstats + (long long)c * abk::NSTATS);
             if (rc) return rc;
             CUDA_TRY(abk::launch_init_decide(g.d_cstats, c + 1, lsrad ? 1 : 0, g.d_cgstats + (long long)c * abk::NSTATS,
                                              g.d_cinit + 2 * c, cs));
@@ -1150,7 +1199,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
             // ... and the chunks whose results have landed in the slab go home
             while (n_home < n_launched && cudaEventQuery(g.ev_out[launched[n_home]]) == cudaSuccess) {
                 const int h = launched[n_home++];
-                bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], false);
+                bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], es, false);
                 home[h] = true;
             }
         }
@@ -1159,7 +1208,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
             if (n_launched - n_home > 2) {
                 const int h = launched[n_home++];
                 CUDA_TRY(cudaEventSynchronize(g.ev_k[h]));
-                bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], false);
+                bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], es, false);
             }
         }
     }
@@ -1194,7 +1243,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     while (path == BOUNCE && n_home < n_launched) {
         const int h = launched[n_home++];
         CUDA_TRY(cudaEventSynchronize(g.ev_k[h]));
-        bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], false);
+        bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], es, false);
     }
     CUDA_TRY(cudaMemcpyAsync(g.h_bad, g.d_bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, cs));
     CUDA_TRY(cudaEventRecord(g.ev_bad, cs));
@@ -1203,6 +1252,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
     g.last_Ni = Ni;
     g.last_taux = out_d[2];
     g.last_tauy = out_d[3];
+    g.last_es = es;
 
     const bool last = (jt == g.nitend);
     const bool never_sync = device_ptrs && g.async_device;   // the caller collects errors with aerobulk_gpu_synchronize()
@@ -1212,7 +1262,7 @@ int model_impl(bool device_ptrs, int jt, int Nt, const char *calgo, double zt, d
         if (slab_first) {   // what is not home yet (everything, without the chunk-wise feed)
             for (int c = 0; c < nchunks; ++c) {
                 const long long s0 = cstart[c], len = cstart[c + 1] - s0;
-                if (len > 0 && !home[c]) bounce_copy(6, user_out, 8, s0, len, false);
+                if (len > 0 && !home[c]) bounce_copy(6, user_out, 8, s0, len, es, false);
             }
         }
         rc = resolve_init();   // an asynchronous AEROBULK_INIT of this session reports first, as in the reference
@@ -1321,10 +1371,10 @@ int plan_shards(long long n, int nd_max, long long *start)
     return nd;
 }
 
-int model_multi(int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj, const double *sst,
-                const double *t_zt, const double *hum_zt, const double *U_zu, const double *V_zu, const double *slp,
-                double *QL, double *QH, double *Tau_x, double *Tau_y, double *Evap, const int *Niter,
-                const int *l_use_skin, const double *rad_sw, const double *rad_lw, double *T_s)
+int model_multi(size_t es, int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj, const void *sst,
+                const void *t_zt, const void *hum_zt, const void *U_zu, const void *V_zu, const void *slp,
+                void *QL, void *QH, void *Tau_x, void *Tau_y, void *Evap, const int *Niter,
+                const int *l_use_skin, const void *rad_sw, const void *rad_lw, void *T_s)
 {
     Session &s0 = sess[0];
     int rc = check_model_args(jt, calgo, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap);
@@ -1367,9 +1417,11 @@ int model_multi(int jt, int Nt, const char *calgo, double zt, double zu, int Ni,
         sd.stats_hook = need_stats ? &hook : nullptr;
         const long long o = start[d];
         const int len = (int)(start[d + 1] - o);
-        rcs[d] = model_impl(false, jt, Nt, calgo, zt, zu, len, 1, sst + o, t_zt + o, hum_zt + o, U_zu + o, V_zu + o, slp + o,
-                            QL + o, QH + o, Tau_x + o, Tau_y + o, Evap + o, Niter, l_use_skin, rad_sw ? rad_sw + o : nullptr,
-                            rad_lw ? rad_lw + o : nullptr, T_s ? T_s + o : nullptr);
+        auto in = [&](const void *p) { return elem_at(static_cast<const char *>(p), o, es); };
+        auto out = [&](void *p) { return elem_at(static_cast<char *>(p), o, es); };
+        rcs[d] = model_impl(false, es, jt, Nt, calgo, zt, zu, len, 1, in(sst), in(t_zt), in(hum_zt), in(U_zu), in(V_zu), in(slp),
+                            out(QL), out(QH), out(Tau_x), out(Tau_y), out(Evap), Niter, l_use_skin, in(rad_sw), in(rad_lw),
+                            out(T_s));
         if (need_stats && rcs[d]) hook.combine(d, nullptr, false, nullptr);   // failed before the rendezvous: release the others
         sd.stats_hook = nullptr;
     });
@@ -1408,21 +1460,34 @@ void end_session_after_error(int jt, bool skin_before)
 }
 
 // host-array AEROBULK_MODEL: one device, or split over aerobulk_gpu_set_devices(n) of them
-int model_host(int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj, const double *sst,
-               const double *t_zt, const double *hum_zt, const double *U_zu, const double *V_zu, const double *slp,
-               double *QL, double *QH, double *Tau_x, double *Tau_y, double *Evap, const int *Niter,
-               const int *l_use_skin, const double *rad_sw, const double *rad_lw, double *T_s)
+int model_host(size_t es, int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj, const void *sst,
+               const void *t_zt, const void *hum_zt, const void *U_zu, const void *V_zu, const void *slp,
+               void *QL, void *QH, void *Tau_x, void *Tau_y, void *Evap, const int *Niter,
+               const int *l_use_skin, const void *rad_sw, const void *rad_lw, void *T_s)
 {
     const bool skin_before = sess[0].l_use_skin_schemes;
     int rc;
     if (n_devices > 1) {
-        rc = model_multi(jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap,
+        rc = model_multi(es, jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap,
                          Niter, l_use_skin, rad_sw, rad_lw, T_s);
     } else {
         split_nd = 1;
-        rc = model_impl(false, jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap,
+        rc = model_impl(false, es, jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap,
                         Niter, l_use_skin, rad_sw, rad_lw, T_s);
     }
+    if (rc) end_session_after_error(jt, skin_before);
+    return rc;
+}
+
+// device-pointer AEROBULK_MODEL (one device)
+int model_device(size_t es, int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj, const void *sst,
+                 const void *t_zt, const void *hum_zt, const void *U_zu, const void *V_zu, const void *slp,
+                 void *QL, void *QH, void *Tau_x, void *Tau_y, void *Evap, const int *Niter,
+                 const int *l_use_skin, const void *rad_sw, const void *rad_lw, void *T_s)
+{
+    const bool skin_before = sess[0].l_use_skin_schemes;
+    const int rc = model_impl(true, es, jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x,
+                              Tau_y, Evap, Niter, l_use_skin, rad_sw, rad_lw, T_s);
     if (rc) end_session_after_error(jt, skin_before);
     return rc;
 }
@@ -1478,7 +1543,7 @@ struct HostTransport {
         if (!zerocopy_on()) return STAGED;
         bool pinned = true;
         for (Array &a : arrays)
-            if (a.host && !(a.dev = const_cast<double *>(device_alias(a.host)))) {
+            if (a.host && !(a.dev = device_alias(a.host))) {
                 pinned = false;
                 break;
             }
@@ -1494,8 +1559,8 @@ struct HostTransport {
         std::vector<CopyPiece> pieces;
         for (const Array &a : arrays)
             if (a.host && (to_slab ? a.in : a.home)) {
-                if (to_slab) add_pieces(pieces, g.hx + a.off, a.host, a.len);
-                else add_pieces(pieces, a.host, g.hx + a.off, a.len);
+                if (to_slab) add_pieces(pieces, g.hx + a.off, a.host, sizeof(double) * (size_t)a.len);
+                else add_pieces(pieces, a.host, g.hx + a.off, sizeof(double) * (size_t)a.len);
             }
         pool_run(pieces.data(), (int)pieces.size());
     }
@@ -2106,8 +2171,8 @@ int aerobulk_gpu_model(int jt, int Nt, const char *calgo, double zt, double zu, 
                        const int *Niter, const int *l_use_skin, const double *rad_sw, const double *rad_lw, double *T_s)
 {
     std::lock_guard<std::mutex> lk(g_mu);
-    return model_host(jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y,
-                      Evap, Niter, l_use_skin, rad_sw, rad_lw, T_s);
+    return model_host(sizeof(double), jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x,
+                      Tau_y, Evap, Niter, l_use_skin, rad_sw, rad_lw, T_s);
 }
 
 int aerobulk_gpu_model_device(int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj,
@@ -2117,11 +2182,29 @@ int aerobulk_gpu_model_device(int jt, int Nt, const char *calgo, double zt, doub
                               const double *rad_sw, const double *rad_lw, double *T_s)
 {
     std::lock_guard<std::mutex> lk(g_mu);
-    const bool skin_before = sess[0].l_use_skin_schemes;
-    const int rc = model_impl(true, jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y,
-                              Evap, Niter, l_use_skin, rad_sw, rad_lw, T_s);
-    if (rc) end_session_after_error(jt, skin_before);
-    return rc;
+    return model_device(sizeof(double), jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x,
+                        Tau_y, Evap, Niter, l_use_skin, rad_sw, rad_lw, T_s);
+}
+
+int aerobulk_gpu_model_f32(int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj, const float *sst,
+                           const float *t_zt, const float *hum_zt, const float *U_zu, const float *V_zu,
+                           const float *slp, float *QL, float *QH, float *Tau_x, float *Tau_y, float *Evap,
+                           const int *Niter, const int *l_use_skin, const float *rad_sw, const float *rad_lw, float *T_s)
+{
+    std::lock_guard<std::mutex> lk(g_mu);
+    return model_host(sizeof(float), jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x,
+                      Tau_y, Evap, Niter, l_use_skin, rad_sw, rad_lw, T_s);
+}
+
+int aerobulk_gpu_model_device_f32(int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj,
+                                  const float *sst, const float *t_zt, const float *hum_zt, const float *U_zu,
+                                  const float *V_zu, const float *slp, float *QL, float *QH, float *Tau_x,
+                                  float *Tau_y, float *Evap, const int *Niter, const int *l_use_skin,
+                                  const float *rad_sw, const float *rad_lw, float *T_s)
+{
+    std::lock_guard<std::mutex> lk(g_mu);
+    return model_device(sizeof(float), jt, Nt, calgo, zt, zu, Ni, Nj, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x,
+                        Tau_y, Evap, Niter, l_use_skin, rad_sw, rad_lw, T_s);
 }
 
 static void copy_algo(char *dst, size_t cap, const char *calgo, int l)
@@ -2144,7 +2227,7 @@ void aerobulk_cxx_skin(const int *jt, const int *Nt, const char *calgo, const do
     copy_algo(algo, sizeof(algo), calgo, *l);
     const int lskin = (*(const unsigned char *)l_skin) != 0;
     std::lock_guard<std::mutex> lk(g_mu);
-    model_host(*jt, *Nt, algo, *zt, *zu, *m, 1, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap,
+    model_host(sizeof(double), *jt, *Nt, algo, *zt, *zu, *m, 1, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap,
                Niter, &lskin, rad_sw, rad_lw, T_s);
 }
 
@@ -2156,7 +2239,7 @@ void aerobulk_cxx_no_skin(const int *jt, const int *Nt, const char *calgo, const
     char algo[64];
     copy_algo(algo, sizeof(algo), calgo, *l);
     std::lock_guard<std::mutex> lk(g_mu);
-    model_host(*jt, *Nt, algo, *zt, *zu, *m, 1, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap,
+    model_host(sizeof(double), *jt, *Nt, algo, *zt, *zu, *m, 1, sst, t_zt, hum_zt, U_zu, V_zu, slp, QL, QH, Tau_x, Tau_y, Evap,
                Niter, nullptr, nullptr, nullptr, nullptr);
 }
 
@@ -2243,8 +2326,8 @@ int aerobulk_gpu_selftest_host_copy(long long n, int rounds)
     for (int r = 0; r < rounds; ++r) {
         for (long long i = 0; i < n; ++i) src[(size_t)i] = (double)(i * 31 + r);
         std::vector<CopyPiece> there, back;
-        add_pieces(there, mid.data(), src.data(), n);
-        add_pieces(back, dst.data(), mid.data(), n);
+        add_pieces(there, mid.data(), src.data(), sizeof(double) * (size_t)n);
+        add_pieces(back, dst.data(), mid.data(), sizeof(double) * (size_t)n);
         copy_pool().run(there.data(), (int)there.size());
         copy_pool().run(back.data(), (int)back.size());
         bad += memcmp(src.data(), dst.data(), sizeof(double) * (size_t)n) != 0;
@@ -2353,7 +2436,7 @@ int aerobulk_gpu_init_local_stats(int Ni, int Nj, const double *sst, const doubl
         }
         return 0;
     }
-    return local_stats(n, sst, t_zt, hum_zt, U_zu, V_zu, slp, rad_lw, compute_stream(), stats);
+    return local_stats(n, sizeof(double), sst, t_zt, hum_zt, U_zu, V_zu, slp, rad_lw, compute_stream(), stats);
 }
 
 int aerobulk_gpu_stats_reduce_op(int i)
@@ -2395,13 +2478,13 @@ int aerobulk_gpu_init(int Nt, const char *calgo, int Ni, int Nj, const double *s
     double st[abk::NSTATS];
     memset(st, 0, sizeof(st));
     if (n > 0) {
-        rc = ensure_staging(n);
+        rc = ensure_staging(n * (long long)sizeof(double));
         if (rc) return rc;
         cudaStream_t cs = compute_stream();
         const double *h[7] = {sst, t_zt, hum_zt, U_zu, V_zu, slp, lsrad ? rad_lw : nullptr};
         for (int k = 0; k < 7; ++k)
             if (h[k]) CUDA_TRY(cudaMemcpyAsync(g.d_in[k], h[k], sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, cs));
-        rc = local_stats(n, g.d_in[0], g.d_in[1], g.d_in[2], g.d_in[3], g.d_in[4], g.d_in[5], lsrad ? g.d_in[6] : nullptr, cs, st);
+        rc = local_stats(n, sizeof(double), g.d_in[0], g.d_in[1], g.d_in[2], g.d_in[3], g.d_in[4], g.d_in[5], lsrad ? g.d_in[6] : nullptr, cs, st);
         if (rc) return rc;
     }
     const bool skin_before = g.l_use_skin_schemes;
@@ -2434,7 +2517,7 @@ int aerobulk_gpu_init_local_stats_device(int Ni, int Nj, const double *sst, cons
     if (n <= 0) return fail(AEROBULK_GPU_ERR_ARG, "init_local_stats_device: empty row block (give it the identity vector instead)");
     int rc = ensure_device();
     if (rc) return rc;
-    return launch_local_stats(n, sst, t_zt, hum_zt, U_zu, V_zu, slp, rad_lw, compute_stream(), d_stats);
+    return launch_local_stats(n, sizeof(double), sst, t_zt, hum_zt, U_zu, V_zu, slp, rad_lw, compute_stream(), d_stats);
 }
 
 int aerobulk_gpu_init_from_gathered_stats(int Nt, const char *calgo, const int *l_use_skin, int have_rad,

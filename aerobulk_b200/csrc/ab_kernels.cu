@@ -12,6 +12,11 @@
 //       (src/mod_aerobulk.f90:104-153): mask, per-field masked sum/min/max, raw min/max; init_decide_kernel judges them
 //       on the device (humidity type, unit checks) for asynchronous jt == 1 calls.
 //   dfma_peak_kernel             dependent-chain DFMA microbenchmark (FP64 roofline denominator).
+//   flux_io_kernel<T,ALGO,SKIN,ZTEQ>, classify_io_kernel<T>, stats_fast_io_kernel<T>, stats_fix_io_kernel<T>
+//       the same for per-point arrays of element type T (float: aerobulk_gpu_model*_f32): the body is shared, only the
+//       loads (widened exactly) and stores (rounded once to nearest) differ, and the arithmetic stays FP64.  The shared
+//       bodies take threadIdx.x from the kernel: read in a __device__ function it would lose the range the kernel's
+//       launch bounds give it, and the FP64 kernels' machine code would change.
 //
 // The path is FP64-pipe bound (no contraction -> no tensor cores): see DESIGN.md.
 #include "ab_kernels.cuh"
@@ -56,15 +61,25 @@ static constexpr int FLUX_BLOCK = AB_FLUX_BLOCK;
 #ifndef AB_SORT_BAND_NOQ
 #define AB_SORT_BAND_NOQ 1.0 // the same when the humidity is rh / dp (the proxy ignores it)
 #endif
+// Per-point arrays of element type T (FluxArgs, StatsArgs): `ld` widens to FP64 (exact for float), `st` rounds once to
+// nearest.  With T = double both are the plain load and store.
+template <class T>
+__device__ __forceinline__ double ld(const void *p, long long i) { return (double)__ldg(static_cast<const T *>(p) + i); }
+template <class T>
+__device__ __forceinline__ void st(void *p, long long i, double v) { static_cast<T *>(p)[i] = v; }
+template <>
+__device__ __forceinline__ void st<float>(void *p, long long i, double v) { static_cast<float *>(p)[i] = __double2float_rn(v); }
+
 // The proxy only groups points, so it runs in FP32 (FP32 pipe and MUFU, both idle in this FP64 path): the temperature
 // difference is taken in FP64 first (exact to 1e-13 K), the humidity correction 0.608 (T_a q - T_s q_s) ~ 1 K is good to
 // 1e-6 K in FP32 -- against a band of 0.15 K.  classify_kernel is then bound by its 34 bytes per point.
+template <class T>
 __device__ __forceinline__ float stability_proxy(const FluxArgs &a, int ihum, double skin_off, long long i)
 {
-    const double sst = __ldg(a.sst + i) + skin_off, ta = __ldg(a.t_zt + i) + RGAMMA_DRY * a.u.zt;
+    const double sst = ld<T>(a.sst, i) + skin_off, ta = ld<T>(a.t_zt, i) + RGAMMA_DRY * a.u.zt;
     const float d0 = (float)(ta - sst);
     if (ihum != 0) return d0;
-    const float q = (float)__ldg(a.hum_zt + i), p = (float)__ldg(a.slp + i);
+    const float q = (float)ld<T>(a.hum_zt, i), p = (float)ld<T>(a.slp, i);
     const float tc = (float)(sst - 273.15);
     const float es = 611.2f * __expf(17.67f * tc * __frcp_rn(tc + 243.5f));     // Magnus
     const float qs = 0.98f * 0.622f * es * __frcp_rn(p - 0.378f * es);
@@ -86,13 +101,14 @@ static constexpr int SORT_BLOCK = 256;
 static constexpr int SORT_ITEMS = SORT_WIN / SORT_BLOCK;
 static constexpr int SORT_CLASSES = 3;
 
-__global__ void __launch_bounds__(SORT_BLOCK) classify_kernel(const FluxArgs a, unsigned short *perm, int skin)
+template <class T>
+__device__ __forceinline__ void classify_block(const FluxArgs &a, unsigned short *perm, int skin, int tid)
 {
     constexpr int NW = SORT_BLOCK / 32, NG = SORT_ITEMS * NW;
     __shared__ unsigned short s_c[SORT_CLASSES][NG], s_off[SORT_CLASSES][NG];
     __shared__ int s_tot[SORT_CLASSES];
     const long long base = (long long)blockIdx.x * SORT_WIN;
-    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    const int lane = tid & 31, w = tid >> 5;
     const int ihum = a.init_dev ? __ldg(a.init_dev) : a.ihum;
     const float band = (ihum != 0) ? (float)AB_SORT_BAND_NOQ : (skin ? (float)AB_SORT_BAND_SKIN : (float)AB_SORT_BAND);
     const bool wl = skin && !a.first_step && a.dT_wl != nullptr;
@@ -103,7 +119,7 @@ __global__ void __launch_bounds__(SORT_BLOCK) classify_kernel(const FluxArgs a, 
         cls[k] = SORT_CLASSES;   // padding beyond n
         if (i < a.n) {
             const double off = skin ? (-0.25 + (wl ? a.dT_wl[i] : 0.)) : 0.;
-            const float d = stability_proxy(a, ihum, off, i);
+            const float d = stability_proxy<T>(a, ihum, off, i);
             cls[k] = (d >= band) ? 0 : (d > -band) ? 1 : 2;
         }
     }
@@ -159,6 +175,18 @@ __global__ void __launch_bounds__(SORT_BLOCK) classify_kernel(const FluxArgs a, 
     }
 }
 
+__global__ void __launch_bounds__(SORT_BLOCK) classify_kernel(const FluxArgs a, unsigned short *perm, int skin)
+{
+    classify_block<double>(a, perm, skin, threadIdx.x);
+}
+
+// the same for arrays of element type T
+template <class T>
+__global__ void __launch_bounds__(SORT_BLOCK) classify_io_kernel(const FluxArgs a, unsigned short *perm, int skin)
+{
+    classify_block<T>(a, perm, skin, threadIdx.x);
+}
+
 // warm-layer state of point i at the start of a step (*_INIT values at kt == nit000), and its write-back
 template <int ALGO, class Args>
 __device__ __forceinline__ void load_warm_layer(const Args &a, long long i, WarmLayer &wl)
@@ -186,11 +214,12 @@ __device__ __forceinline__ void store_warm_layer(const Args &a, long long i, con
     }
 }
 
-template <int ALGO, bool SKIN, bool ZTEQ>
-__global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOCKS_NOSKIN) flux_kernel(const FluxArgs a)
+// one thread's point of flux_kernel (T = double) and flux_io_kernel<T>: only the loads and stores depend on T
+template <class T, int ALGO, bool SKIN, bool ZTEQ>
+__device__ __forceinline__ void flux_point(const FluxArgs &a, unsigned tid)
 {
     abm::load_tables();
-    long long i = (long long)blockIdx.x * FLUX_BLOCK + threadIdx.x;
+    long long i = (long long)blockIdx.x * FLUX_BLOCK + tid;
     if (a.perm) i = (i / SORT_WIN) * SORT_WIN + a.perm[i];   // slot -> point (perm is padded to whole windows)
     if (i >= a.n) return;
     int ihum = a.ihum;
@@ -200,12 +229,12 @@ __global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOC
     }
 
     // ---- coalesced loads of the 6 (8) input fields
-    const double sst = __ldg(a.sst + i);
-    const double t_air = __ldg(a.t_zt + i);
-    const double hum = __ldg(a.hum_zt + i);
-    const double U = __ldg(a.U_zu + i);
-    const double V = __ldg(a.V_zu + i);
-    const double slp = __ldg(a.slp + i);
+    const double sst = ld<T>(a.sst, i);
+    const double t_air = ld<T>(a.t_zt, i);
+    const double hum = ld<T>(a.hum_zt, i);
+    const double U = ld<T>(a.U_zu, i);
+    const double V = ld<T>(a.V_zu, i);
+    const double slp = ld<T>(a.slp, i);
 
     PointIn p;
     p.sst = sst;
@@ -225,8 +254,8 @@ __global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOC
 
     WarmLayer wl = {0., 0., 0., 0.};
     if (SKIN) {
-        p.Qsw = (1. - ROCE_ALB0) * __ldg(a.rad_sw + i);            // :135,:146,:161
-        p.rlw = __ldg(a.rad_lw + i);
+        p.Qsw = (1. - ROCE_ALB0) * ld<T>(a.rad_sw, i);             // :135,:146,:161
+        p.rlw = ld<T>(a.rad_lw, i);
         if (a.lon) {
             p.lon = __ldg(a.lon + i);
             p.has_lon = true;
@@ -248,22 +277,38 @@ __global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOC
         tx = s * U;
         ty = s * V;
     }
-    a.QL[i] = f.qlat;
-    a.QH[i] = f.qsen;
-    a.Tau_x[i] = tx;
-    a.Tau_y[i] = ty;
-    a.Evap[i] = f.evap;
-    if (a.T_s) a.T_s[i] = c.Ts;
+    st<T>(a.QL, i, f.qlat);
+    st<T>(a.QH, i, f.qsen);
+    st<T>(a.Tau_x, i, tx);
+    st<T>(a.Tau_y, i, ty);
+    st<T>(a.Evap, i, f.evap);
+    if (a.T_s) st<T>(a.T_s, i, c.Ts);
 }
 
-static auto flux_kernel_for(int algo, bool skin, bool zteq)
+template <int ALGO, bool SKIN, bool ZTEQ>
+__global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOCKS_NOSKIN) flux_kernel(const FluxArgs a)
 {
-    return pick_ocean(algo, skin, zteq, [](auto A, auto S, auto Z) { return flux_kernel<A(), S(), Z()>; });
+    flux_point<double, ALGO, SKIN, ZTEQ>(a, threadIdx.x);
 }
 
-cudaError_t launch_flux(int algo, bool skin, bool zteq, const FluxArgs &a, cudaStream_t s)
+// flux_kernel on per-point arrays of element type T, same launch bounds.  T is a type argument: the kernel-matrix
+// census of the FP64 kernels takes the instantiations whose template arguments are all int or bool.
+template <class T, int ALGO, bool SKIN, bool ZTEQ>
+__global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOCKS_NOSKIN) flux_io_kernel(const FluxArgs a)
 {
-    const auto k = flux_kernel_for(algo, skin, zteq);
+    flux_point<T, ALGO, SKIN, ZTEQ>(a, threadIdx.x);
+}
+
+static auto flux_kernel_for(int algo, bool skin, bool zteq, size_t elem = ELEM_F64)
+{
+    return pick_ocean(algo, skin, zteq, [elem](auto A, auto S, auto Z) {
+        return elem == ELEM_F64 ? flux_kernel<A(), S(), Z()> : elem == ELEM_F32 ? flux_io_kernel<float, A(), S(), Z()> : nullptr;
+    });
+}
+
+cudaError_t launch_flux(int algo, bool skin, bool zteq, size_t elem, const FluxArgs &a, cudaStream_t s)
+{
+    const auto k = flux_kernel_for(algo, skin, zteq, elem);
     if (!k) return cudaErrorInvalidValue;
     if (a.n <= 0) return cudaSuccess;
     const long long span = a.perm ? (a.n + SORT_WIN - 1) / SORT_WIN * SORT_WIN : a.n;   // whole windows of slots
@@ -342,11 +387,13 @@ int flux_block_size() { return FLUX_BLOCK; }
 
 int sort_window() { return SORT_WIN; }
 
-cudaError_t launch_classify(const FluxArgs &a, unsigned short *perm, bool skin, cudaStream_t s)
+cudaError_t launch_classify(size_t elem, const FluxArgs &a, unsigned short *perm, bool skin, cudaStream_t s)
 {
+    const auto k = elem == ELEM_F64 ? classify_kernel : elem == ELEM_F32 ? classify_io_kernel<float> : nullptr;
+    if (!k) return cudaErrorInvalidValue;
     if (a.n <= 0) return cudaSuccess;
     const long long nwin = (a.n + SORT_WIN - 1) / SORT_WIN;
-    classify_kernel<<<(unsigned)nwin, SORT_BLOCK, 0, s>>>(a, perm, skin ? 1 : 0);
+    k<<<(unsigned)nwin, SORT_BLOCK, 0, s>>>(a, perm, skin ? 1 : 0);
     return cudaGetLastError();
 }
 
@@ -409,7 +456,7 @@ static constexpr int STATS_REDO_SLOT = NSTATS - 1;
 // same order: the row is bit-identical to what the one-kernel version produced).  NaNs: `x < lo || x > hi` is false for a
 // NaN (the reference does not mask it) and the (v < acc ? v : acc) min / max skip it -- the derived test agrees.
 // rad_lw is held against both radiation ranges (the reference's prsw=rad_lw slip): fields 7 and 8 are the same values.
-template <int UNROLL>
+template <class T, int UNROLL>
 __device__ __forceinline__ void stats_fast_body(const StatsArgs &a, double (&sum)[8], double (&mn)[8], double (&mx)[8], double &cnt)
 {
     const bool rad = (a.rad_lw != nullptr);
@@ -422,13 +469,13 @@ __device__ __forceinline__ void stats_fast_body(const StatsArgs &a, double (&sum
         for (int u = 0; u < UNROLL; ++u) {
             const long long i = i0 + u * stride;
             const long long j = (i < a.n) ? i : i0;
-            in[u][0] = __ldg(a.sst + j);
-            in[u][1] = __ldg(a.t_zt + j);
-            in[u][2] = __ldg(a.slp + j);
-            in[u][3] = __ldg(a.U_zu + j);
-            in[u][4] = __ldg(a.V_zu + j);
-            in[u][5] = __ldg(a.hum_zt + j);
-            in[u][6] = rad ? __ldg(a.rad_lw + j) : 0.;
+            in[u][0] = ld<T>(a.sst, j);
+            in[u][1] = ld<T>(a.t_zt, j);
+            in[u][2] = ld<T>(a.slp, j);
+            in[u][3] = ld<T>(a.U_zu, j);
+            in[u][4] = ld<T>(a.V_zu, j);
+            in[u][5] = ld<T>(a.hum_zt, j);
+            in[u][6] = rad ? ld<T>(a.rad_lw, j) : 0.;
         }
 #pragma unroll
         for (int u = 0; u < UNROLL; ++u) {
@@ -456,7 +503,8 @@ __device__ __forceinline__ void stats_fast_body(const StatsArgs &a, double (&sum
 #ifndef AB_STATS_UNROLL
 #define AB_STATS_UNROLL 3   // 120 registers, no spills, 2 blocks/SM x 21 loads in flight per thread
 #endif
-__global__ void __launch_bounds__(STATS_BLOCK, 2) stats_fast_kernel(const StatsArgs a)
+template <class T>
+__device__ __forceinline__ void stats_fast_block(const StatsArgs &a, unsigned tid)
 {
     double sum[8], mn[8], mx[8], cnt = 0.;
 #pragma unroll
@@ -465,10 +513,10 @@ __global__ void __launch_bounds__(STATS_BLOCK, 2) stats_fast_kernel(const StatsA
         mn[f] = DBL_MAX;
         mx[f] = -DBL_MAX;
     }
-    stats_fast_body<AB_STATS_UNROLL>(a, sum, mn, mx, cnt);   // a thread meets its points in the same order for any unroll
+    stats_fast_body<T, AB_STATS_UNROLL>(a, sum, mn, mx, cnt);   // a thread meets its points in the same order for any unroll
     // block reduction in the order of the one-kernel version: lanes by shuffle, then the warps in index order
     __shared__ double sm[STATS_BLOCK / 32][1 + 3 * 8];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     {
         const double r = warp_reduce(cnt, 0);
         if (lane == 0) sm[warp][0] = r;
@@ -484,15 +532,15 @@ __global__ void __launch_bounds__(STATS_BLOCK, 2) stats_fast_kernel(const StatsA
     }
     __syncthreads();
     double *row = a.partials + (long long)blockIdx.x * NSTATS;
-    if (threadIdx.x < 1 + 3 * 8) {
-        const int k = threadIdx.x, op = (k == 0) ? 0 : (k - 1) % 3;
+    if (tid < 1 + 3 * 8) {
+        const int k = tid, op = (k == 0) ? 0 : (k - 1) % 3;
         double r = sm[0][k];
         for (int w = 1; w < STATS_BLOCK / 32; ++w)
             r = (op == 0) ? r + sm[w][k] : (op == 1) ? fmin(r, sm[w][k]) : fmax(r, sm[w][k]);
         sm[0][k] = r;
     }
     __syncthreads();
-    if (threadIdx.x == 0) {
+    if (tid == 0) {
         const double *b = sm[0];
         const bool rad = (a.rad_lw != nullptr);
         // min / max of field f: b[2 + 3 f], b[3 + 3 f]; field order sst t_zt slp U V wnd hum rad_lw
@@ -512,8 +560,15 @@ __global__ void __launch_bounds__(STATS_BLOCK, 2) stats_fast_kernel(const StatsA
     }
 }
 
+__global__ void __launch_bounds__(STATS_BLOCK, 2) stats_fast_kernel(const StatsArgs a) { stats_fast_block<double>(a, threadIdx.x); }
+
+// the same for arrays of element type T
+template <class T>
+__global__ void __launch_bounds__(STATS_BLOCK, 2) stats_fast_io_kernel(const StatsArgs a) { stats_fast_block<T>(a, threadIdx.x); }
+
 // the full accumulator set (masked and raw statistics side by side), for the blocks stats_fast_kernel flagged
-__global__ void __launch_bounds__(STATS_BLOCK) stats_fix_kernel(const StatsArgs a)
+template <class T>
+__device__ __forceinline__ void stats_fix_block(const StatsArgs &a, unsigned tid)
 {
     if (a.partials[(long long)blockIdx.x * NSTATS + STATS_REDO_SLOT] == 0.) return;
     double acc[2 + 5 * NFIELDS];
@@ -532,20 +587,20 @@ __global__ void __launch_bounds__(STATS_BLOCK) stats_fix_kernel(const StatsArgs 
     // STATS_UNROLL points per trip with all their loads issued first: the pass is bound by memory latency, not by its
     // arithmetic (one point per trip ran at 1.5 TB/s: ~47 accumulators leave room for 2 blocks per SM only)
     constexpr int STATS_UNROLL = 4;
-    for (long long i0 = (long long)blockIdx.x * STATS_BLOCK + threadIdx.x; i0 < a.n; i0 += stride * STATS_UNROLL) {
+    for (long long i0 = (long long)blockIdx.x * STATS_BLOCK + tid; i0 < a.n; i0 += stride * STATS_UNROLL) {
         double in[STATS_UNROLL][7];
 #pragma unroll
         for (int u = 0; u < STATS_UNROLL; ++u) {
             const long long i = i0 + u * stride;
             const bool ok = i < a.n;
             const long long j = ok ? i : i0;
-            in[u][0] = __ldg(a.sst + j);
-            in[u][1] = __ldg(a.t_zt + j);
-            in[u][2] = __ldg(a.slp + j);
-            in[u][3] = __ldg(a.U_zu + j);
-            in[u][4] = __ldg(a.V_zu + j);
-            in[u][5] = __ldg(a.hum_zt + j);
-            in[u][6] = rad ? __ldg(a.rad_lw + j) : 0.;
+            in[u][0] = ld<T>(a.sst, j);
+            in[u][1] = ld<T>(a.t_zt, j);
+            in[u][2] = ld<T>(a.slp, j);
+            in[u][3] = ld<T>(a.U_zu, j);
+            in[u][4] = ld<T>(a.V_zu, j);
+            in[u][5] = ld<T>(a.hum_zt, j);
+            in[u][6] = rad ? ld<T>(a.rad_lw, j) : 0.;
         }
 #pragma unroll
         for (int u = 0; u < STATS_UNROLL; ++u) {
@@ -577,21 +632,26 @@ __global__ void __launch_bounds__(STATS_BLOCK) stats_fix_kernel(const StatsArgs 
         }
     }
     __shared__ double sm[STATS_BLOCK / 32][2 + 5 * NFIELDS];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
 #pragma unroll
     for (int k = 0; k < 2 + 5 * NFIELDS; ++k) {
         const double r = warp_reduce(acc[k], stat_op(k));
         if (lane == 0) sm[warp][k] = r;
     }
     __syncthreads();
-    if (threadIdx.x < 2 + 5 * NFIELDS) {
-        const int k = threadIdx.x, op = stat_op(k);
+    if (tid < 2 + 5 * NFIELDS) {
+        const int k = tid, op = stat_op(k);
         double r = sm[0][k];
         for (int w = 1; w < STATS_BLOCK / 32; ++w)
             r = (op == 0) ? r + sm[w][k] : (op == 1) ? fmin(r, sm[w][k]) : fmax(r, sm[w][k]);
         a.partials[(long long)blockIdx.x * NSTATS + k] = r;
     }
 }
+
+__global__ void __launch_bounds__(STATS_BLOCK) stats_fix_kernel(const StatsArgs a) { stats_fix_block<double>(a, threadIdx.x); }
+
+template <class T>
+__global__ void __launch_bounds__(STATS_BLOCK) stats_fix_io_kernel(const StatsArgs a) { stats_fix_block<T>(a, threadIdx.x); }
 
 // fixed-order final reduction (one block of 128 threads per statistic) -> results do not depend on scheduling
 static constexpr int FINAL_BLOCK = 128;
@@ -621,12 +681,15 @@ __global__ void __launch_bounds__(FINAL_BLOCK) stats_final(const double *partial
 
 int stats_max_blocks() { return STATS_MAX_BLOCKS; }
 
-cudaError_t launch_stats(const StatsArgs &a, int nblocks, cudaStream_t s)
+cudaError_t launch_stats(size_t elem, const StatsArgs &a, int nblocks, cudaStream_t s)
 {
-    stats_fast_kernel<<<nblocks, STATS_BLOCK, 0, s>>>(a);
+    const auto fast = elem == ELEM_F64 ? stats_fast_kernel : elem == ELEM_F32 ? stats_fast_io_kernel<float> : nullptr;
+    const auto fix = elem == ELEM_F64 ? stats_fix_kernel : elem == ELEM_F32 ? stats_fix_io_kernel<float> : nullptr;
+    if (!fast) return cudaErrorInvalidValue;
+    fast<<<nblocks, STATS_BLOCK, 0, s>>>(a);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    stats_fix_kernel<<<nblocks, STATS_BLOCK, 0, s>>>(a);   // returns at once in every block that holds no masked point
+    fix<<<nblocks, STATS_BLOCK, 0, s>>>(a);   // returns at once in every block that holds no masked point
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     stats_final<<<NSTATS, FINAL_BLOCK, 0, s>>>(a.partials, nblocks, a.out);

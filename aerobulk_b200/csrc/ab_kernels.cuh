@@ -30,15 +30,22 @@ auto pick_ocean(int algo, bool skin, bool zteq, F f) -> decltype(f(IntC<abd::NCA
     }
 }
 
+// Element type of the caller's per-point arrays in one aerobulk_model launch, given by its size in bytes:
+// sizeof(double) runs the FP64 kernels (flux_kernel, classify_kernel, stats_*_kernel); sizeof(float) runs their
+// *_io_kernel<float> twins, which widen every input exactly on load, compute in FP64 with the same code, and round every
+// output once to nearest on store.  Anything else: cudaErrorInvalidValue.
+constexpr size_t ELEM_F64 = sizeof(double);
+constexpr size_t ELEM_F32 = sizeof(float);
+
 // One fused launch = reference aerobulk_compute (src/mod_aerobulk_compute.f90:22-213)
 // steps 1-9 for `n` consecutive grid points.
 struct FluxArgs {
-    // inputs (device)
-    const double *sst, *t_zt, *hum_zt, *U_zu, *V_zu, *slp;
-    const double *rad_sw, *rad_lw;   // skin only
+    // inputs (device), of the launch's element type
+    const void *sst, *t_zt, *hum_zt, *U_zu, *V_zu, *slp;
+    const void *rad_sw, *rad_lw;     // skin only
     const double *lon;               // optional longitudes [deg E]; NULL -> 0 (mod_aerobulk_compute.f90:126)
-    // outputs (device); T_s may be NULL
-    double *QL, *QH, *Tau_x, *Tau_y, *Evap, *T_s;
+    // outputs (device), of the launch's element type; T_s may be NULL
+    void *QL, *QH, *Tau_x, *Tau_y, *Evap, *T_s;
     // persistent warm-layer state (device); COARE: 4 arrays, ECMWF: dT_wl only
     double *dT_wl, *Hz_wl, *Qnt_ac, *Tau_ac;
     long long n;
@@ -139,7 +146,7 @@ constexpr int NSTATS = 64;
 constexpr int NFIELDS = 9;
 
 struct StatsArgs {
-    const double *sst, *t_zt, *hum_zt, *U_zu, *V_zu, *slp, *rad_lw;   // rad_lw may be NULL
+    const void *sst, *t_zt, *hum_zt, *U_zu, *V_zu, *slp, *rad_lw;   // of the launch's element type; rad_lw may be NULL
     long long n;
     double *partials;   // [gridDim.x][NSTATS]
     double *out;        // [NSTATS]
@@ -157,13 +164,14 @@ struct DiagArgs {
 };
 cudaError_t launch_diag(const DiagArgs &a, int nblocks, cudaStream_t s);
 
-cudaError_t launch_flux(int algo, bool skin, bool zt_eq_zu, const FluxArgs &a, cudaStream_t s);
+// `elem`: ELEM_F64 or ELEM_F32, the element type of the per-point arrays of `a`
+cudaError_t launch_flux(int algo, bool skin, bool zt_eq_zu, size_t elem, const FluxArgs &a, cudaStream_t s);
 // block size / register info for reports
 int flux_block_size();
 int sort_window();
 // fills perm[] (ceil(n / sort_window()) * sort_window() entries) for the launch described by `a`
-cudaError_t launch_classify(const FluxArgs &a, unsigned short *perm, bool skin, cudaStream_t s);
-cudaError_t launch_stats(const StatsArgs &a, int nblocks, cudaStream_t s);
+cudaError_t launch_classify(size_t elem, const FluxArgs &a, unsigned short *perm, bool skin, cudaStream_t s);
+cudaError_t launch_stats(size_t elem, const StatsArgs &a, int nblocks, cudaStream_t s);
 // AEROBULK_INIT's stats-dependent decisions on the device (src/mod_aerobulk.f90:104-153, src/mod_phymbl.f90:1851-2007):
 // combines the statistics vectors of `nranks` row blocks (all[r][NSTATS], rank order: deterministic) into gstats[NSTATS]
 // and writes init[0] = humidity type (0 'sh', 1 'dp', 2 'rh'), init[1] = 0 or the AEROBULK_GPU_ERR_* code the host will

@@ -38,7 +38,7 @@ def lib():
     L = C.CDLL(_SO)
     model_args = ([C.c_int, C.c_int, C.c_char_p, C.c_double, C.c_double, C.c_int, C.c_int] + [C.c_void_p] * 11 +
                   [_ip, _ip, C.c_void_p, C.c_void_p, C.c_void_p])
-    for name in ("aerobulk_gpu_model", "aerobulk_gpu_model_device"):
+    for name in ("aerobulk_gpu_model", "aerobulk_gpu_model_device", "aerobulk_gpu_model_f32", "aerobulk_gpu_model_device_f32"):
         f = getattr(L, name)
         f.restype = C.c_int
         f.argtypes = model_args
@@ -145,11 +145,25 @@ def _f64(a, shape=None):
     return a
 
 
-def _check_out(name, a, shape):
-    """A caller-supplied output array must be exactly what the library writes: float64, the grid's shape, column-major
+def _f32(a, shape=None):
+    """A float32 input of aerobulk_model_f32 in the layout of _f64; any other dtype is refused, never cast."""
+    if not isinstance(a, np.ndarray) or a.dtype != np.float32:
+        raise AerobulkError(101, f"aerobulk_model_f32 needs float32 numpy arrays, got {getattr(a, 'dtype', type(a).__name__)}")
+    if a.ndim >= 2:
+        if not a.flags.f_contiguous:
+            a = np.asfortranarray(a)
+    elif not a.flags.c_contiguous:
+        a = np.ascontiguousarray(a)
+    if shape is not None and a.shape != shape:
+        raise AerobulkError(101, f"AEROBULK_INIT => arrays do not agree in shape: {a.shape} vs {shape}")
+    return a
+
+
+def _check_out(name, a, shape, dtype=np.float64):
+    """A caller-supplied output array must be exactly what the library writes: `dtype`, the grid's shape, column-major
     (2-D) or contiguous (1-D), writeable -- anything else would silently pair different grid points across fields."""
-    if not isinstance(a, np.ndarray) or a.dtype != np.float64:
-        raise AerobulkError(101, f"out['{name}'] must be a float64 numpy array")
+    if not isinstance(a, np.ndarray) or a.dtype != dtype:
+        raise AerobulkError(101, f"out['{name}'] must be a {np.dtype(dtype).name} numpy array")
     if a.shape != shape:
         raise AerobulkError(101, f"out['{name}'] has shape {a.shape}, the fields have {shape}")
     if not (a.flags.f_contiguous if a.ndim >= 2 else a.flags.c_contiguous):
@@ -175,26 +189,44 @@ def aerobulk_model(jt: int, Nt: int, calgo: str, zt: float, zu: float, sst, t_zt
     Returns {"QL","QH","Tau_x","Tau_y","Evap"[,"T_s"]}; T_s is present iff rad_sw and rad_lw
     are given (mod_aerobulk.f90:246-253).  `out` may hold preallocated (e.g. pinned) arrays.
     """
-    L = lib()
-    sst = _f64(sst)
+    return _model_host(lib().aerobulk_gpu_model, _f64, np.float64, jt, Nt, calgo, zt, zu,
+                       (sst, t_zt, hum_zt, U_zu, V_zu, slp), Niter, l_use_skin, rad_sw, rad_lw, out)
+
+
+def aerobulk_model_f32(jt: int, Nt: int, calgo: str, zt: float, zu: float, sst, t_zt, hum_zt, U_zu, V_zu, slp,
+                       Niter: Optional[int] = None, l_use_skin: Optional[bool] = None, rad_sw=None, rad_lw=None,
+                       out: Optional[dict] = None) -> dict:
+    """:func:`aerobulk_model` on float32 numpy arrays (Fortran order), returning float32 arrays.
+
+    Every output is the FP64 call on the exactly widened inputs, rounded once to nearest: bit for bit
+    ``aerobulk_model(..., x.astype(float64), ...)[k].astype(float32)``.  The warm-layer state stays FP64 on the device,
+    so float32 and float64 calls may alternate within one session.  Arrays of any other dtype raise
+    AerobulkError(101); nothing is cast.  `out` may hold preallocated (e.g. pinned) float32 arrays.
+    """
+    return _model_host(lib().aerobulk_gpu_model_f32, _f32, np.float32, jt, Nt, calgo, zt, zu,
+                       (sst, t_zt, hum_zt, U_zu, V_zu, slp), Niter, l_use_skin, rad_sw, rad_lw, out)
+
+
+def _model_host(fn, prep, dtype, jt, Nt, calgo, zt, zu, fields, Niter, l_use_skin, rad_sw, rad_lw, out):
+    sst = prep(fields[0])
     shape = sst.shape
     Ni, Nj = _shape2(shape)
-    ins = [sst] + [_f64(a, shape) for a in (t_zt, hum_zt, U_zu, V_zu, slp)]
-    rs = None if rad_sw is None else _f64(rad_sw, shape)
-    rl = None if rad_lw is None else _f64(rad_lw, shape)
+    ins = [sst] + [prep(a, shape) for a in fields[1:]]
+    rs = None if rad_sw is None else prep(rad_sw, shape)
+    rl = None if rad_lw is None else prep(rad_lw, shape)
     names = ["QL", "QH", "Tau_x", "Tau_y", "Evap"] + (["T_s"] if (rs is not None and rl is not None) else [])
     res = {}
     for k in names:
         if out is not None and k in out:
-            res[k] = _check_out(k, out[k], shape)
+            res[k] = _check_out(k, out[k], shape, dtype)
         else:
-            res[k] = np.empty(shape, dtype=np.float64, order="F")
+            res[k] = np.empty(shape, dtype=dtype, order="F")
     ni = None if Niter is None else C.byref(C.c_int(int(Niter)))
     ls = None if l_use_skin is None else C.byref(C.c_int(int(bool(l_use_skin))))
     ptr = lambda a: None if a is None else a.ctypes.data
-    rc = L.aerobulk_gpu_model(int(jt), int(Nt), calgo.encode(), float(zt), float(zu), Ni, Nj,
-                              *[ptr(a) for a in ins], *[ptr(res[k]) for k in names[:5]],
-                              ni, ls, ptr(rs), ptr(rl), ptr(res.get("T_s")))
+    rc = fn(int(jt), int(Nt), calgo.encode(), float(zt), float(zu), Ni, Nj,
+            *[ptr(a) for a in ins], *[ptr(res[k]) for k in names[:5]],
+            ni, ls, ptr(rs), ptr(rl), ptr(res.get("T_s")))
     _check(rc)
     return res
 
@@ -209,22 +241,35 @@ def aerobulk_model_device(jt: int, Nt: int, calgo: str, zt: float, zu: float, ss
     grid (default (numel,1)).  The launch goes to the stream set by :func:`set_stream`
     (default: the library's own).
     """
-    L = lib()
-    tensors = [sst, t_zt, hum_zt, U_zu, V_zu, slp]
-    n = sst.numel()
+    return _model_device(lib().aerobulk_gpu_model_device, "float64", jt, Nt, calgo, zt, zu,
+                         (sst, t_zt, hum_zt, U_zu, V_zu, slp), out, Niter, l_use_skin, rad_sw, rad_lw, shape)
+
+
+def aerobulk_model_device_f32(jt: int, Nt: int, calgo: str, zt: float, zu: float, sst, t_zt, hum_zt, U_zu, V_zu, slp,
+                              out: dict, Niter: Optional[int] = None, l_use_skin: Optional[bool] = None,
+                              rad_sw=None, rad_lw=None, shape=None) -> dict:
+    """:func:`aerobulk_model_device` on contiguous torch.float32 CUDA tensors, `out` included (see
+    :func:`aerobulk_model_f32` for what the outputs are).  Tensors of any other dtype raise AerobulkError(101)."""
+    return _model_device(lib().aerobulk_gpu_model_device_f32, "float32", jt, Nt, calgo, zt, zu,
+                         (sst, t_zt, hum_zt, U_zu, V_zu, slp), out, Niter, l_use_skin, rad_sw, rad_lw, shape)
+
+
+def _model_device(fn, dtype, jt, Nt, calgo, zt, zu, tensors, out, Niter, l_use_skin, rad_sw, rad_lw, shape):
+    tensors = list(tensors)
+    n = tensors[0].numel()
     for t in tensors + [x for x in (rad_sw, rad_lw) if x is not None] + list(out.values()):
-        if (not t.is_cuda) or str(t.dtype) != "torch.float64" or not t.is_contiguous() or t.numel() != n:
-            raise AerobulkError(101, "device API needs contiguous float64 CUDA tensors of one size")
+        if (not t.is_cuda) or str(t.dtype) != f"torch.{dtype}" or not t.is_contiguous() or t.numel() != n:
+            raise AerobulkError(101, f"device API needs contiguous {dtype} CUDA tensors of one size")
     Ni, Nj = (n, 1) if shape is None else (int(shape[0]), int(shape[1]))
     if Ni * Nj != n:
         raise AerobulkError(101, f"shape {shape} does not match {n} points")
     ni = None if Niter is None else C.byref(C.c_int(int(Niter)))
     ls = None if l_use_skin is None else C.byref(C.c_int(int(bool(l_use_skin))))
     ptr = lambda t: None if t is None else t.data_ptr()
-    rc = L.aerobulk_gpu_model_device(int(jt), int(Nt), calgo.encode(), float(zt), float(zu), Ni, Nj,
-                                     *[ptr(t) for t in tensors],
-                                     *[ptr(out[k]) for k in ("QL", "QH", "Tau_x", "Tau_y", "Evap")],
-                                     ni, ls, ptr(rad_sw), ptr(rad_lw), ptr(out.get("T_s")))
+    rc = fn(int(jt), int(Nt), calgo.encode(), float(zt), float(zu), Ni, Nj,
+            *[ptr(t) for t in tensors],
+            *[ptr(out[k]) for k in ("QL", "QH", "Tau_x", "Tau_y", "Evap")],
+            ni, ls, ptr(rad_sw), ptr(rad_lw), ptr(out.get("T_s")))
     _check(rc)
     return out
 

@@ -13,7 +13,7 @@
  * AEROBULK_MODEL signature of src/mod_aerobulk.f90:176-230) binds through
  * ISO_C_BINDING.  Plain pointers and sizes only; no C++/torch types.
  *
- * Arrays are FP64, (Ni,Nj) column-major (Fortran order), contiguous.
+ * Arrays are FP64 (FP32 for the *_f32 calls), (Ni,Nj) column-major (Fortran order), contiguous.
  * Unless stated otherwise a call is blocking and returns 0 on success or an
  * AEROBULK_GPU_ERR_* code.  Error behaviour mirrors the reference: by default
  * (fail-stop mode) an error prints ' *** E R R O R :' + message on stdout and
@@ -110,6 +110,33 @@ int aerobulk_gpu_model_device(int jt, int Nt, const char *calgo, double zt, doub
                               double *QL, double *QH, double *Tau_x, double *Tau_y, double *Evap,
                               const int *Niter, const int *l_use_skin,
                               const double *rad_sw, const double *rad_lw, double *T_s);
+
+/* ---- AEROBULK_MODEL on float32 fields ---------------------------------------------------------------------------
+ * aerobulk_gpu_model_f32 (host arrays) and aerobulk_gpu_model_device_f32 (device pointers) take the same arguments as
+ * the two calls above, with EVERY array float32: the 6 (8) inputs and the 5 (6) outputs.  Inputs are widened exactly to
+ * FP64, everything from there on is the FP64 call's own computation -- AEROBULK_INIT's statistics and verdicts, the
+ * stability sort, the bulk solve, the tau > 10 N/m^2 test -- and every output is rounded once, to nearest:
+ *
+ *     f32_call(x) == (float) f64_call((double) x)     bit for bit, at every point and every step.
+ *
+ * The warm-layer state stays FP64 on the device and after every step is bit-identical to the FP64 session's on the
+ * widened inputs, so FP32 and FP64 calls may alternate within one jt = 1..Nt session, and aerobulk_gpu_get_state /
+ * aerobulk_gpu_set_state are unchanged.  Errors are the FP64 call's: same code, same AEROBULK_INIT message, same
+ * (ji, jj) for tau > 10 (the stress it prints is computed from the float outputs).  Host arrays take the same paths as
+ * FP64 ones (device staging, zero-copy on pinned arrays, the pinned slab for pageable ones, aerobulk_gpu_set_devices
+ * splits) with half the bytes per point to move. */
+int aerobulk_gpu_model_f32(int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj,
+                           const float *sst, const float *t_zt, const float *hum_zt,
+                           const float *U_zu, const float *V_zu, const float *slp,
+                           float *QL, float *QH, float *Tau_x, float *Tau_y, float *Evap,
+                           const int *Niter, const int *l_use_skin,
+                           const float *rad_sw, const float *rad_lw, float *T_s);
+int aerobulk_gpu_model_device_f32(int jt, int Nt, const char *calgo, double zt, double zu, int Ni, int Nj,
+                                  const float *sst, const float *t_zt, const float *hum_zt,
+                                  const float *U_zu, const float *V_zu, const float *slp,
+                                  float *QL, float *QH, float *Tau_x, float *Tau_y, float *Evap,
+                                  const int *Niter, const int *l_use_skin,
+                                  const float *rad_sw, const float *rad_lw, float *T_s);
 
 /* ---- direct TURB_* entry (what GCMs such as NEMO's sbcblk and the reference's test programs call) ------ */
 
@@ -402,12 +429,14 @@ void aerobulk_gpu_reset_launch_count(void);
  * instructions per second (all SMs), the denominator of the FP64 roofline. */
 double aerobulk_gpu_measure_fp64_peak(void);
 /* Algorithmic FP64-pipe work per point (SURVEY.md 8d: fx + nb_iter*it) and
- * algorithmic bytes per point for (algo, skin). */
+ * algorithmic bytes per point for (algo, skin), of the FP64 calls.  A float32 call (aerobulk_gpu_model*_f32) does the
+ * same work and moves half the per-point array bytes; these two functions do not describe it. */
 double aerobulk_gpu_work_per_point(const char *calgo, int skin, int nb_iter);
 double aerobulk_gpu_bytes_per_point(const char *calgo, int skin);
 /* Resources of the flux kernel a call with (algo, skin, zt == zu) launches, on the session device: registers per thread,
  * local-memory (spill) bytes per thread, resident blocks per SM at the launch configuration (256 threads).  For reports
- * and regression tests: the skin kernels are built for 3 blocks/SM, the others for 4 (DESIGN.md 3.1).  0 on success. */
+ * and regression tests: the skin kernels are built for 3 blocks/SM, the others for 4 (DESIGN.md 3.1).  0 on success.
+ * It reports the FP64 kernel; the float32 twin a *_f32 call launches is listed in profiles/f32_kernels_r03b.txt. */
 int aerobulk_gpu_kernel_info(const char *calgo, int skin, int zt_eq_zu, int *registers, int *local_bytes, int *blocks_per_sm);
 const char *aerobulk_gpu_version(void);
 
