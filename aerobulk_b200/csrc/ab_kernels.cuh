@@ -192,7 +192,9 @@ enum ProbeFunc {
     PROBE_PSI_M_ANDREAS, PROBE_PSI_H_ANDREAS,
     PROBE_Z0TQ_LKB = 30, PROBE_CD_N10_NCAR, PROBE_CHARN_COARE3P0, PROBE_CHARN_COARE3P6, PROBE_CS_COARE, PROBE_CS_ECMWF,
     PROBE_EXP = 40, PROBE_EXP10, PROBE_LOG, PROBE_ATAN, PROBE_SQRT, PROBE_RSQRT, PROBE_CBRT, PROBE_RCBRT, PROBE_POW075,
-    PROBE_RCP, PROBE_POWR
+    PROBE_RCP, PROBE_POWR, PROBE_ATAN_GE1, PROBE_LOG10, PROBE_EXP_B, PROBE_EXP10_B,
+    PROBE_E_SAT_ICE = 60, PROBE_Q_SAT_ICE, PROBE_PSI_M_ICE, PROBE_PSI_H_ICE, PROBE_F_M_LOUIS, PROBE_F_H_LOUIS,
+    PROBE_ROUGH_LENG_M, PROBE_Z0T_AN87, PROBE_Z0Q_AN87, PROBE_CDN10_LU13, PROBE_CDN_LG15
 };
 cudaError_t launch_probe(int func, long long n, int nargs, const double *args, double *out, cudaStream_t s);
 

@@ -1,7 +1,7 @@
-// ab_probe.cu -- probe_kernel: evaluates ONE __device__ building block of ab_device.cuh / ab_math.cuh per
-// launch on n argument tuples, so that every function of the hot path can be unit-tested on the GPU against the
-// CPU restatement of the reference function it replaces (SURVEY.md 4: per-function unit tests;
-// tests/test_gpu_functions.py).  Test support inside the product library: nothing on the flux path calls it.
+// ab_probe.cu -- probe_kernel: evaluates ONE __device__ building block of ab_device.cuh / ab_ice.cuh / ab_math.cuh
+// per launch on n argument tuples, so that every function of the hot path can be unit-tested on the GPU against the
+// CPU restatement of the reference function it replaces (SURVEY.md 4: per-function unit tests; tests/test_gpu_functions.py,
+// tests/test_gpu_ice_functions.py).  Test support inside the product library: nothing on the flux path calls it.
 #include "ab_kernels.cuh"
 
 namespace abk {
@@ -36,7 +36,10 @@ __global__ void __launch_bounds__(256) probe_kernel(int func, long long n, int n
     // ---- stability functions, rows a15-a25 (the solvers call the one-sided evaluators; the sign selects the side
     //      exactly as `zstab = 0.5 + SIGN(0.5, zeta)` does in the reference)
     case PROBE_PSI_M_NCAR: r = psi_m_ncar(a[0]); break;
-    case PROBE_PSI_H_NCAR: r = psi_h_ncar(a[0]); break;
+    case PROBE_PSI_H_NCAR:   // the solvers take psi_h(zeta_u) from the paired evaluator: NaN where it differs
+        r = psi_h_ncar(a[0]);
+        if (!nonneg(a[0]) && psi_mh_ncar_unstable(a[0]).h != r) r = nan("");
+        break;
     case PROBE_PSI_M_COARE:
     case PROBE_PSI_H_COARE: {
         double m, h, ht;
@@ -46,12 +49,16 @@ __global__ void __launch_bounds__(256) probe_kernel(int func, long long n, int n
         break;
     }
     case PROBE_PSI_M_ECMWF: r = nonneg(a[0]) ? psi_m_ecmwf_stable(a[0]) : psi_m_ecmwf_unstable(a[0]); break;
-    case PROBE_PSI_H_ECMWF: r = nonneg(a[0]) ? psi_h_ecmwf_stable(a[0]) : psi_h_ecmwf_unstable(a[0]); break;
+    case PROBE_PSI_H_ECMWF:
+        r = nonneg(a[0]) ? psi_h_ecmwf_stable(a[0]) : psi_h_ecmwf_unstable(a[0]);
+        if (!nonneg(a[0]) && psi_mh_ecmwf_unstable(a[0]).h != r) r = nan("");
+        break;
     case PROBE_PSI_M_ANDREAS:
         r = nonneg(abm::dmin(a[0], 15.)) ? psi_m_andreas_stable(a[0]) : psi_mh_andreas_unstable(a[0]).m;
         break;
     case PROBE_PSI_H_ANDREAS:
         r = nonneg(abm::dmin(a[0], 15.)) ? psi_h_andreas_stable(a[0]) : psi_h_andreas_unstable(a[0]);
+        if (!nonneg(abm::dmin(a[0], 15.)) && psi_mh_andreas_unstable(a[0]).h != r) r = nan("");
         break;
     // ---- roughness / neutral coefficients
     case PROBE_Z0TQ_LKB: {   // (iflag, Rer, z0) -> z0t or z0q; the device works in log space
@@ -77,6 +84,28 @@ __global__ void __launch_bounds__(256) probe_kernel(int func, long long n, int n
     case PROBE_POW075: r = abm::pow075(a[0]); break;
     case PROBE_RCP: r = abm::fast_rcp(a[0]); break;
     case PROBE_POWR: r = abm::dpowr(a[0], a[1]); break;
+    case PROBE_ATAN_GE1: r = abm::datan_ge1(a[0]); break;
+    case PROBE_LOG10: r = abm::dlog10(a[0]); break;
+    case PROBE_EXP_B: r = abm::dexp_b(a[0]); break;
+    case PROBE_EXP10_B: r = abm::dexp10_b(a[0]); break;
+    // ---- sea ice (ab_ice.cuh)
+    case PROBE_E_SAT_ICE: r = e_sat_ice(a[0]); break;
+    case PROBE_Q_SAT_ICE: r = q_sat_ice(a[0], a[1]); break;
+    case PROBE_PSI_M_ICE: r = psi_m_ice(a[0]); break;
+    case PROBE_PSI_H_ICE: r = psi_h_ice(a[0]); break;
+    case PROBE_F_M_LOUIS: r = f_m_louis(a[0], a[1], a[2], a[3]); break;
+    case PROBE_F_H_LOUIS: r = f_h_louis(a[0], a[1], a[2], a[3]); break;
+    case PROBE_ROUGH_LENG_M: r = rough_leng_m(a[0], a[1]); break;
+    case PROBE_Z0T_AN87:
+    case PROBE_Z0Q_AN87: {   // (z0, u*, nu) -> z0t or z0q as solve_ice computes them (log space); NaN where it sets `bad`
+        double log_z0t, log_z0q;
+        bool bad = false;
+        log_rough_leng_tq(a[0], abm::dlog(a[0]), a[1], a[2], log_z0t, log_z0q, bad);
+        r = bad ? nan("") : abm::dexp(func == PROBE_Z0T_AN87 ? log_z0t : log_z0q);
+        break;
+    }
+    case PROBE_CDN10_LU13: r = CdN10_f_LU13(a[0]); break;
+    case PROBE_CDN_LG15: r = CdN_f_LG15_light(a[0], a[1]); break;   // (LOG(10/z0w) / LOG(zu/z0w), A)
     default: r = nan(""); break;
     }
     out[i] = r;

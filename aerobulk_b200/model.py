@@ -650,7 +650,10 @@ PROBE = {"e_sat": 1, "q_sat": 2, "theta_from_z_P0_T_q": 3, "rho_air": 4, "visc_a
          "psi_m_ncar": 20, "psi_h_ncar": 21, "psi_m_coare": 22, "psi_h_coare": 23, "psi_m_ecmwf": 24, "psi_h_ecmwf": 25,
          "psi_m_andreas": 26, "psi_h_andreas": 27, "z0tq_LKB": 30, "cd_n10_ncar": 31, "charn_coare3p0": 32,
          "charn_coare3p6": 33, "cs_coare": 34, "cs_ecmwf": 35, "exp": 40, "exp10": 41, "log": 42, "atan": 43, "sqrt": 44,
-         "rsqrt": 45, "cbrt": 46, "rcbrt": 47, "pow075": 48, "rcp": 49, "powr": 50}
+         "rsqrt": 45, "cbrt": 46, "rcbrt": 47, "pow075": 48, "rcp": 49, "powr": 50, "atan_ge1": 51, "log10": 52,
+         "exp_b": 53, "exp10_b": 54, "e_sat_ice": 60, "q_sat_ice": 61, "psi_m_ice": 62, "psi_h_ice": 63,
+         "f_m_louis": 64, "f_h_louis": 65, "rough_leng_m": 66, "z0t_an87": 67, "z0q_an87": 68, "CdN10_f_LU13": 69,
+         "CdN_f_LG15_light": 70}
 
 
 def probe(func: str, *args) -> np.ndarray:

@@ -450,7 +450,13 @@ const char *aerobulk_gpu_version(void);
  *    20/21 psi_m/psi_h NCAR  22/23 COARE  24/25 ECMWF  26/27 ANDREAS  (zeta)
  *    30 z0tq_LKB(iflag,Rer,z0)  31 cd_n10_ncar(w)  32 charn_coare3p0(w)  33 charn_coare3p6(w)
  *    34 dT_cs of CS_COARE(alpha,Qsw,Qnsol,us,Qlat)  35 dT_cs of CS_ECMWF(alpha,Qsw,Qnsol,us)
+ *    (21, 25 and 27 return NaN where the paired psi_m/psi_h evaluator the solvers use differs from the single psi_h)
  *    40 exp  41 exp10  42 log  43 atan  44 sqrt  45 x**-1/2  46 cbrt  47 x**-1/3  48 x**0.75  49 1/x  50 x**y
+ *    51 atan(x), x >= 1  52 log10  53 exp, |x| <= 700  54 exp10, |x| <= 300
+ *    60 e_sat_ice(T)  61 q_sat_ice(T,p)  62/63 psi_m_ice/psi_h_ice(zeta), |zeta| <= 50
+ *    64/65 f_m_louis/f_h_louis(zu,Rib,Cxn,z0)  66 rough_leng_m(us,nu)
+ *    67/68 z0t/z0q of rough_leng_tq(z0,us,nu), NaN where the reference stops  69 CdN10_f_LU13(A)
+ *    70 CdN_f_LG15_light(LOG(10/z0w)/LOG(zu/z0w), A)          (src/ice/, SURVEY.md 8f row 4)
  * Returns 0, or an AEROBULK_GPU_ERR_* code. */
 int aerobulk_gpu_probe(int func, long long n, int nargs, const double *args, double *out);
 

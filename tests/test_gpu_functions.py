@@ -5,7 +5,9 @@ the reference function it replaces (file:line in the table below).
 
 Tolerances, written here: the device functions use their own exp/log/atan/roots (<= 4 ulp each) and FMA
 contraction, so a building block agrees with glibc arithmetic to a few 1e-16 relative per transcendental;
-REL is the bound asserted per function on |gpu - oracle| / max(|oracle|, FLOOR)."""
+REL is the bound asserted per function on |gpu - oracle| / max(|oracle|, FLOOR).  The kernels' own math (MATH below) is
+held to mpmath; the sea-ice building blocks are in tests/test_gpu_ice_functions.py."""
+import mpmath as mp
 import numpy as np
 import pytest
 
@@ -53,7 +55,9 @@ CASES = {
     "charn_coare3p6": (lambda L: L.abo_charn_coare3p6, (np.concatenate([WIND, [0.0, 2.9, 19.5, 35.0]]),), 1e-14, 1e-3,
                        "mod_blk_coare3p6.f90:417-432"),
 }
-# psi: absolute floor 1 (psi is O(1..100)); COARE convective branch mixes 3 logs, 2 atans and a cube root
+# psi: absolute floor 1 (psi is O(1..100)); COARE convective branch mixes 3 logs, 2 atans and a cube root.  The solvers take
+# psi_h(zeta_u) from the paired psi_mh_*_unstable evaluators and psi_h(zeta_t) from the single ones: the psi_h probes
+# return NaN where the two differ, which the finiteness check below catches
 PSI = {"ncar": (3, 2e-14), "coare": (2, 1e-13), "ecmwf": (4, 5e-14), "andreas": (5, 1e-13)}
 
 
@@ -143,22 +147,106 @@ def test_cool_skin_matches_oracle(ab, OL, coare):
     assert err.max() <= 1e-12, float(err.max())
 
 
+ULP = 2.0 ** -52
+TAN_PI8 = [0.41421356237309503, 0.41421356237309515]      # the doubles either side of tan(pi/8) and tan(3 pi/8)
+TAN_3PI8 = [2.414213562373095, 2.4142135623730954]
+_next = lambda x, d: np.atleast_1d(np.nextafter(np.asarray(x, dtype=np.float64), d))
+_ATAN_EDGES = np.array(TAN_PI8 + TAN_3PI8 + [1.0])
+_ATAN_EDGES = np.concatenate([_ATAN_EDGES, _next(_ATAN_EDGES, 0.0), _next(_ATAN_EDGES, 10.0)])
+_GE1 = np.concatenate([U(1.0, 6.0), 1.0 + np.exp(U(-36.0, 3.0)), np.exp(U(0.0, 40.0)),
+                       [1.0, np.nextafter(1.0, 2.0), 1.7320508, 1e30] + TAN_3PI8])
+_L10 = np.exp(U(-5.0, 5.0))
+_POWR_X = np.exp(U(-12.0, 12.0))
+_POWR_Y = rng.choice([0.25, 0.3333, 0.5, 0.6, 0.72, 0.75, 0.79, 1.5, -0.599, -3.935, 0.929, 2.0 / 3.0, 1.4, 1.0 + 1.0 / 14.0, 0.0],
+                     _POWR_X.size)
+_P100 = 2.0 ** -100                               # the guard of pow075 / fast_cbrt: 0 below it
+
+# name -> (mpmath function, [(label, arguments, bound)], arguments that must give exactly 0).  A bound is a relative error
+# against mpmath (50 digits): "core" keeps the bound of the ranges checked since round 2; every other set takes the bound
+# tests/test_math_accuracy.py proves for the host build of the same source (whose seeds are degraded to 2**-21), in ulp
+# of 2**-52.  powr: (4 + 2 |y log x|) ulp, the error of the logarithm amplified by the exponent.
 MATH = {
-    "exp": (np.exp, U(-690.0, 690.0), 4.5e-16), "exp10": (lambda x: 10.0 ** x, U(-300.0, 300.0), 4.5e-16),
-    "log": (np.log, 10.0 ** U(-300, 300), 4.5e-16), "atan": (np.arctan, np.concatenate([U(-50.0, 50.0), 10.0 ** U(-8, 8)]), 4.5e-16),
-    "sqrt": (np.sqrt, 10.0 ** U(-280, 300), 4.5e-16), "rsqrt": (lambda x: 1.0 / np.sqrt(x), 10.0 ** U(-30, 30), 6e-16),
-    "cbrt": (np.cbrt, 10.0 ** U(-28, 30), 6e-16), "rcbrt": (lambda x: 1.0 / np.cbrt(x), 10.0 ** U(-28, 30), 6e-16),
-    "pow075": (lambda x: x ** 0.75, 10.0 ** U(-28, 30), 6e-16), "rcp": (lambda x: 1.0 / x, 10.0 ** U(-280, 280) * np.sign(U(-1, 1)), 4.5e-16),
+    "exp": (mp.exp, [("core", (U(-690.0, 690.0),), 4.5e-16),
+                     ("near 0, flush threshold", (np.concatenate([U(-1.0, 1.0), U(-700.0, -690.0, 500), [-700.0, 0.0, -0.0],
+                                                                  _next(-700.0, 0.0)]),), 4 * ULP)],
+            (np.array([np.nextafter(-700.0, -800.0), -700.5, -701.0, -1500.0, -1e9]),)),
+    "exp10": (lambda x: mp.mpf(10) ** x, [("core", (U(-300.0, 300.0),), 4.5e-16),
+                                          ("e_sat range, flush threshold",
+                                           (np.concatenate([U(-0.2, 4.0), U(-304.0, -300.0, 500), [-304.0, 0.0],
+                                                            _next(-304.0, 0.0)]),), 4 * ULP)],
+              (np.array([np.nextafter(-304.0, -400.0), -304.5, -305.0, -1e9]),)),
+    "log": (mp.log, [("core", (10.0 ** U(-300, 300),), 4.5e-16),
+                     ("near 1", (np.concatenate([1.0 + U(-3e-3, 3e-3), U(0.5, 2.0), _next(1.0, 0.0), _next(1.0, 2.0),
+                                                 [2.0, 0.5, 1e-9, 10.0]]),), 4 * ULP)],
+            (np.array([1.0]),)),
+    "atan": (mp.atan, [("core", (np.concatenate([U(-50.0, 50.0), 10.0 ** U(-8, 8)]),), 4.5e-16),
+                       ("range switches", (np.concatenate([U(0.3, 3.0), _ATAN_EDGES, -_ATAN_EDGES[_ATAN_EDGES > 0]]),), 4 * ULP)],
+             (np.array([0.0]),)),
+    "atan_ge1": (mp.atan, [("x >= 1", (_GE1,), 3 * ULP)], None),
+    "log10": (mp.log10, [("|log10 x| > 1e-3", (np.concatenate([_L10[np.abs(np.log10(_L10)) > 1e-3], 10.0 ** U(-300, 300)]),),
+                          5 * ULP)], (np.array([1.0]),)),
+    "exp_b": (mp.exp, [("[-700, 700]", (np.concatenate([U(-700.0, 700.0), U(-1.0, 1.0), [-700.0, 700.0, 0.0]]),), 4 * ULP)],
+              None),
+    "exp10_b": (lambda x: mp.mpf(10) ** x, [("[-300, 300]", (np.concatenate([U(-300.0, 300.0), U(-0.2, 4.0), [-300.0, 300.0]]),),
+                                            4 * ULP)], None),
+    "sqrt": (mp.sqrt, [("core", (10.0 ** U(-280, 300),), 4.5e-16), ("e**[-60, 60]", (np.exp(U(-60.0, 60.0)),), 2 * ULP)],
+             (np.array([0.0, 1e-300]),)),
+    "rsqrt": (lambda x: 1 / mp.sqrt(x), [("core", (10.0 ** U(-30, 30),), 6e-16), ("e**[-60, 60]", (np.exp(U(-60.0, 60.0)),), 2 * ULP)],
+              None),
+    "cbrt": (mp.cbrt, [("core", (10.0 ** U(-28, 30),), 6e-16),
+                       ("guard", (np.concatenate([[_P100, np.nextafter(_P100, 1.0), 2.0 * _P100, 1e-30], U(0.5, 4.0)]),), 3 * ULP)],
+             (np.array([np.nextafter(_P100, 0.0), 1e-31, 1e-300, 0.0]),)),
+    "rcbrt": (lambda x: 1 / mp.cbrt(x), [("core", (10.0 ** U(-28, 30),), 6e-16), ("e**[-60, 60]", (np.exp(U(-60.0, 60.0)),), 2 * ULP)],
+              None),
+    "pow075": (lambda x: x ** mp.mpf(0.75), [("core", (10.0 ** U(-28, 30),), 6e-16),
+                                            ("guard", (np.concatenate([[_P100, np.nextafter(_P100, 1.0), 2.0 * _P100, 1e-30],
+                                                                       U(0.5, 4.0)]),), 3 * ULP)],
+               (np.array([np.nextafter(_P100, 0.0), 1e-31, 1e-300, 0.0]),)),
+    "rcp": (lambda x: 1 / x, [("core", (10.0 ** U(-280, 280) * np.sign(U(-1, 1)),), 4.5e-16),
+                              ("e**[-30, 30]", (np.exp(U(-30.0, 30.0)) * np.sign(U(-1, 1)),), 2 * ULP)], None),
+    "powr": (lambda x, y: x ** y, [("e**[-12, 12] ** y", (_POWR_X, _POWR_Y),
+                                    lambda x, y: (4 + 2 * np.abs(y * np.log(x))) * ULP)],
+             (np.zeros(4), np.array([0.75, 0.79, 2.0 / 3.0, 1.4]))),
 }
+
+
+def _mp_relerr(f, got, cols):
+    with mp.workdps(50):
+        return np.array([float(abs((mp.mpf(float(g)) - r) / r))
+                         for g, r in ((got[i], f(*[mp.mpf(float(c[i])) for c in cols])) for i in range(got.size))])
 
 
 @pytest.mark.parametrize("name", sorted(MATH))
 def test_own_math_on_device(ab, name):
-    """ab_math.cuh on the device against numpy/glibc (the host-compiled copy is held to mpmath in
-    tests/test_math_accuracy.py): <= 2 ulp (4.5e-16) for exp/log/atan/sqrt/rcp, <= 2.7 ulp for the root family."""
-    f, x, rel = MATH[name]
-    got = ab.probe(name, x)
-    ref = f(x)
-    err = np.abs(got - ref) / np.abs(ref)
-    print(f"[function] abm::{name}: max rel err {err.max():.2e}")
-    assert err.max() <= rel, (name, float(err.max()), float(x[err.argmax()]))
+    """ab_math.cuh as the device compiles it (MUFU seeds, FMA contraction) against mpmath, over the ranges the physics
+    uses and the tails where the functions switch: the flush thresholds of exp / exp10, log near 1, atan's range switches
+    at tan(pi/8) and tan(3 pi/8), the 2**-100 guard of pow075 / cbrt.  The host build of the same source is held to the
+    same bounds in tests/test_math_accuracy.py; a device value outside them points at contraction or a seed."""
+    f, sets, zeros = MATH[name]
+    for label, cols, bound in sets:
+        cols = [np.asarray(c, dtype=np.float64) for c in cols]
+        got = ab.probe(name, *cols)
+        err = _mp_relerr(f, got, cols)
+        b = bound(*cols) if callable(bound) else np.full(err.size, bound)
+        print(f"[function] abm::{name:8s} {label:28s}: max rel err {err.max():.2e} ({err.max() / ULP:.2f} ulp), "
+              f"worst err/bound {(err / b).max():.2f}")
+        assert (err <= b).all(), (name, label, float(err.max()), [float(c[(err / b).argmax()]) for c in cols])
+    if zeros is not None:
+        got = ab.probe(name, *zeros)
+        assert (got == 0.0).all(), (name, got)
+    if name == "atan":
+        assert np.signbit(ab.probe("atan", np.array([-0.0]))[0])
+
+
+def test_atan_ge1_correctly_rounded_at_its_expansion_point(ab):
+    """datan_ge1(x) = atan_hi(c) + (t + atan_lo(c)), c = tan(3 pi/8), t = atan((x - c) / (1 + c x)).  For x within a few
+    hundred ulp of c, t is a few ulp of the result and exact to ~1e-30, so the one rounding left is the final addition:
+    the result must be correctly rounded.  The low part of atan(c) (0.12 ulp) decides the rounding of about one point in
+    eight here; an error of 3 ulp elsewhere cannot show its loss."""
+    c = TAN_3PI8[0]
+    x = c + np.arange(-300, 301) * np.spacing(c)
+    got = ab.probe("atan_ge1", x)
+    with mp.workdps(50):
+        err = np.array([float(abs(mp.mpf(float(g)) - mp.atan(mp.mpf(float(v))))) for g, v in zip(got, x)]) / np.spacing(got)
+    print(f"[function] abm::atan_ge1 around tan(3 pi/8): max err {err.max():.4f} ulp of the result")
+    assert err.max() <= 0.5, (float(err.max()), float(x[err.argmax()]))

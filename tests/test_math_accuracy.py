@@ -94,6 +94,10 @@ def test_atan_of_arguments_from_one_up(abm):
     assert _relerr(abm(16, x), x, mp.atan) <= 3 * ULP
     # and it agrees with the general-purpose version to rounding
     assert np.abs(abm(16, x) - abm(4, x)).max() <= 4 * ULP
+    # around c the only rounding left is atan_hi(c) + (t + atan_lo(c)): correctly rounded (the low part decides it)
+    x = 2.414213562373095 + np.arange(-300, 301) * np.spacing(2.414213562373095)
+    got = abm(16, x)
+    assert all(abs(mp.mpf(float(g)) - mp.atan(mp.mpf(float(v)))) <= np.spacing(g) / 2 for g, v in zip(got, x))
 
 
 def test_guard_free_roots(abm):
