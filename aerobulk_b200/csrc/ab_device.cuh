@@ -100,6 +100,13 @@ constexpr double ZBM_A = 5. / 6.5;                   // b_m                     
 constexpr double ZBBM_A = 0x1.56bfea66ef78dp-1;      // ABS((1-b_m)/b_m)**(1/3)   mod_blk_andreas.f90:345
 
 enum Algo { COARE3P0 = 1, COARE3P6 = 2, NCAR = 3, ECMWF = 4, ANDREAS = 5 };
+// the psi tables an algorithm's solver reads (abm::load_tables<PSI_TABLES_OF<ALGO>>()); ECMWF starts from the COARE first
+// guess, NCAR and ANDREAS read none.  A kernel that reads a table it does not load computes garbage: -Xptxas -v shows which tables a kernel's shared
+// memory holds (7.7 KB without psi tables, 9.75 KB more per family)
+template <int ALGO>
+constexpr int PSI_TABLES_OF = (ALGO == COARE3P0 || ALGO == COARE3P6) ? abm::PSI_TABLES_COARE
+                              : (ALGO == ECMWF)                      ? abm::PSI_TABLES_ALL
+                                                                     : abm::PSI_TABLES_NONE;
 
 // ---------------------------------------------------------------------------
 // small helpers
@@ -293,6 +300,26 @@ struct PsiMH {
     double m, h;
 };
 
+// Unstable psi_m / psi_h from the tables of ab_math.cuh (abm::psi_row): the COARE blend (COARE 3.x and the first guess
+// of ECMWF) and the Paulson pair with coefficient 16 (ECMWF).  The COARE first guess does not clip zeta: below -50, and for
+// NaN, psi_*_coare_formula runs.  NCAR and ANDREAS keep their Paulson formulas: the table's 96 bytes of coefficients per
+// function are shared-memory bound where the formula is cheap (profiles/psi_probe_r03d.txt), and both kernels were
+// slower with it (profiles/ab_psi_table_r03d.txt).
+template <int FAM>
+ABD PsiMH psi_mh_table(double z)
+{
+    const abm::PsiRow a = abm::psi_row(z);
+    PsiMH r;
+    r.m = abm::psi_poly<0>(abm::psi_coeffs<FAM>(), a);
+    r.h = abm::psi_poly<1>(abm::psi_coeffs<FAM>(), a);
+    return r;
+}
+template <int FAM>
+ABD double psi_m_table(double z) { return abm::psi_poly<0>(abm::psi_coeffs<FAM>(), abm::psi_row(z)); }
+template <int FAM>
+ABD double psi_h_table(double z) { return abm::psi_poly<1>(abm::psi_coeffs<FAM>(), abm::psi_row(z)); }
+ABD bool in_psi_table(double z) { return z >= -abm::PSI_ZMAX; }
+
 // Large & Yeager, src/mod_blk_ncar.f90:333-407
 ABD PsiMH psi_mh_ncar_unstable(double z)
 {
@@ -333,7 +360,7 @@ ABD double psi_h_coare_stable(double z)
     const double a = fabs(1. + 2. * z * KC(1. / 3.));
     return -(a * abm::fast_sqrt_pos(a) + KC(.6667) * (z - KC(14.28)) * e + KC(8.525));
 }
-ABD PsiMH psi_mh_coare_unstable(double z)
+ABD PsiMH psi_mh_coare_formula(double z)
 {
     const double phi_h = abm::fast_sqrt_pos(fabs(1. - 15. * z));                               // **.5
     const double phi_m = abm::fast_sqrt_pos(phi_h);                                            // **.25
@@ -351,7 +378,8 @@ ABD PsiMH psi_mh_coare_unstable(double z)
     r.h = (1. - f) * kh + f * ch;
     return r;
 }
-ABD double psi_h_coare_unstable(double z)
+ABD PsiMH psi_mh_coare_unstable(double z) { return in_psi_table(z) ? psi_mh_table<abm::PSI_TABLES_COARE>(z) : psi_mh_coare_formula(z); }
+ABD double psi_h_coare_formula(double z)
 {
     const double phi_h = abm::fast_sqrt_pos(fabs(1. - 15. * z));
     double f = z * z;
@@ -360,6 +388,7 @@ ABD double psi_h_coare_unstable(double z)
     const double ch = psi_coare_convective(powr(fabs(1. - KC(34.15) * z), KC(.3333)));
     return (1. - f) * kh + f * ch;
 }
+ABD double psi_h_coare_unstable(double z) { return in_psi_table(z) ? psi_h_table<abm::PSI_TABLES_COARE>(z) : psi_h_coare_formula(z); }
 // psi_m(zeta_u), psi_h(zeta_u), psi_h(zeta_t); zeta_t has the sign of zeta_u
 template <bool ZTEQ>
 ABD void psi3_coare(double zeta_u, double zeta_t, double &m_u, double &h_u, double &h_t)
@@ -391,25 +420,12 @@ ABD PsiMH psi_mh_ecmwf_stable(double zeta)
     r.h = -t - a * abm::fast_sqrt_pos(a) - KC(2. / 3. * zc) + 1.;
     return r;
 }
-ABD PsiMH psi_mh_ecmwf_unstable(double zeta)
-{
-    const double z = cap_zeta(zeta);
-    const double x2 = abm::fast_sqrt_pos(fabs(1. - 16. * z));
-    const double x = abm::fast_sqrt_pos(x2);
-    const double t = 1. + x;
-    PsiMH r;
-    r.m = abm::dlog(0.125 * t * t * (1. + x2)) - 2. * abm::datan_ge1(x) + KC(0.5 * RPI);
-    r.h = 2. * abm::dlog(0.5 * (1. + x2));
-    return r;
-}
+// unstable: the cap keeps zeta inside the Paulson table (a NaN zeta is capped to -50, as before)
+ABD PsiMH psi_mh_ecmwf_unstable(double zeta) { return psi_mh_table<abm::PSI_TABLES_PAULSON>(cap_zeta(zeta)); }
 ABD double psi_m_ecmwf_stable(double zeta) { return psi_mh_ecmwf_stable(zeta).m; }
 ABD double psi_h_ecmwf_stable(double zeta) { return psi_mh_ecmwf_stable(zeta).h; }
-ABD double psi_m_ecmwf_unstable(double zeta) { return psi_mh_ecmwf_unstable(zeta).m; }
-ABD double psi_h_ecmwf_unstable(double zeta)
-{
-    const double x2 = abm::fast_sqrt_pos(fabs(1. - 16. * cap_zeta(zeta)));
-    return 2. * abm::dlog(0.5 * (1. + x2));
-}
+ABD double psi_m_ecmwf_unstable(double zeta) { return psi_m_table<abm::PSI_TABLES_PAULSON>(cap_zeta(zeta)); }
+ABD double psi_h_ecmwf_unstable(double zeta) { return psi_h_table<abm::PSI_TABLES_PAULSON>(cap_zeta(zeta)); }
 
 // Andreas et al. 2015 (Paulson unstable / Grachev 2007 stable), src/mod_blk_andreas.f90:307-410
 // the two terms of the stable functions that do not depend on zeta, as glibc evaluates them (the reference computes them

@@ -19,7 +19,7 @@ static constexpr int ICE_MIN_BLOCKS = 3;
 template <int IALGO, bool ZTEQ>
 __global__ void __launch_bounds__(ICE_BLOCK, ICE_MIN_BLOCKS) ice_turb_kernel(const IceTurbArgs a)
 {
-    abm::load_tables();
+    abm::load_tables<abm::PSI_TABLES_NONE>();
     const long long i = (long long)blockIdx.x * ICE_BLOCK + threadIdx.x;
     if (i >= a.n) return;
     double fr = 0., frf = 0.;
@@ -46,7 +46,7 @@ __device__ __forceinline__ double humidity_to_q(int kind, double hum, double T, 
 template <int IALGO, bool ZTEQ>
 __global__ void __launch_bounds__(ICE_BLOCK, ICE_MIN_BLOCKS) ice_flux_kernel(const OceIceArgs a)
 {
-    abm::load_tables();
+    abm::load_tables<abm::PSI_TABLES_NONE>();
     const long long i = (long long)blockIdx.x * ICE_BLOCK + threadIdx.x;
     if (i >= a.n) return;
     const double sit = __ldg(a.sit + i), T = __ldg(a.t_zt + i), slp = __ldg(a.slp + i), wnd = __ldg(a.wnd + i);
@@ -91,7 +91,7 @@ __global__ void __launch_bounds__(ICE_BLOCK, ICE_MIN_BLOCKS) ice_flux_kernel(con
 template <int IALGO, bool ZTEQ>
 __global__ void __launch_bounds__(ICE_BLOCK, ICE_MIN_BLOCKS) ice_series_kernel(const IceSeriesArgs a)
 {
-    abm::load_tables();
+    abm::load_tables<abm::PSI_TABLES_NONE>();
     const long long i = (long long)blockIdx.x * ICE_BLOCK + threadIdx.x;
     if (i >= a.n) return;
     const double sit = __ldg(a.sit + i), T = __ldg(a.t_zt + i), slp = __ldg(a.slp + i), wnd = __ldg(a.wnd + i);
@@ -130,7 +130,7 @@ __global__ void __launch_bounds__(ICE_BLOCK, ICE_MIN_BLOCKS) ice_series_kernel(c
 template <int OALGO, bool ZTEQ>
 __global__ void __launch_bounds__(ICE_BLOCK, ICE_MIN_BLOCKS) leads_kernel(const OceIceArgs a)
 {
-    abm::load_tables();
+    abm::load_tables<PSI_TABLES_OF<OALGO>>();
     const long long i = (long long)blockIdx.x * ICE_BLOCK + threadIdx.x;
     if (i >= a.n) return;
     const double sst = __ldg(a.sst + i), T = __ldg(a.t_zt + i), slp = __ldg(a.slp + i), wnd = __ldg(a.wnd + i);

@@ -218,7 +218,7 @@ __device__ __forceinline__ void store_warm_layer(const Args &a, long long i, con
 template <class T, int ALGO, bool SKIN, bool ZTEQ>
 __device__ __forceinline__ void flux_point(const FluxArgs &a, unsigned tid)
 {
-    abm::load_tables();
+    abm::load_tables<PSI_TABLES_OF<ALGO>>();
     long long i = (long long)blockIdx.x * FLUX_BLOCK + tid;
     if (a.perm) i = (i / SORT_WIN) * SORT_WIN + a.perm[i];   // slot -> point (perm is padded to whole windows)
     if (i >= a.n) return;
@@ -322,7 +322,7 @@ cudaError_t launch_flux(int algo, bool skin, bool zteq, size_t elem, const FluxA
 template <int ALGO, bool CS, bool WL, bool ZTEQ>
 __global__ void __launch_bounds__(FLUX_BLOCK, (CS || WL) ? AB_MIN_BLOCKS : AB_MIN_BLOCKS_NOSKIN) turb_kernel(const TurbArgs a)
 {
-    abm::load_tables();
+    abm::load_tables<PSI_TABLES_OF<ALGO>>();
     const long long i = (long long)blockIdx.x * FLUX_BLOCK + threadIdx.x;
     if (i >= a.n) return;
     constexpr bool SKIN = CS || WL;

@@ -1,4 +1,5 @@
-// ab_math.cuh -- the kernels' own FP64 exp / exp10 / log / log10 / atan / pow, and Goff's e_sat as a piecewise polynomial.
+// ab_math.cuh -- the kernels' own FP64 exp / exp10 / log / log10 / atan / pow, and Goff's e_sat and the unstable stability
+// functions as piecewise polynomials.
 //
 // Why not libdevice: ptxas builds every FP64 literal of CUDA's math functions with two 32-bit moves
 // (UMOV / IMAD.MOV), which made ~35 % of the issued instructions of the flux kernels and a 188 KB
@@ -222,28 +223,46 @@ ABM_BIG double dlog_poly(double x)
 #ifndef ABM_SMEM_TABLES
 #define ABM_SMEM_TABLES 1   // measured 3 % faster than __ldg of the global tables (64-bit address arithmetic)
 #endif
+// which psi tables a kernel reads (psi_table): load_tables copies only those
+enum { PSI_TABLES_NONE = 0, PSI_TABLES_COARE = 1, PSI_TABLES_PAULSON = 2, PSI_TABLES_ALL = 3 };
 #if ABM_SMEM_TABLES && !defined(ABM_HOST_TEST)
-// block-local copies of the tables in shared memory (4.5 KB, and 3.2 KB of e_sat coefficients; 32-bit addressing, LDS
-// instead of LDG); every kernel must call abm::load_tables() (all threads) before the first exp/log/esat_table
+// block-local copies of the tables in shared memory (4.5 KB, 3.2 KB of e_sat coefficients and 10 KB per family of psi
+// coefficients; 32-bit addressing, LDS instead of LDG); every kernel must call abm::load_tables() (all threads) before the
+// first exp/log/esat_table/psi_table, naming in PSI every psi family it evaluates from a table (a shared array a kernel
+// does not reference takes no shared memory)
 __shared__ double S_EXP_T[64];
 __shared__ double S_LOG_T[512];
 __shared__ __align__(16) double S_ESAT_T[8 * ESAT_ROWS];
+__shared__ __align__(16) double S_PSI_COARE_T[2 * (PSI_DEG + 1) * PSI_ROWS];
+__shared__ __align__(16) double S_PSI_PAULSON_T[2 * (PSI_DEG + 1) * PSI_ROWS];
+ABM_FN void copy_table2(double *dst, const double *src, int n2)
+{
+    for (int i = threadIdx.x; i < n2; i += blockDim.x)
+        reinterpret_cast<double2 *>(dst)[i] = reinterpret_cast<const double2 *>(src)[i];
+}
+template <int PSI = PSI_TABLES_ALL>
 ABM_FN void load_tables()
 {
     for (int i = threadIdx.x; i < 64; i += blockDim.x) S_EXP_T[i] = EXP_T[i];
     for (int i = threadIdx.x; i < 512; i += blockDim.x) S_LOG_T[i] = LOG_T[i];
-    for (int i = threadIdx.x; i < 4 * ESAT_ROWS; i += blockDim.x)
-        reinterpret_cast<double2 *>(S_ESAT_T)[i] = reinterpret_cast<const double2 *>(ESAT_T)[i];
+    copy_table2(S_ESAT_T, ESAT_T, 4 * ESAT_ROWS);
+    if (PSI & PSI_TABLES_COARE) copy_table2(S_PSI_COARE_T, PSI_COARE_T, (PSI_DEG + 1) * PSI_ROWS);
+    if (PSI & PSI_TABLES_PAULSON) copy_table2(S_PSI_PAULSON_T, PSI_PAULSON_T, (PSI_DEG + 1) * PSI_ROWS);
     __syncthreads();
 }
 #define ABM_EXP_T(i) S_EXP_T[i]
 #define ABM_LOG_T(i) S_LOG_T[i]
 #define ABM_ESAT_T2(i) reinterpret_cast<const double2 *>(S_ESAT_T)[i]
+#define ABM_PSI_T(fam) S_PSI_##fam##_T
+#define ABM_PSI_T2(t, i) reinterpret_cast<const double2 *>(t)[i]
 #else
+template <int PSI = PSI_TABLES_ALL>
 ABM_FN void load_tables() {}
 #define ABM_EXP_T(i) ABM_LDG(&EXP_T[i])
 #define ABM_LOG_T(i) ABM_LDG(&LOG_T[i])
 #define ABM_ESAT_T2(i) ABM_LDG(reinterpret_cast<const double2 *>(ESAT_T) + (i))
+#define ABM_PSI_T(fam) PSI_##fam##_T
+#define ABM_PSI_T2(t, i) ABM_LDG(reinterpret_cast<const double2 *>(t) + (i))
 #endif
 
 // exp(r) for |r| <= ln2/128 times 2^(k/64), k = 64 m + j
@@ -353,6 +372,57 @@ ABM_FN double esat_table(double T)
     const double x2 = x * x;
     const double a0 = fma(c01.y, x, c01.x), a1 = fma(c23.y, x, c23.x), a2 = fma(c45.y, x, c45.x), a3 = fma(c67.y, x, c67.x);
     return fma(fma(a3, x2, a2), x2 * x2, fma(a1, x2, a0));
+}
+
+// Unstable psi_m / psi_h (zeta in [-PSI_ZMAX, 0], NaN excluded; the caller checks the range) from the piecewise
+// polynomials PSI_COARE_T / PSI_PAULSON_T: ~25 instructions per function instead of the roots, logarithms, arctangents
+// and powers of the formulas (two roots, three logs, three atans and two powr per COARE pair).  The row comes from the
+// high word of |zeta| (its exponent and PSI_K mantissa bits, integer instructions only), u = |zeta| - c is exact (c, the
+// row's centre, shares the binade of |zeta|), and row 0 (|zeta| < 2^PSI_E0, c = 0) has c_0 = 0: psi(-0) = 0.
+struct PsiRow {
+    int r;
+    double u;
+};
+ABM_FN PsiRow psi_row(double z)
+{
+    constexpr int S = 20 - PSI_K;
+    const int hx = hi_word(z) & 0x7fffffff;
+    int d = hx - ((1023 + PSI_E0) << 20) + (1 << S);
+    d = (d > 0) ? d : 0;
+    const int r = d >> S;
+    const int hc = (hx & -(1 << S)) | (1 << (S - 1));
+    PsiRow a;
+    a.r = r;
+    a.u = -z - make_double(r ? hc : 0, 0);
+    return a;
+}
+// F = 0: psi_m, 1: psi_h.  Estrin: depth 5 instead of 11 dependent FMAs
+template <int F>
+ABM_FN double psi_poly(const double *T, PsiRow a)
+{
+    constexpr int NP = (PSI_DEG + 1) / 2;
+    double c[NP];
+#pragma unroll
+    for (int j = 0; j < NP; ++j) {
+        const double2 p = ABM_PSI_T2(T, (F * NP + j) * PSI_ROWS + a.r);
+        c[j] = fma(p.y, a.u, p.x);
+    }
+    double x = a.u * a.u;
+#pragma unroll
+    for (int n = NP; n > 1; n = (n + 1) / 2) {
+#pragma unroll
+        for (int j = 0; j < n / 2; ++j) c[j] = fma(c[2 * j + 1], x, c[2 * j]);
+        if (n & 1) c[n / 2] = c[n - 1];
+        x = x * x;
+    }
+    return c[0];
+}
+// the coefficients of one family (PSI_TABLES_COARE or PSI_TABLES_PAULSON)
+template <int FAM>
+ABM_FN const double *psi_coeffs()
+{
+    if constexpr (FAM == PSI_TABLES_COARE) return ABM_PSI_T(COARE);
+    else return ABM_PSI_T(PAULSON);
 }
 
 // atan(t) for |t| <= tan(pi/8) (Estrin)

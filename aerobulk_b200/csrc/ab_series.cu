@@ -27,7 +27,7 @@ static constexpr int SERIES_MIN_BLOCKS = AB_SERIES_MIN_BLOCKS;
 template <int ALGO, bool SKIN, bool ZTEQ>
 __global__ void __launch_bounds__(SERIES_BLOCK, SERIES_MIN_BLOCKS) series_kernel(const SeriesArgs a)
 {
-    abm::load_tables();
+    abm::load_tables<PSI_TABLES_OF<ALGO>>();
     const long long s = (long long)blockIdx.x * SERIES_BLOCK + threadIdx.x;
     if (s >= a.S) return;
     const double lon = __ldg(a.lon + s);

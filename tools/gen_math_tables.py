@@ -57,6 +57,118 @@ def emit(name, cs, comment):
     return s + "\n};\n\n"
 
 
+# ---- unstable stability functions psi(zeta), zeta in [-PSI_ZMAX, 0], as piecewise polynomials of |zeta|.  Row 0 covers
+# |zeta| < 2^PSI_E0 with a polynomial in u = |zeta| whose constant term is 0 (psi(-0) = 0, and absolute accuracy at the
+# tiny zeta of the roughness heights); row 1 + 2^PSI_K (e - PSI_E0) + j covers [2^e (1 + j 2^-K), 2^e (1 + (j+1) 2^-K))
+# with a polynomial in u = |zeta| - c, c its centre: the row index and c come from the high word of |zeta| and u is exact.
+# The nearest singularities are branch points on the stable side (zeta = 1/34.15, 1/15, 1/10.15 for COARE, 1/16 for
+# Paulson) and the poles of zeta^2/(1+zeta^2) at +-i; with 2^PSI_K intervals per binade every interval is at least
+# 2^(K+1) + 1 of its half-widths away from them.  The COARE functions are written as mod_common_coare.f90 writes them, with
+# its truncated literals (as doubles, like the reference build).
+PSI_E0, PSI_K, PSI_DEG, PSI_ZMAX = -7, 2, 11, 50
+
+
+def _lit(s):
+    return mp.mpf(float(s))
+
+
+def psi_coare_m(z):
+    phi_m = mp.power(1 - 15 * z, mp.mpf(1) / 4)
+    k = 2 * mp.log((1 + phi_m) / 2) + mp.log((1 + phi_m * phi_m) / 2) - 2 * mp.atan(phi_m) + mp.pi / 2
+    return _coare_blend(z, k, _coare_conv(mp.power(1 - _lit("10.15") * z, _lit(".3333"))))
+
+
+def psi_coare_h(z):
+    k = 2 * mp.log((1 + mp.sqrt(1 - 15 * z)) / 2)
+    return _coare_blend(z, k, _coare_conv(mp.power(1 - _lit("34.15") * z, _lit(".3333"))))
+
+
+def _coare_conv(phi):
+    return (mp.mpf("1.5") * mp.log((1 + phi + phi * phi) / 3) - _lit("1.7320508") * mp.atan((1 + 2 * phi) / _lit("1.7320508"))
+            + _lit("1.813799447"))
+
+
+def _coare_blend(z, k, c):
+    f = z * z / (1 + z * z)
+    return (1 - f) * k + f * c
+
+
+def psi_paulson_m(z):
+    x = mp.power(1 - 16 * z, mp.mpf(1) / 4)
+    return 2 * mp.log((1 + x) / 2) + mp.log((1 + x * x) / 2) - 2 * mp.atan(x) + mp.pi / 2
+
+
+def psi_paulson_h(z):
+    return 2 * mp.log((1 + mp.sqrt(1 - 16 * z)) / 2)
+
+
+PSI_FUNCS = {"COARE": (psi_coare_m, psi_coare_h), "PAULSON": (psi_paulson_m, psi_paulson_h)}
+
+
+def psi_rows(e0, k):
+    """[(lo, hi, centre)] of |zeta| for every row."""
+    rows = [(mp.mpf(0), mp.mpf(2) ** e0, mp.mpf(0))]
+    e = e0
+    while rows[-1][1] < PSI_ZMAX:
+        for j in range(2 ** k):
+            lo = mp.mpf(2) ** e * (1 + mp.mpf(j) / 2 ** k)
+            hi = lo + mp.mpf(2) ** (e - k)
+            rows.append((lo, hi, (lo + hi) / 2))
+            if hi > PSI_ZMAX:
+                break
+        e += 1
+    return rows
+
+
+def psi_fit(psi, row, deg):
+    """FP64 coefficients c_0..c_deg of the row's polynomial in u (u = |zeta| - centre)."""
+    lo, hi, c = row
+    if c == 0:     # row 0: u * q(u), q of degree deg - 1
+        q = cheb_fit(lambda u: psi(-u) / u, lo, hi, deg - 1)
+        return [0.0] + [float(x) for x in q]
+    return [float(x) for x in cheb_fit(lambda u: psi(-(c + u)), lo - c, hi - c, deg)]
+
+
+def psi_err(psi, row, cs, n=61):
+    """Worst |p(u) - psi| / max(|psi|, 1) over the row (FP64 coefficients, exact arithmetic), both ends included."""
+    lo, hi, c = row
+    worst = mp.mpf(0)
+    for i in range(n):
+        a = lo + (hi - lo) * i / (n - 1)
+        ref = psi(-a) if a != 0 else mp.mpf(0)
+        worst = max(worst, abs(horner_double(cs, a - c) - ref) / max(abs(ref), 1))
+    return worst
+
+
+def psi_tables(deg=PSI_DEG, e0=PSI_E0, k=PSI_K, quiet=False):
+    """Header text of the psi tables and the worst error of each.  In a table, pair j = (c_2j, c_2j+1) of row r is
+    double2 number j * PSI_ROWS + r (pair j of every row contiguous: lanes on different rows hit different banks), psi_m's
+    pairs first, then psi_h's."""
+    rows = psi_rows(e0, k)
+    text = ("// unstable psi_m, psi_h for zeta in [-%d, 0] as piecewise polynomials of degree %d in u = |zeta| - c: row 0 is\n"
+            "// |zeta| < 2^%d (c = 0, c_0 = 0), row 1 + %d (e - %d) + j is [2^e (1 + j/%d), 2^e (1 + (j+1)/%d)), c its centre\n"
+            "constexpr int PSI_E0 = %d, PSI_K = %d, PSI_DEG = %d, PSI_ROWS = %d;\nconstexpr double PSI_ZMAX = %d.;\n"
+            % (PSI_ZMAX, deg, e0, 2 ** k, e0, 2 ** k, 2 ** k, e0, k, deg, len(rows), PSI_ZMAX))
+    worst = {}
+    for fam, fns in PSI_FUNCS.items():
+        tabs = []
+        for name, psi in zip("mh", fns):
+            coefs = [psi_fit(psi, r, deg) for r in rows]
+            errs = [psi_err(psi, r, cs) for r, cs in zip(rows, coefs)]
+            i = max(range(len(rows)), key=lambda i: errs[i])
+            worst[fam + "_" + name] = errs[i]
+            if not quiet:
+                print("psi_%s %-7s deg %d, %d rows: worst |err| / max(|psi|, 1) %.3e (2^%.1f) on |zeta| in [%.4g, %.4g]"
+                      % (name, fam, deg, len(rows), errs[i], mp.log(errs[i], 2), rows[i][0], rows[i][1]))
+            tabs.append(coefs)
+        text += ("// %s: worst |err| / max(|psi|, 1) of psi_m %.2e, psi_h %.2e (coefficients rounded, exact arithmetic)\n"
+                 "alignas(16) ABM_GTABLE double PSI_%s_T[%d] = {\n"
+                 % (fam, worst[fam + "_m"], worst[fam + "_h"], fam, 2 * len(rows) * (deg + 1)) +
+                 ",\n".join(f"    {cs[2 * j].hex()}, {cs[2 * j + 1].hex()}"
+                            for coefs in tabs for j in range((deg + 1) // 2) for cs in coefs) + "\n};\n")
+    return text + "\n", worst
+
+
 def main():
     parts = ["// GENERATED by tools/gen_math_tables.py -- do not edit.\n#pragma once\n\n"
              "#ifndef ABM_TABLE\n#define ABM_TABLE __constant__\n#endif\n"
@@ -170,6 +282,8 @@ def main():
                  % (ESAT_M0, ESAT_M1, ESAT_DEG, ESAT_M0, ESAT_M0, worst[0], ESAT_H, ESAT_M0, len(rows), len(rows) * (ESAT_DEG + 1)) +
                  ",\n".join(f"    {float(cs[2 * j]).hex()}, {float(cs[2 * j + 1]).hex()}"
                              for j in range((ESAT_DEG + 1) // 2) for cs in rows) + "\n};\n\n")
+
+    parts.append(psi_tables()[0])
 
     def hilo(x):
         hi = float(x)
