@@ -42,21 +42,18 @@ def _stale(target: str, deps) -> bool:
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build(force: bool = False, verbose: bool = False, defines=(), tag: str = "") -> str:
-    """Build the library.  `defines`/`tag` produce an experiment variant build/lib<tag>.so
-    (loaded with AEROBULK_GPU_LIB=<path>); the default build is the shipped one."""
+def build(force: bool = False, verbose: bool = False) -> str:
+    """Build the library."""
     os.makedirs(OBJ, exist_ok=True)
     nvcc = _nvcc()
     objs = []
-    lib = LIB if not tag else os.path.join(OBJ, f"libaerobulk_gpu_{tag}.so")
-    extra = [f"-D{d}" for d in defines]
     jobs = []
     for src in SOURCES:
         path = os.path.join(CSRC, src)
-        obj = os.path.join(OBJ, os.path.splitext(src)[0] + (f"_{tag}" if tag else "") + ".o")
+        obj = os.path.join(OBJ, os.path.splitext(src)[0] + ".o")
         objs.append(obj)
         if force or _stale(obj, [path] + HEADERS):
-            cmd = [nvcc, "-ccbin", "/usr/bin/g++"] + ARCH + NVCC_FLAGS + extra + ["-c", path, "-o", obj]
+            cmd = [nvcc, "-ccbin", "/usr/bin/g++"] + ARCH + NVCC_FLAGS + ["-c", path, "-o", obj]
             if src.endswith(".cu") and verbose:
                 cmd += ["-Xptxas", "-v"]
             if verbose:
@@ -65,14 +62,14 @@ def build(force: bool = False, verbose: bool = False, defines=(), tag: str = "")
     for cmd, job in jobs:
         if job.wait() != 0:
             raise subprocess.CalledProcessError(job.returncode, cmd)
-    if force or _stale(lib, objs):
+    if force or _stale(LIB, objs):
         # -z nodelete: the copy threads of ab_copy_pool.hpp must outlive any dlclose of the library
-        cmd = [nvcc, "-ccbin", "/usr/bin/g++"] + ARCH + ["-shared", "-o", lib] + objs + [
+        cmd = [nvcc, "-ccbin", "/usr/bin/g++"] + ARCH + ["-shared", "-o", LIB] + objs + [
             "-cudart", "static", "-Xlinker", "--exclude-libs,ALL", "-Xlinker", "-z", "-Xlinker", "nodelete"]
         if verbose:
             print(" ".join(cmd), flush=True)
         subprocess.check_call(cmd)
-    return lib
+    return LIB
 
 
 if __name__ == "__main__":

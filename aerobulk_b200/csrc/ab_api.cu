@@ -40,19 +40,11 @@
 
 namespace {
 
-constexpr int MAX_CHUNKS = 16;          // capacity; the number used is chunk_limit() (default 6, measured best)
+constexpr int MAX_CHUNKS = 16;          // capacity of a chunk plan (plan_chunks)
+// the staged pipelines (plan_chunks kinds 1 and 3): chunks of at least MIN_CHUNK_POINTS, at most STAGED_CHUNKS of them
+// (6, measured best on B200) or SPEC_CHUNKS with the speculative AEROBULK_INIT
+constexpr int STAGED_CHUNKS = 6, SPEC_CHUNKS = 12;
 constexpr long long MIN_CHUNK_POINTS = 200000;
-
-// tuning knobs of the host-array pipeline (experiments: tools/diag_e2e.py)
-int chunk_limit()
-{
-    static int v = [] {
-        const char *e = getenv("AEROBULK_GPU_MAX_CHUNKS");
-        int k = e ? atoi(e) : 6;
-        return k < 1 ? 1 : (k > MAX_CHUNKS ? MAX_CHUNKS : k);
-    }();
-    return v;
-}
 // Zero-copy host-array calls.  When EVERY array of a call is pinned host memory (cudaHostAlloc / cudaHostRegister: it has a
 // device alias under unified virtual addressing) the flux kernel loads its inputs from and stores its outputs to the
 // caller's arrays directly: each byte crosses PCIe once, both directions busy for the whole launch, no staging, no
@@ -83,15 +75,6 @@ template <class T>
 T *elem_at(T *p, long long i, size_t es)
 {
     return p ? p + i * (long long)es : nullptr;
-}
-long long min_chunk_points()
-{
-    static long long v = [] {
-        const char *e = getenv("AEROBULK_GPU_MIN_CHUNK_POINTS");
-        long long k = e ? atoll(e) : MIN_CHUNK_POINTS;
-        return k < 2048 ? 2048 : k;
-    }();
-    return v;
 }
 
 
@@ -831,15 +814,6 @@ int deferred_errors()
     return rc ? rc : check_bad_flag(nullptr, nullptr);
 }
 
-int spec_chunk_limit()
-{
-    static int v = [] {
-        const char *e = getenv("AEROBULK_GPU_SPEC_CHUNKS");
-        int k = e ? atoi(e) : 12;
-        return k < 2 ? 2 : (k > MAX_CHUNKS ? MAX_CHUNKS : k);
-    }();
-    return v;
-}
 // Row-block chunk plan of a host-array call: cstart[0..nchunks], boundaries on multiples of 2048 points (whole sort
 // windows / thread blocks).
 //   kind 0: one chunk (device arrays, zero-copy on pinned arrays);
@@ -858,11 +832,11 @@ int plan_chunks(long long n, int kind, long long *cstart)
         nchunks = (int)((n + bounce_chunk_points() - 1) / bounce_chunk_points());
         nchunks = nchunks < 1 ? 1 : (nchunks > MAX_CHUNKS ? MAX_CHUNKS : nchunks);
     } else if (kind == 1) {
-        nchunks = (int)(n / min_chunk_points());
-        nchunks = nchunks < 1 ? 1 : (nchunks > chunk_limit() ? chunk_limit() : nchunks);
+        nchunks = (int)(n / MIN_CHUNK_POINTS);
+        nchunks = nchunks < 1 ? 1 : (nchunks > STAGED_CHUNKS ? STAGED_CHUNKS : nchunks);
     } else if (kind == 3) {
-        nchunks = (int)(n / min_chunk_points());
-        nchunks = nchunks < 1 ? 1 : (nchunks > spec_chunk_limit() ? spec_chunk_limit() : nchunks);
+        nchunks = (int)(n / MIN_CHUNK_POINTS);
+        nchunks = nchunks < 1 ? 1 : (nchunks > SPEC_CHUNKS ? SPEC_CHUNKS : nchunks);
     }
     double w[MAX_CHUNKS], wsum = 0.;
     for (int c = 0; c < nchunks; ++c) {
@@ -1086,7 +1060,7 @@ int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, d
             return fail(AEROBULK_GPU_ERR_STATE, "warm-layer state missing or of another size at jt=%d (no jt==1 call for this session?)", jt);
     }
 
-    // Stability sort (classify_kernel).  Auto policy = where it measured faster on B200 (tools/exp_sort.sh, KBENCH_SORT=1/2,
+    // Stability sort (classify_kernel).  Auto policy = where it measured faster on B200 (kbench with KBENCH_SORT=1/2,
     // profiles/exp_sort_r02d.txt, 4320x2160): everything but NCAR (too little work per point: 0.97 -> 1.06 ms).  Since the
     // proxy follows the skin temperature (T_s starts 0.25 K below the SST and carries the warm-layer increment) and keeps
     // the doubtful points to themselves, ECMWF + skin gains the most (5.01 -> 4.54 ms by day, 4.46 -> 3.88 ms by night;

@@ -26,22 +26,7 @@
 
 namespace abd {
 
-#ifndef AB_CS_UNROLL
-#define AB_CS_UNROLL 1   // cool-skin passes rolled: the delta code exists once (instruction-cache footprint)
-#endif
-constexpr int CS_UNROLL = AB_CS_UNROLL;
-#ifndef AB_PASS_UNROLL
-#define AB_PASS_UNROLL 1   // cool-skin pass and warm-layer pass rolled: UPDATE_QNSOL_TAU and q_sat exist once in the loop body
-#endif
-constexpr int PASS_UNROLL = AB_PASS_UNROLL;
 #define ABD __device__ __forceinline__
-// heavy helpers can be kept out of line (one shared body instead of 2-5 inlined copies) to shrink the
-// instruction footprint: -DAB_NOINLINE=1
-#if defined(AB_NOINLINE) && AB_NOINLINE
-#define ABD_HEAVY static __device__ __noinline__
-#else
-#define ABD_HEAVY __device__ __forceinline__
-#endif
 
 // FP64 literals in the constant bank.  ptxas builds a double that does not fit a 32-bit immediate with two moves
 // (UMOV / IMAD.MOV): ~20 % of the instructions the COARE + skin kernel executed in the round-1b profile.  KC(x) puts
@@ -141,7 +126,7 @@ constexpr double INV_GRAV = 1. / GRAV;
 ABD double virt_temp(double T, double q) { return T * (1. + KC(RCTV0) * q); }           // :247-269
 
 // Goff (1957) saturation vapour pressure [Pa], :777-800 (rt0, not the triple point)
-ABD_HEAVY double e_sat_goff(double T)
+ABD double e_sat_goff(double T)
 {
     const double zta = abm::dmax(T, 180.);
     const double ztmp = fdiv(KC(RT0), zta);
@@ -258,9 +243,9 @@ ABD Flux bulk_formula(const AirZu &air, double Ts, double qs, double tha, double
 }
 
 // UPDATE_QNSOL_TAU_SCLR, :1059-1103 -> non-solar flux, stress and latent flux
-ABD_HEAVY void update_qnsol_tau(const AirZu &air, double Ts, double qs, double tha, double qa, double us, double ts,
-                                double qst, double wnd, double Ub, double rlw,
-                                double &Qns, double &Tau, double &Qlat)
+ABD void update_qnsol_tau(const AirZu &air, double Ts, double qs, double tha, double qa, double us, double ts,
+                          double qst, double wnd, double Ub, double rlw,
+                          double &Qns, double &Tau, double &Qlat)
 {
     const double dt = floor_abs(tha - Ts, KC(1.E-09));
     const double dq = floor_abs(qa - qs, KC(1.E-12));
@@ -579,7 +564,7 @@ ABD double cool_skin_dT(double alpha, double Qsw, double Qnsol, double us, doubl
     // delta(Qnsol), then 4 x { solar absorption fr(delta) -> Qabs -> delta(Qabs) }: one rolled loop so that
     // the delta code exists once (instruction-cache footprint)
     double Qabs = Qnsol, d = 0.;
-#pragma unroll CS_UNROLL
+#pragma unroll 1   // cool-skin passes rolled: the delta code exists once (instruction-cache footprint)
     for (int jc = 0; jc < 5; ++jc) {
         const double d_prev = d;
         if (jc > 0) {
@@ -935,7 +920,7 @@ ABD Coeffs solve_coare(const Uniform &u, const PointIn &p, WarmLayer &wl, Diag &
             // iwait = MOD(nb_iter, jit) == 0 (mod_blk_coare3p6.f90:370), from a host-computed bit mask: the integer
             // division cost 1.2 % of the kernel
             const bool commit = (jit < 64) ? ((u.wl_commit_mask >> jit) & 1ull) != 0ull : (u.nb_iter % jit) == 0;
-#pragma unroll PASS_UNROLL
+#pragma unroll 1   // cool-skin pass and warm-layer pass rolled: UPDATE_QNSOL_TAU and q_sat exist once in the loop body
             for (int pass = CS ? 0 : 1; pass < (WL ? 2 : 1); ++pass) {
                 const double Ts_q = Ts;
                 if (CS && pass == 0) {
@@ -1098,7 +1083,7 @@ ABD Coeffs solve_ecmwf(const Uniform &u, const PointIn &p, WarmLayer &wl, Diag &
         if (SKIN) {
             // pass 0: cool skin, pass 1: warm layer -- advanced at every iteration (SURVEY 8a quirk 2)
             const AirZu air = air_at_zu(u.zu, t_zu, q_zu, p.slp);
-#pragma unroll PASS_UNROLL
+#pragma unroll 1   // cool-skin pass and warm-layer pass rolled: UPDATE_QNSOL_TAU and q_sat exist once in the loop body
             for (int pass = CS ? 0 : 1; pass < (WL ? 2 : 1); ++pass) {
                 double Qns, Tau, Qlat;
                 update_qnsol_tau(air, Ts, qs_, t_zu, q_zu, us, ts, qst, p.wnd, Ub, p.rlw, Qns, Tau, Qlat);

@@ -28,21 +28,13 @@ namespace abk {
 
 using namespace abd;
 
-#ifndef AB_FLUX_BLOCK
-#define AB_FLUX_BLOCK 256
-#endif
+static constexpr int FLUX_BLOCK = 256;
 // Resident blocks per SM (x 256 threads).  Skin kernels: 3 (24 warps/SM, <= 85 registers: the ~28 doubles they carry across
 // the bulk iteration do not fit 64 registers without spilling into the loop).  Kernels without skin: 4 (32 warps/SM, 64
 // registers; their few spills sit outside the loop).  Measured at 4320x2160 (profiles/exp_variants_r02i.txt, 256x3 ->
 // 256x4): NCAR 0.900 -> 0.877 ms, ANDREAS 1.372 -> 1.322, COARE 3.6 1.900 -> 1.842; COARE 3.6 + skin 3.147 -> 3.204 (night),
 // ECMWF + skin 4.126 -> 4.226.  128 x 7 (73 registers) loses everywhere but ANDREAS.
-#ifndef AB_MIN_BLOCKS
-#define AB_MIN_BLOCKS 3
-#endif
-#ifndef AB_MIN_BLOCKS_NOSKIN
-#define AB_MIN_BLOCKS_NOSKIN 4
-#endif
-static constexpr int FLUX_BLOCK = AB_FLUX_BLOCK;
+static constexpr int MIN_BLOCKS = 3, MIN_BLOCKS_NOSKIN = 4;
 
 // Cheap proxy of the air-sea virtual potential temperature difference [K], whose sign is the stability class every
 // psi_m / psi_h evaluation branches on.  Only used to GROUP points (performance); the physics never sees it.
@@ -52,15 +44,8 @@ static constexpr int FLUX_BLOCK = AB_FLUX_BLOCK;
 // (profiles/exp_sort_r02d.txt; band 0 / 0.1 / 0.25 / 0.5): COARE 3.6 2.146 / 2.080 / 2.099 / 2.136 ms, ECMWF 2.318 /
 // 2.233 / 2.248 / 2.306 ms, COARE 3.6 + skin by day 4.495 / 4.459 / 4.411 / 4.377 ms and by night 3.635 / 3.538 / 3.449 /
 // 3.419 ms, ECMWF + skin 4.731 / 4.631 / 4.555 / 4.535 ms: the skin schemes move T_s by a few tenths of a kelvin more.
-#ifndef AB_SORT_BAND
-#define AB_SORT_BAND 0.15
-#endif
-#ifndef AB_SORT_BAND_SKIN
-#define AB_SORT_BAND_SKIN 0.5
-#endif
-#ifndef AB_SORT_BAND_NOQ
-#define AB_SORT_BAND_NOQ 1.0 // the same when the humidity is rh / dp (the proxy ignores it)
-#endif
+static constexpr float SORT_BAND = 0.15f, SORT_BAND_SKIN = 0.5f;
+static constexpr float SORT_BAND_NOQ = 1.0f;   // the same when the humidity is rh / dp (the proxy ignores it)
 // Per-point arrays of element type T (FluxArgs, StatsArgs): `ld` widens to FP64 (exact for float), `st` rounds once to
 // nearest.  With T = double both are the plain load and store.
 template <class T>
@@ -110,7 +95,7 @@ __device__ __forceinline__ void classify_block(const FluxArgs &a, unsigned short
     const long long base = (long long)blockIdx.x * SORT_WIN;
     const int lane = tid & 31, w = tid >> 5;
     const int ihum = a.init_dev ? __ldg(a.init_dev) : a.ihum;
-    const float band = (ihum != 0) ? (float)AB_SORT_BAND_NOQ : (skin ? (float)AB_SORT_BAND_SKIN : (float)AB_SORT_BAND);
+    const float band = (ihum != 0) ? SORT_BAND_NOQ : (skin ? SORT_BAND_SKIN : SORT_BAND);
     const bool wl = skin && !a.first_step && a.dT_wl != nullptr;
     int cls[SORT_ITEMS];
 #pragma unroll
@@ -286,7 +271,7 @@ __device__ __forceinline__ void flux_point(const FluxArgs &a, unsigned tid)
 }
 
 template <int ALGO, bool SKIN, bool ZTEQ>
-__global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOCKS_NOSKIN) flux_kernel(const FluxArgs a)
+__global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? MIN_BLOCKS : MIN_BLOCKS_NOSKIN) flux_kernel(const FluxArgs a)
 {
     flux_point<double, ALGO, SKIN, ZTEQ>(a, threadIdx.x);
 }
@@ -294,7 +279,7 @@ __global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOC
 // flux_kernel on per-point arrays of element type T, same launch bounds.  T is a type argument: the kernel-matrix
 // census of the FP64 kernels takes the instantiations whose template arguments are all int or bool.
 template <class T, int ALGO, bool SKIN, bool ZTEQ>
-__global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? AB_MIN_BLOCKS : AB_MIN_BLOCKS_NOSKIN) flux_io_kernel(const FluxArgs a)
+__global__ void __launch_bounds__(FLUX_BLOCK, SKIN ? MIN_BLOCKS : MIN_BLOCKS_NOSKIN) flux_io_kernel(const FluxArgs a)
 {
     flux_point<T, ALGO, SKIN, ZTEQ>(a, threadIdx.x);
 }
@@ -320,7 +305,7 @@ cudaError_t launch_flux(int algo, bool skin, bool zteq, size_t elem, const FluxA
 // turb_kernel<ALGO,CS,WL,ZTEQ>: the direct TURB_* entry (SURVEY.md 8f row 1) on the same solvers
 // ---------------------------------------------------------------------------
 template <int ALGO, bool CS, bool WL, bool ZTEQ>
-__global__ void __launch_bounds__(FLUX_BLOCK, (CS || WL) ? AB_MIN_BLOCKS : AB_MIN_BLOCKS_NOSKIN) turb_kernel(const TurbArgs a)
+__global__ void __launch_bounds__(FLUX_BLOCK, (CS || WL) ? MIN_BLOCKS : MIN_BLOCKS_NOSKIN) turb_kernel(const TurbArgs a)
 {
     abm::load_tables<PSI_TABLES_OF<ALGO>>();
     const long long i = (long long)blockIdx.x * FLUX_BLOCK + threadIdx.x;
@@ -456,17 +441,18 @@ static constexpr int STATS_REDO_SLOT = NSTATS - 1;
 // same order: the row is bit-identical to what the one-kernel version produced).  NaNs: `x < lo || x > hi` is false for a
 // NaN (the reference does not mask it) and the (v < acc ? v : acc) min / max skip it -- the derived test agrees.
 // rad_lw is held against both radiation ranges (the reference's prsw=rad_lw slip): fields 7 and 8 are the same values.
-template <class T, int UNROLL>
+static constexpr int STATS_FAST_UNROLL = 3;   // 120 registers, no spills, 2 blocks/SM x 21 loads in flight per thread
+template <class T>
 __device__ __forceinline__ void stats_fast_body(const StatsArgs &a, double (&sum)[8], double (&mn)[8], double (&mx)[8], double &cnt)
 {
     const bool rad = (a.rad_lw != nullptr);
     const long long stride = (long long)gridDim.x * STATS_BLOCK;
-    // UNROLL points per trip with all their loads issued first; a thread meets its points (base + k stride) in the same
-    // order as in stats_fix_kernel whatever the unroll factor: the sums add up identically
-    for (long long i0 = (long long)blockIdx.x * STATS_BLOCK + threadIdx.x; i0 < a.n; i0 += stride * UNROLL) {
-        double in[UNROLL][7];
+    // STATS_FAST_UNROLL points per trip with all their loads issued first; a thread meets its points (base + k stride) in
+    // the same order as in stats_fix_kernel whatever the unroll factor: the sums add up identically
+    for (long long i0 = (long long)blockIdx.x * STATS_BLOCK + threadIdx.x; i0 < a.n; i0 += stride * STATS_FAST_UNROLL) {
+        double in[STATS_FAST_UNROLL][7];
 #pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
+        for (int u = 0; u < STATS_FAST_UNROLL; ++u) {
             const long long i = i0 + u * stride;
             const long long j = (i < a.n) ? i : i0;
             in[u][0] = ld<T>(a.sst, j);
@@ -478,7 +464,7 @@ __device__ __forceinline__ void stats_fast_body(const StatsArgs &a, double (&sum
             in[u][6] = rad ? ld<T>(a.rad_lw, j) : 0.;
         }
 #pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
+        for (int u = 0; u < STATS_FAST_UNROLL; ++u) {
             if (i0 + u * stride >= a.n) break;
             double v[8];
             v[0] = in[u][0];
@@ -500,9 +486,6 @@ __device__ __forceinline__ void stats_fast_body(const StatsArgs &a, double (&sum
     }
 }
 
-#ifndef AB_STATS_UNROLL
-#define AB_STATS_UNROLL 3   // 120 registers, no spills, 2 blocks/SM x 21 loads in flight per thread
-#endif
 template <class T>
 __device__ __forceinline__ void stats_fast_block(const StatsArgs &a, unsigned tid)
 {
@@ -513,7 +496,7 @@ __device__ __forceinline__ void stats_fast_block(const StatsArgs &a, unsigned ti
         mn[f] = DBL_MAX;
         mx[f] = -DBL_MAX;
     }
-    stats_fast_body<T, AB_STATS_UNROLL>(a, sum, mn, mx, cnt);   // a thread meets its points in the same order for any unroll
+    stats_fast_body<T>(a, sum, mn, mx, cnt);
     // block reduction in the order of the one-kernel version: lanes by shuffle, then the warps in index order
     __shared__ double sm[STATS_BLOCK / 32][1 + 3 * 8];
     const int lane = tid & 31, warp = tid >> 5;

@@ -23,10 +23,8 @@
 #include <cstdint>
 #include <cstring>
 #define ABM_FN static inline
-#define ABM_BIG static inline
 #define ABM_TABLE static const
 #define ABM_GTABLE static const
-#define ABM_LDG(p) (*(p))
 struct double2 { double x, y; };
 namespace abm {
 static inline int hi_word(double x) { int64_t b; std::memcpy(&b, &x, 8); return (int)(b >> 32); }
@@ -46,14 +44,6 @@ static inline double pow_seed(double y, float p) { return (double)(float)std::po
 #else
 #include <cuda_runtime.h>
 #define ABM_FN __device__ __forceinline__
-#define ABM_LDG(p) __ldg(p)
-// -DABM_NOINLINE=1 keeps exp/log/atan out of line (one body per kernel): smaller instruction footprint
-// at the price of call overhead and less interleaving
-#if defined(ABM_NOINLINE) && ABM_NOINLINE
-#define ABM_BIG static __device__ __noinline__
-#else
-#define ABM_BIG __device__ __forceinline__
-#endif
 namespace abm {
 ABM_FN int hi_word(double x) { return __double2hiint(x); }
 ABM_FN int lo_word(double x) { return __double2loint(x); }
@@ -158,78 +148,18 @@ ABM_FN double fast_cbrt(double x)
     return x * (r * r);
 }
 
-// p(r) ~ exp(r) on |r| <= ln2/2 (Estrin: depth 5 instead of 11 dependent FMAs), then * 2^k through
-// the exponent field
-ABM_FN double exp_core(double r, int k)
-{
-    const double r2 = r * r, r4 = r2 * r2, r8 = r4 * r4;
-    const double a0 = fma(EXP_C[1], r, EXP_C[0]), a1 = fma(EXP_C[3], r, EXP_C[2]), a2 = fma(EXP_C[5], r, EXP_C[4]);
-    const double a3 = fma(EXP_C[7], r, EXP_C[6]), a4 = fma(EXP_C[9], r, EXP_C[8]), a5 = fma(EXP_C[11], r, EXP_C[10]);
-    const double b0 = fma(a1, r2, a0), b1 = fma(a3, r2, a2), b2 = fma(a5, r2, a4);
-    const double p = fma(b2, r8, fma(b1, r4, b0));
-    return make_double(hi_word(p) + (k << 20), lo_word(p));
-}
-
-ABM_BIG double dexp_poly(double x)
-{
-    const double MAGIC = 6755399441055744.0;   // 1.5 * 2^52: adding it rounds to nearest integer
-    const double t = fma(x, MATH_K[K_L2E], MAGIC);
-    const int k = lo_word(t);
-    const double kf = t - MAGIC;
-    double r = fma(kf, -MATH_K[K_LN2_HI], x);
-    r = fma(kf, -MATH_K[K_LN2_LO], r);
-    const double v = exp_core(r, k);
-    return (x < -700.) ? 0. : v;
-}
-
-ABM_BIG double dexp10_poly(double x)
-{
-    const double MAGIC = 6755399441055744.0;
-    const double t = fma(x, MATH_K[K_L2T], MAGIC);
-    const int k = lo_word(t);
-    const double kf = t - MAGIC;
-    double r = fma(kf, -MATH_K[K_LG2_HI], x);
-    r = fma(kf, -MATH_K[K_LG2_LO], r);
-    const double v = exp_core(r * MATH_K[K_LN10], k);
-    return (x < -304.) ? 0. : v;
-}
-
-// log(x) = k ln2 + log(m), m in [sqrt(2)/2, sqrt(2)); log(m) = 2 atanh(s), s = (m-1)/(m+1)
-ABM_BIG double dlog_poly(double x)
-{
-    int hx = hi_word(x);
-    int k = (hx >> 20) - 1023;
-    hx &= 0x000fffff;
-    const int i = (hx + 0x95f64) & 0x100000;
-    hx |= (i ^ 0x3ff00000);
-    k += (i >> 20);
-    const double f = make_double(hx, lo_word(x)) - 1.0;
-    const double s = f * fast_rcp(2.0 + f);
-    const double z = s * s;
-    const double z2 = z * z;
-    const double a0 = fma(LOG_C[1], z, LOG_C[0]), a1 = fma(LOG_C[3], z, LOG_C[2]), a2 = fma(LOG_C[5], z, LOG_C[4]);
-    const double p = fma(fma(LOG_C[6], z2, a2), z2 * z2, fma(a1, z2, a0));
-    const double R = z * p;
-    const double hfsq = 0.5 * f * f;
-    const double dk = (double)k;
-    return dk * MATH_K[K_LN2_HI] - ((hfsq - fma(s, hfsq + R, dk * MATH_K[K_LN2_LO])) - f);
-}
-
 // ---------------------------------------------------------------------------
-// Table-driven exp / log (default): a 64-entry table of 2^(j/64) and a 256-entry table of
+// Table-driven exp / log: a 64-entry table of 2^(j/64) and a 256-entry table of
 // {1/c_j, -log(1/c_j)} (4.5 KB, copied to shared memory by each block) shrink the polynomials to degree 3 / 4:
 // 10 FP64 instructions per exp instead of 18, 13 per log instead of 23 (no reciprocal).
 // ---------------------------------------------------------------------------
-#ifndef ABM_SMEM_TABLES
-#define ABM_SMEM_TABLES 1   // measured 3 % faster than __ldg of the global tables (64-bit address arithmetic)
-#endif
 // which psi tables a kernel reads (psi_table): load_tables copies only those
 enum { PSI_TABLES_NONE = 0, PSI_TABLES_COARE = 1, PSI_TABLES_PAULSON = 2, PSI_TABLES_ALL = 3 };
-#if ABM_SMEM_TABLES && !defined(ABM_HOST_TEST)
+#ifndef ABM_HOST_TEST
 // block-local copies of the tables in shared memory (4.5 KB, 3.2 KB of e_sat coefficients and 10 KB per family of psi
-// coefficients; 32-bit addressing, LDS instead of LDG); every kernel must call abm::load_tables() (all threads) before the
-// first exp/log/esat_table/psi_table, naming in PSI every psi family it evaluates from a table (a shared array a kernel
-// does not reference takes no shared memory)
+// coefficients; 32-bit addressing, LDS instead of LDG: measured 3 % faster than __ldg of the global tables); every kernel
+// must call abm::load_tables() (all threads) before the first exp/log/esat_table/psi_table, naming in PSI every psi family
+// it evaluates from a table (a shared array a kernel does not reference takes no shared memory)
 __shared__ double S_EXP_T[64];
 __shared__ double S_LOG_T[512];
 __shared__ __align__(16) double S_ESAT_T[8 * ESAT_ROWS];
@@ -256,13 +186,14 @@ ABM_FN void load_tables()
 #define ABM_PSI_T(fam) S_PSI_##fam##_T
 #define ABM_PSI_T2(t, i) reinterpret_cast<const double2 *>(t)[i]
 #else
+// the host build reads the arrays themselves
 template <int PSI = PSI_TABLES_ALL>
 ABM_FN void load_tables() {}
-#define ABM_EXP_T(i) ABM_LDG(&EXP_T[i])
-#define ABM_LOG_T(i) ABM_LDG(&LOG_T[i])
-#define ABM_ESAT_T2(i) ABM_LDG(reinterpret_cast<const double2 *>(ESAT_T) + (i))
+#define ABM_EXP_T(i) EXP_T[i]
+#define ABM_LOG_T(i) LOG_T[i]
+#define ABM_ESAT_T2(i) reinterpret_cast<const double2 *>(ESAT_T)[i]
 #define ABM_PSI_T(fam) PSI_##fam##_T
-#define ABM_PSI_T2(t, i) ABM_LDG(reinterpret_cast<const double2 *>(t) + (i))
+#define ABM_PSI_T2(t, i) reinterpret_cast<const double2 *>(t)[i]
 #endif
 
 // exp(r) for |r| <= ln2/128 times 2^(k/64), k = 64 m + j
@@ -276,7 +207,7 @@ ABM_FN double expt_core(double r, int k)
     const double v = fma(T, fma(r2, q, r), T);
     return make_double(hi_word(v) + ((k >> 6) << 20), lo_word(v));
 }
-ABM_BIG double dexp_table(double x)
+ABM_FN double dexp_table(double x)
 {
     const double MAGIC = 6755399441055744.0;
     const double t = fma(x, MATH_K[K_L2E64], MAGIC);
@@ -288,7 +219,7 @@ ABM_BIG double dexp_table(double x)
     return (x < -700.) ? 0. : v;
 }
 // the same without the underflow guard, for call sites whose argument is provably inside [-700, 700]
-ABM_BIG double dexp_table_bounded(double x)
+ABM_FN double dexp_table_bounded(double x)
 {
     const double MAGIC = 6755399441055744.0;
     const double t = fma(x, MATH_K[K_L2E64], MAGIC);
@@ -298,7 +229,7 @@ ABM_BIG double dexp_table_bounded(double x)
     r = fma(kf, -MATH_K[K_LN2_64_LO], r);
     return expt_core(r, k);
 }
-ABM_BIG double dexp10_table(double x)
+ABM_FN double dexp10_table(double x)
 {
     const double MAGIC = 6755399441055744.0;
     const double t = fma(x, MATH_K[K_L2T64], MAGIC);
@@ -309,7 +240,7 @@ ABM_BIG double dexp10_table(double x)
     const double v = expt_core(r * MATH_K[K_LN10], k);
     return (x < -304.) ? 0. : v;
 }
-ABM_BIG double dexp10_table_bounded(double x)   // |x| <= 300 guaranteed by the caller
+ABM_FN double dexp10_table_bounded(double x)   // |x| <= 300 guaranteed by the caller
 {
     const double MAGIC = 6755399441055744.0;
     const double t = fma(x, MATH_K[K_L2T64], MAGIC);
@@ -321,7 +252,7 @@ ABM_BIG double dexp10_table_bounded(double x)   // |x| <= 300 guaranteed by the 
 }
 // log(x) = e ln2 + lc_j + log1p(m rc_j - 1), m in [0.708, 1.416) (so that x ~ 1 has e = 0 and the exact
 // entry c = 1), j = interval of m's hi word
-ABM_BIG double dlog_table(double x)
+ABM_FN double dlog_table(double x)
 {
     const int hx = hi_word(x);
     const int e = (hx - 0x3fe6a800) >> 20;
@@ -340,19 +271,11 @@ ABM_BIG double dlog_table(double x)
     return fma(de, MATH_K[K_LN2_HI], lc) + fma(de, MATH_K[K_LN2_LO], lp);
 }
 
-#if defined(ABM_POLY_MATH) && ABM_POLY_MATH
-ABM_FN double dexp(double x) { return dexp_poly(x); }
-ABM_FN double dexp10(double x) { return dexp10_poly(x); }
-ABM_FN double dexp_b(double x) { return dexp_poly(x); }
-ABM_FN double dexp10_b(double x) { return dexp10_poly(x); }
-ABM_FN double dlog(double x) { return dlog_poly(x); }
-#else
 ABM_FN double dexp(double x) { return dexp_table(x); }
 ABM_FN double dexp10(double x) { return dexp10_table(x); }
 ABM_FN double dexp_b(double x) { return dexp_table_bounded(x); }      // argument inside [-700, 700]
 ABM_FN double dexp10_b(double x) { return dexp10_table_bounded(x); }  // argument inside [-300, 300]
 ABM_FN double dlog(double x) { return dlog_table(x); }
-#endif
 
 ABM_FN double dlog10(double x) { return dlog(x) * MATH_K[K_LOG10E]; }
 
@@ -436,7 +359,7 @@ ABM_FN double atan_core(double t)
     return fma(t * z, q, t);
 }
 // atan: |x| <= tan(pi/8): poly; <= tan(3pi/8): pi/4 + atan((x-1)/(x+1)); else pi/2 - atan(1/x)
-ABM_BIG double datan(double x)
+ABM_FN double datan(double x)
 {
     const double ax = fabs(x);
     double num = ax, den = 1.0, bhi = 0., blo = 0.;
@@ -453,7 +376,7 @@ ABM_BIG double datan(double x)
 // inner argument stays inside [-tan(pi/8), tan(pi/8)] for ALL x in [1, inf): the polynomial's range, one formula, no
 // range selection (the three-way selection of datan cost 2 compares and ~10 predicated moves per call: 18 % of the
 // register moves the COARE + skin kernel executed) and no sign handling.
-ABM_BIG double datan_ge1(double x)
+ABM_FN double datan_ge1(double x)
 {
     const double c = MATH_K[K_TAN3PIO8];
     const double a = atan_core((x - c) * fast_rcp(fma(c, x, 1.0)));

@@ -15,14 +15,8 @@ namespace abk {
 
 using namespace abd;
 
-#ifndef AB_SERIES_BLOCK
-#define AB_SERIES_BLOCK 64
-#endif
-#ifndef AB_SERIES_MIN_BLOCKS
-#define AB_SERIES_MIN_BLOCKS 8
-#endif
-static constexpr int SERIES_BLOCK = AB_SERIES_BLOCK;
-static constexpr int SERIES_MIN_BLOCKS = AB_SERIES_MIN_BLOCKS;
+static constexpr int SERIES_BLOCK = 64;
+static constexpr int SERIES_MIN_BLOCKS = 8;
 
 template <int ALGO, bool SKIN, bool ZTEQ>
 __global__ void __launch_bounds__(SERIES_BLOCK, SERIES_MIN_BLOCKS) series_kernel(const SeriesArgs a)

@@ -10,7 +10,7 @@ from typing import Optional
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# AEROBULK_GPU_LIB selects an experiment build (see aerobulk_b200/build.py); default: the in-tree library
+# AEROBULK_GPU_LIB loads another build of the library (a parent commit's, for A/B runs); default: the in-tree library
 _SO = os.environ.get("AEROBULK_GPU_LIB") or os.path.join(_HERE, "libaerobulk_gpu.so")
 _dp = C.POINTER(C.c_double)
 _ip = C.POINTER(C.c_int)

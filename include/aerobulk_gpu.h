@@ -29,9 +29,8 @@
  * (cudaHostAlloc / cudaHostRegister) the kernels read and write the caller's memory directly over PCIe ("zero-copy":
  * same results, ~20 % faster end to end, no staging memory).
  * Environment: AEROBULK_GPU_DEVICE (or LOCAL_RANK) device ordinal; AEROBULK_GPU_ZEROCOPY=0 staged copies even for pinned
- * arrays (and no pinned slab for pageable ones); AEROBULK_GPU_MAX_CHUNKS / AEROBULK_GPU_MIN_CHUNK_POINTS pipeline
- * tuning; pageable arrays: AEROBULK_GPU_BOUNCE=0 driver-staged
- * copies, AEROBULK_GPU_HOST_THREADS copy threads (default: 3/4 of the CPUs the process may run on, at most 12),
+ * arrays (and no pinned slab for pageable ones); pageable arrays: AEROBULK_GPU_BOUNCE=0 driver-staged copies,
+ * AEROBULK_GPU_HOST_THREADS copy threads (default: 3/4 of the CPUs the process may run on, at most 12),
  * AEROBULK_GPU_BOUNCE_CHUNK_POINTS, AEROBULK_GPU_COPY_STREAMING=0 plain instead of non-temporal stores,
  * AEROBULK_GPU_BOUNCE_MAX_MB largest pinned slab the library may allocate for them (default 12288; beyond it, or when the
  * host refuses the allocation, the driver-staged copies are used).

@@ -13,9 +13,6 @@ void abm_eval(int fn, const double *x, const double *y, double *out, long n)
         case 4: out[i] = abm::datan(x[i]); break;
         case 5: out[i] = abm::dpowr(x[i], y[i]); break;
         case 6: out[i] = abm::fast_rcp(x[i]); break;
-        case 7: out[i] = abm::dexp_poly(x[i]); break;
-        case 8: out[i] = abm::dexp10_poly(x[i]); break;
-        case 9: out[i] = abm::dlog_poly(x[i]); break;
         case 10: out[i] = abm::fast_rsqrt(x[i]); break;
         case 11: out[i] = abm::fast_rcbrt(x[i]); break;
         case 12: out[i] = abm::fast_r4rt(x[i]); break;

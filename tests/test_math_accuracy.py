@@ -53,28 +53,24 @@ N = 4000
 
 def test_exp(abm):
     x = np.concatenate([RNG.uniform(-60, 60, N), RNG.uniform(-1, 1, N), RNG.uniform(-700, -600, 200), [0.0, -0.0, 1e-300]])
-    assert _relerr(abm(0, x), x, mp.exp) <= 4 * ULP          # table-driven (default)
-    assert _relerr(abm(7, x), x, mp.exp) <= 4 * ULP          # polynomial variant
+    assert _relerr(abm(0, x), x, mp.exp) <= 4 * ULP
     assert (abm(0, np.array([-701.0, -1500.0, -1e9])) == 0).all()     # flush (EXP(-zHwl/0.014) in WL_COARE)
 
 
 def test_exp10(abm):
     x = np.concatenate([RNG.uniform(-10, 10, N), RNG.uniform(-0.2, 4.0, N)])   # e_sat uses [-0.2, 3.8]
     assert _relerr(abm(1, x), x, lambda v: mp.mpf(10) ** v) <= 4 * ULP
-    assert _relerr(abm(8, x), x, lambda v: mp.mpf(10) ** v) <= 4 * ULP
 
 
 def test_log_log10(abm):
     x = np.concatenate([np.exp(RNG.uniform(-40, 40, N)), RNG.uniform(0.5, 2.0, N), [1.0, 2.0, 0.5, 1e-9, 10.0]])
     x = np.concatenate([x, 1.0 + RNG.uniform(-3e-3, 3e-3, N), np.nextafter(1.0, [0.0, 2.0])])
     mp.mp.dps = 50
-    for fn in (2, 9):                                   # table-driven (default), polynomial variant
-        got = abm(fn, x)
-        for xi, gi in zip(x, got):
-            ref = mp.log(mp.mpf(float(xi)))
-            err = abs(mp.mpf(float(gi)) - ref)
-            assert err <= 4 * ULP * abs(ref), (fn, xi, gi, float(ref))
-        assert abm(fn, np.array([1.0]))[0] == 0.0
+    for xi, gi in zip(x, abm(2, x)):
+        ref = mp.log(mp.mpf(float(xi)))
+        err = abs(mp.mpf(float(gi)) - ref)
+        assert err <= 4 * ULP * abs(ref), (xi, gi, float(ref))
+    assert abm(2, np.array([1.0]))[0] == 0.0
     x = np.exp(RNG.uniform(-5, 5, N))
     assert _relerr(abm(3, x)[np.abs(np.log10(x)) > 1e-3], x[np.abs(np.log10(x)) > 1e-3], mp.log10) <= 5 * ULP
 

@@ -1,4 +1,4 @@
-"""Per-call wall time of the host-array API (pinned buffers) for the bench workload; env knobs are read by the library."""
+"""Per-call wall time of the host-array API (pinned buffers) for the bench workload."""
 import os, sys, time
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -42,4 +42,4 @@ for s in range(4):
     best.append(np.median(ts[2:-1]))
     if os.environ.get("E2E_SORT"):
         ab.set_sort(int(os.environ["E2E_SORT"]))
-print(f"slab={os.environ.get('E2E_SLAB','1')} chunks={os.environ.get('AEROBULK_GPU_MAX_CHUNKS','6')} minpts={os.environ.get('AEROBULK_GPU_MIN_CHUNK_POINTS','200000')}: median per call {min(best):.3f} ms  ({n / min(best) / 1e3:.0f} Mpt/s)")
+print(f"slab={os.environ.get('E2E_SLAB','1')}: median per call {min(best):.3f} ms  ({n / min(best) / 1e3:.0f} Mpt/s)")

@@ -175,12 +175,18 @@ def main():
              "#ifndef ABM_GTABLE\n#define ABM_GTABLE __device__ const\n#endif\n\nnamespace abm {\n\n"]
     ln2 = mp.log(2)
 
+    # EXP_C, LOG_C and the MATH_K entries L2E, L2T, LG2_HI, LG2_LO belong to the polynomial exp / exp10 / log, which the
+    # table-driven ones replaced: no code reads them.  They stay because ptxas pairs constant loads into LDCU.128 by their
+    # offsets in constant bank 3, which follow from every table declared before them.  Deleting the tables re-pairs the loads
+    # of every flux kernel; aligning every table to 16 bytes, which makes the deletion neutral, by itself changes the
+    # registers and spills of 61 of the 126 kernels and made ANDREAS 3.9 % slower on a B200 (profiles/sass_compare_r03e.txt,
+    # profiles/ptxas_align_r03e.txt, profiles/kbench_4320x2160_r03e.txt).
     # exp(r), |r| <= ln2/2, degree 11
     a = ln2 / 2 * mp.mpf("1.0001")
     cs = cheb_fit(mp.exp, -a, a, 11)
     e = max_err(mp.exp, cs, -a, a)
     print("exp  deg 11 rel err %.3e (2^%.1f)" % (e, mp.log(e, 2)))
-    parts.append(emit("EXP_C", cs, "exp(r) on |r| <= ln2/2, c0..c11; max rel err %.2e" % e))
+    parts.append(emit("EXP_C", cs, "exp(r) on |r| <= ln2/2, c0..c11; max rel err %.2e (read by no kernel, kept for the bank layout)" % e))
 
     # log: P(z) = (2 atanh(s) - 2 s) / s^3 with z = s^2, s in [0, 0.1716]; log(m) = 2s + s*z*P(z)
     zmax = ((mp.sqrt(2) - 1) / (mp.sqrt(2) + 1)) ** 2 * mp.mpf("1.001")
@@ -196,7 +202,7 @@ def main():
         # error contribution relative to log(m) ~ 2s: s*z*dP / (2s) = z*dP/2
         print("log  deg %d rel err of P %.3e -> rel err of log <= %.3e" % (deg, e, e * zmax / 2 * mp.mpf(2) / 3))
     cs = cheb_fit(P, mp.mpf(0), zmax, 6)
-    parts.append(emit("LOG_C", cs, "(2 atanh(s) - 2s)/s^3 in z = s^2 on [0, 0.0295], c0..c6"))
+    parts.append(emit("LOG_C", cs, "(2 atanh(s) - 2s)/s^3 in z = s^2 on [0, 0.0295], c0..c6 (read by no kernel, kept for the bank layout)"))
 
     # atan(t) = t + t*z*Q(z), z = t^2, |t| <= tan(pi/8); Q(z) = (atan(t) - t)/t^3
     tmax = mp.tan(mp.pi / 8) * mp.mpf("1.0001")
@@ -223,7 +229,7 @@ def main():
     print("exp(table) q deg 3: rel err of q %.3e -> rel err of exp <= %.3e" % (e, e * a * a))
     parts.append(emit("EXPT_C", cs, "(exp(r) - 1 - r)/r^2 on |r| <= ln2/128, c0..c3"))
     tab = [mp.mpf(2) ** (mp.mpf(j) / 64) for j in range(64)]
-    parts.append("// 2^(j/64), j = 0..63 (read with __ldg: stays in L1)\nABM_GTABLE double EXP_T[64] = {\n" +
+    parts.append("// 2^(j/64), j = 0..63 (copied to shared memory by abm::load_tables)\nABM_GTABLE double EXP_T[64] = {\n" +
                  ",\n".join(f"    {float(t).hex()}" for t in tab) + "\n};\n\n")
 
     # ---- table-driven log: m in [0.708, 1.416) cut into 256 intervals of 4096 hi-word units; c_j = centre

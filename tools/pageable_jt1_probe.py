@@ -1,6 +1,5 @@
 """Wall time of a jt = Nt = 1 host-array call with PAGEABLE arrays (the plain relink case at the first step of a session):
-the copy threads feed the staged pipeline chunk by chunk.  Env knobs of the library apply (AEROBULK_GPU_HOST_THREADS,
-AEROBULK_GPU_SPEC_CHUNKS, ...).   usage: python tools/pageable_jt1_probe.py [Ni Nj] [algo] [skin 0/1]"""
+the copy threads feed the staged pipeline chunk by chunk.  AEROBULK_GPU_HOST_THREADS applies.   usage: python tools/pageable_jt1_probe.py [Ni Nj] [algo] [skin 0/1]"""
 import os, sys, time
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -24,4 +23,4 @@ for rep in range(6):
 ms = 1e3 * float(np.median(ts[2:]))
 nb = (8 + 6 if skin else 6 + 5) * 8 * Ni * Nj
 print(f"{algo}{'+skin' if skin else ''} {Ni}x{Nj} pageable jt=1: {ms:8.2f} ms  {Ni * Nj / ms / 1e6:6.3f} Gpt/s  host arrays {nb / 1e9:.2f} GB -> {nb / ms / 1e6:6.1f} GB/s "
-      f"(threads {os.environ.get('AEROBULK_GPU_HOST_THREADS', 'default')}, chunks {os.environ.get('AEROBULK_GPU_SPEC_CHUNKS', 'default')})")
+      f"(threads {os.environ.get('AEROBULK_GPU_HOST_THREADS', 'default')})")

@@ -31,7 +31,7 @@ for f in set(k[0] for k in cnt if k):
         continue
     name = "?"
     for n, line in enumerate(open(path), 1):
-        m = re.match(r"^(?:template.*\n)?(?:ABD|ABD_HEAVY|ABM_FN|__global__|__device__|static)[^(;]*?(\w+)\s*\(", line)
+        m = re.match(r"^(?:template.*\n)?(?:ABD|ABM_FN|__global__|__device__|static)[^(;]*?(\w+)\s*\(", line)
         if m and not line.startswith(" "):
             name = m.group(1)
         fmap[(f, n)] = name
