@@ -7,8 +7,10 @@
 // (Fortran, column-major) order, FP64 -- or FP32 for the whole of an aerobulk_gpu_model*_f32
 // call; a row block j0..j1 is the byte range [j0*Ni*es, j1*Ni*es) of each field (es = 8 or
 // 4 bytes per element), so chunks and shards are plain pointer offsets.
-// Host-array calls stage through 8 input + 6 output device arrays (grow-only) and are
-// pipelined in row-block chunks over three streams (H2D | kernel | D2H).
+// Every host-array call moves the caller's arrays through one transport (Transport): device pointers, device aliases
+// of pinned arrays, or one pair of grow-only slabs per session (a pinned one the copy threads fill, a device one for
+// staged copies) shared by all entry points; aerobulk_model pipelines it in row-block chunks over three streams
+// (H2D | kernel | D2H).
 // Warm-layer state never leaves the device between jt==1 and jt==nitend.
 // the library is built with -fvisibility=hidden: only the declared C ABI is exported
 #pragma GCC visibility push(default)
@@ -175,23 +177,17 @@ struct Session {
     long long n_coare = 0, n_ecmwf = 0, cap_coare = 0, cap_ecmwf = 0;
     double *c_state[4] = {nullptr, nullptr, nullptr, nullptr};   // dT_wl, Hz_wl, Qnt_ac, Tau_ac
     double *e_dT_wl = nullptr;
-    // ---- staging for host-array calls: 14 rows of `cap` bytes (a multiple of ROW_ALIGN), for FP64 and FP32 calls alike
-    long long cap = 0;
-    char *d_in[8] = {}, *d_out[6] = {};
-    // ---- pinned bounce slab for pageable caller arrays (14 rows, pitch cap_hb bytes: a multiple of ROW_ALIGN) and its device alias
-    char *hb = nullptr, *hb_dev = nullptr;
-    long long cap_hb = 0;
-    // ---- the same for the other host-array entry points (turb, series, ice): arrays packed back to back
-    double *hx = nullptr, *hx_dev = nullptr;
-    long long cap_hx = 0;
-    // ---- device slab of the other host-array entry points: staging and scratch (grow-only, see ensure_turb_slab)
-    double *d_turb = nullptr;
-    long long cap_turb = 0;
+    // ---- the two slabs of every host-array call (see Transport), grow-only, capacities in bytes: the pinned slab of
+    // pageable caller arrays and its device alias, and the device slab of staged copies and scratch
+    char *h_slab = nullptr, *h_slab_dev = nullptr;
+    long long cap_h_slab = 0;
+    char *d_slab = nullptr;
+    long long cap_d_slab = 0;
     // ---- stability-sort permutation (one uint16 per point, see classify_kernel)
     unsigned short *d_perm = nullptr;
     long long cap_perm = 0;
     int sort_points = 1;   // 0 never, 1 auto (where it measured faster), 2 always
-    bool pitched_ok = true;       // pitched (2-D) staging copies allowed, see copy_fields
+    bool pitched_ok = true;       // pitched (2-D) staging copies allowed, see Transport::copy
     int ice_form_per_point = 0;   // 0: LG15 form drag from the LAST point's ice fraction (reference), 1: per point
     // ---- statistics + deferred wind-stress flag
     double *d_partials = nullptr, *d_stats = nullptr;
@@ -418,114 +414,42 @@ void bind_wl_state(Args &a, int ialgo, long long s0)
     }
 }
 
-// Moves elements [s0, s0+len) of `nf` fields of es-byte elements between host and device staging (dev_pitch: bytes
-// between device rows).  Consecutive fields whose HOST arrays are equally spaced in memory (a caller that keeps its
-// fields in one slab) go in ONE pitched copy: with H2D and D2H running concurrently in 0.4-3 MB pieces the DMA engines
-// reach 62 GB/s aggregate, with one pitched copy per chunk 72 GB/s (tools/probes/duplex_probe.cu on this pool's B200:
-// 1.86 -> 1.62 ms per 1 M-point skin call).
-int copy_fields(int nf, char *const *dev, char *const *host, long long dev_pitch, long long s0, long long len, size_t es,
-                bool h2d, cudaStream_t st)
-{
-    const long long MAX_PITCH_BYTES = 0x7fffffffLL;   // cudaDevAttrMaxPitch
-    const long long o = s0 * (long long)es, bytes = len * (long long)es;
-    int k = 0;
-    while (k < nf) {
-        if (!host[k]) { ++k; continue; }
-        int run = 1;
-        if (k + 1 < nf && host[k + 1]) {
-            const long long d = host[k + 1] - host[k];   // bytes
-            if (d >= bytes && d <= MAX_PITCH_BYTES && dev_pitch <= MAX_PITCH_BYTES)
-                while (k + run < nf && host[k + run] && host[k + run] - host[k + run - 1] == d) ++run;
-        }
-        if (run > 1 && g.pitched_ok) {
-            const size_t hp = (size_t)(host[k + 1] - host[k]), dp = (size_t)dev_pitch, w = (size_t)bytes;
-            const cudaError_t e =
-                h2d ? cudaMemcpy2DAsync(dev[k] + o, dp, host[k] + o, hp, w, (size_t)run, cudaMemcpyHostToDevice, st)
-                    : cudaMemcpy2DAsync(host[k] + o, hp, dev[k] + o, dp, w, (size_t)run, cudaMemcpyDeviceToHost, st);
-            if (e == cudaErrorInvalidValue) {
-                // equally spaced but SEPARATE pinned allocations: the driver refuses a pitched copy that spans them.
-                // Nothing was enqueued; use plain copies from now on.
-                cudaGetLastError();
-                g.pitched_ok = false;
-                continue;
-            }
-            CUDA_TRY(e);
-        } else if (run > 1) {
-            for (int j = k; j < k + run; ++j) {
-                if (h2d) CUDA_TRY(cudaMemcpyAsync(dev[j] + o, host[j] + o, (size_t)bytes, cudaMemcpyHostToDevice, st));
-                else CUDA_TRY(cudaMemcpyAsync(host[j] + o, dev[j] + o, (size_t)bytes, cudaMemcpyDeviceToHost, st));
-            }
-        } else {
-            if (h2d) CUDA_TRY(cudaMemcpyAsync(dev[k] + o, host[k] + o, (size_t)bytes, cudaMemcpyHostToDevice, st));
-            else CUDA_TRY(cudaMemcpyAsync(host[k] + o, dev[k] + o, (size_t)bytes, cudaMemcpyDeviceToHost, st));
-        }
-        k += run;
-    }
-    return 0;
-}
-
-// Row pitch of the staging arrays and of the pinned slab: the bytes of one field (points x element size) rounded up to
-// ROW_ALIGN.  Both are grow-only and shared by FP64 and FP32 calls, so a row sized for an odd number of floats must not
-// leave a later, smaller FP64 call with rows that are not 8-byte aligned; 256 bytes also keeps every row on a whole
-// number of 128-byte lines for coalesced access.
+// Offsets in the slabs are multiples of ROW_ALIGN bytes.  Both slabs are grow-only and shared by FP64 and FP32 calls, so
+// an array sized for an odd number of floats must not leave a later, smaller FP64 call with arrays that are not 8-byte
+// aligned; 256 bytes also keeps every array on a whole number of 128-byte lines for coalesced access.
 constexpr long long ROW_ALIGN = 256;
 long long aligned_row(long long bytes) { return (bytes + ROW_ALIGN - 1) / ROW_ALIGN * ROW_ALIGN; }
 
-// `row`: bytes per field (points x element size)
-int ensure_staging(long long row)
+void free_pinned_slab()
 {
-    row = aligned_row(row);
-    if (row <= g.cap) return 0;
-    // one slab, fields equally spaced (pitch = cap bytes): a run of equally spaced caller arrays then moves with ONE
-    // pitched copy per chunk (see copy_fields)
-    if (g.d_in[0]) cudaFree(g.d_in[0]);
-    for (int k = 0; k < 8; ++k) g.d_in[k] = nullptr;
-    for (int k = 0; k < 6; ++k) g.d_out[k] = nullptr;
-    g.cap = 0;
-    char *slab = nullptr;
-    CUDA_TRY(cudaMalloc(&slab, (size_t)row * 14));
-    for (int k = 0; k < 8; ++k) g.d_in[k] = slab + (long long)k * row;
-    for (int k = 0; k < 6; ++k) g.d_out[k] = slab + (long long)(8 + k) * row;
-    g.cap = row;
-    return 0;
+    if (g.h_slab) cudaFreeHost(g.h_slab);
+    g.h_slab = g.h_slab_dev = nullptr;
+    g.cap_h_slab = 0;
 }
-
-void free_bounce()
+// Grows the mapped pinned slab to `bytes`.  False, with the slab released, when the host has no pinned memory to spare:
+// the session stays usable and the caller keeps the driver-staged copies.
+bool grow_mapped(long long bytes)
 {
-    if (g.hb) cudaFreeHost(g.hb);
-    g.hb = g.hb_dev = nullptr;
-    g.cap_hb = 0;
-    if (g.hx) cudaFreeHost(g.hx);
-    g.hx = g.hx_dev = nullptr;
-    g.cap_hx = 0;
-}
-// Grows a mapped pinned slab to `rows` rows of n elements of type T (cap counts n).  False, with the slab released, when
-// the host has no pinned memory to spare: the session stays usable and the caller keeps the driver-staged copies.
-template <class T>
-bool grow_mapped(T *&h, T *&d, long long &cap, long long n, int rows)
-{
-    if (n <= cap) return true;
-    if (h) cudaFreeHost(h);
-    h = d = nullptr;
-    cap = 0;
-    if (cudaHostAlloc(&h, sizeof(T) * (size_t)n * rows, cudaHostAllocPortable | cudaHostAllocMapped) != cudaSuccess ||
-        cudaHostGetDevicePointer(&d, h, 0) != cudaSuccess) {
+    if (bytes <= g.cap_h_slab) return true;
+    free_pinned_slab();
+    if (cudaHostAlloc(&g.h_slab, (size_t)bytes, cudaHostAllocPortable | cudaHostAllocMapped) != cudaSuccess ||
+        cudaHostGetDevicePointer(&g.h_slab_dev, g.h_slab, 0) != cudaSuccess) {
         cudaGetLastError();
-        if (h) cudaFreeHost(h);
-        h = d = nullptr;
+        free_pinned_slab();
         return false;
     }
-    cap = n;
+    g.cap_h_slab = bytes;
     return true;
 }
-// `row`: bytes per field (points x element size)
-bool ensure_bounce(long long row)
+int grow_device_slab(long long bytes)
 {
-    row = aligned_row(row);
-    if (row <= g.cap_hb) return true;
-    if ((size_t)row * 14 > bounce_max_bytes()) return false;
-    free_bounce();
-    return grow_mapped(g.hb, g.hb_dev, g.cap_hb, row, 14);
+    if (bytes <= g.cap_d_slab) return 0;
+    if (g.d_slab) cudaFree(g.d_slab);
+    g.d_slab = nullptr;
+    g.cap_d_slab = 0;
+    CUDA_TRY(cudaMalloc(&g.d_slab, (size_t)bytes));
+    g.cap_d_slab = bytes;
+    return 0;
 }
 // appends the copy of `bytes` bytes from src to dst, cut into COPY_PIECE_BYTES pieces for the copy threads
 void add_pieces(std::vector<CopyPiece> &pieces, void *dst, const void *src, size_t bytes)
@@ -535,22 +459,195 @@ void add_pieces(std::vector<CopyPiece> &pieces, void *dst, const void *src, size
     for (size_t o = 0; o < bytes; o += COPY_PIECE_BYTES)
         pieces.push_back(CopyPiece{d + o, s + o, bytes - o < COPY_PIECE_BYTES ? bytes - o : COPY_PIECE_BYTES});
 }
-// copy points [s0, s0+len) of nf fields of es-byte elements between the caller's arrays and the bounce slab rows
-// row0.., on the copy threads
-void bounce_copy(int nf, char *const *user, int row0, long long s0, long long len, size_t es, bool to_slab)
-{
-    static thread_local std::vector<CopyPiece> pieces;
-    pieces.clear();
-    const long long o = s0 * (long long)es;
-    const size_t bytes = (size_t)len * es;
-    for (int k = 0; k < nf; ++k) {
-        if (!user[k]) continue;
-        char *u = user[k] + o, *b = g.hb + (long long)(row0 + k) * g.cap_hb + o;
-        if (to_slab) add_pieces(pieces, b, u, bytes);
-        else add_pieces(pieces, u, b, bytes);
+
+// ---------------------------------------------------------------------------
+// How the caller's arrays of a host-array call reach the kernel and come back.  The entry point registers each array
+// with its length, element size and role (input, output, or in/out that goes home only if the kernel changes it) and
+// asks for device-only scratch; open() picks the path and stores a device pointer in every registered slot.  The path
+// is the first that applies:
+//   DEVICE  the caller passed device pointers: they pass through, nothing moves;
+//   ALIAS   every array is pinned (cudaHostAlloc / cudaHostRegister) and zerocopy_on(): the kernel works on the
+//           caller's memory through its device aliases;
+//   BOUNCE  the longest array has BOUNCE_MIN_POINTS elements or more and the pinned slab fits bounce_max_bytes(): the
+//           copy threads move the arrays between the caller's memory and the pinned slab and the kernel works on the
+//           slab zero-copy (pageable cudaMemcpy is staged by the driver on one thread at ~14 GB/s; the copy threads move
+//           55-70 GB/s);
+//   STAGED  cudaMemcpyAsync through the device slab.
+// `must_stage` (jt == 1 of aerobulk_model with AEROBULK_INIT still to run) makes any host path STAGED; where it would
+// have been BOUNCE, the host side of the staged copies is the pinned slab (`slab_first`), fed by the copy threads.
+// The copies work on a range of points of every array (clipped to its length): aerobulk_model moves row-block chunks,
+// the other entry points one range over the longest array (copy_in, close).
+// Both slabs hold the arrays in one packed layout, every array at a ROW_ALIGN-byte offset; they are shared by every
+// entry point and both element sizes.  Growing one frees the old buffer: every host-array call ends synchronised, so
+// nothing in flight still uses it.  Scratch lives in the device slab on every path.
+// ---------------------------------------------------------------------------
+enum Path { DEVICE, ALIAS, BOUNCE, STAGED };
+struct Transport {
+    struct Array {
+        void *slot;         // the caller's pointer variable that receives the device pointer
+        char *host;         // the caller's array; NULL: absent (the slot gets NULL)
+        long long len;      // elements (scratch: bytes)
+        size_t es;          // bytes per element
+        bool in, home;      // copied in before the launch / home after it
+        long long off;      // bytes into the slabs
+        char *dev;          // what open() stores in the slot
+    };
+    std::vector<Array> arrays, scratch_rows;
+    Path path = DEVICE;
+    bool slab_first = false;
+    long long longest = 0;   // elements of the longest array
+
+    void add(void *slot, const void *h, long long len, size_t es, bool in, bool home)
+    {
+        arrays.push_back({slot, static_cast<char *>(const_cast<void *>(h)), len, es, in, home, 0, nullptr});
     }
-    pool_run(pieces.data(), (int)pieces.size());
-}
+    template <class T>
+    void in(const T **slot, const T *h, long long len) { add(slot, h, len, sizeof(T), true, false); }
+    template <class T>
+    void out(T **slot, T *h, long long len, bool home = true) { add(slot, h, len, sizeof(T), false, home); }
+    template <class T>
+    void inout(T **slot, T *h, long long len, bool home) { add(slot, h, len, sizeof(T), true, home); }
+    void scratch(void *slot, long long bytes) { scratch_rows.push_back({slot, nullptr, bytes, 1, false, false, 0, nullptr}); }
+
+    Path pick(long long total)
+    {
+        if (!zerocopy_on()) return STAGED;
+        bool pinned = true;
+        for (Array &a : arrays)
+            if (a.host && !(a.dev = device_alias(a.host))) {
+                pinned = false;
+                break;
+            }
+        if (pinned) return ALIAS;
+        if (!bounce_on() || longest < BOUNCE_MIN_POINTS || (size_t)total > bounce_max_bytes() || !grow_mapped(total))
+            return STAGED;
+        return BOUNCE;
+    }
+    int open(bool on_device, bool must_stage = false)
+    {
+        long long total = 0;
+        longest = 0;
+        for (Array &a : arrays) {
+            const long long m = (a.host && a.len > 0) ? a.len : 0;
+            a.off = total;
+            total += aligned_row(m * (long long)a.es);
+            longest = m > longest ? m : longest;
+        }
+        path = on_device ? DEVICE : pick(total);
+        slab_first = must_stage && path == BOUNCE;
+        if (must_stage && path != DEVICE) path = STAGED;
+        long long need = path == STAGED ? total : 0;
+        for (Array &s : scratch_rows) {
+            s.off = need;
+            need += aligned_row(s.len);
+        }
+        const int rc = grow_device_slab(need);
+        if (rc) return rc;
+        for (Array &s : scratch_rows) {
+            s.dev = g.d_slab + s.off;
+            memcpy(s.slot, &s.dev, sizeof(s.dev));
+        }
+        for (Array &a : arrays) {
+            if (!a.host || path == DEVICE) a.dev = a.host;
+            else if (path == BOUNCE) a.dev = g.h_slab_dev + a.off;
+            else if (path == STAGED) a.dev = g.d_slab + a.off;
+            memcpy(a.slot, &a.dev, sizeof(a.dev));
+        }
+        return 0;
+    }
+    // bytes of points [s0, s0+len) of array a (0: none)
+    static long long range_bytes(const Array &a, long long s0, long long len)
+    {
+        const long long e = s0 + len < a.len ? s0 + len : a.len;
+        return a.host && e > s0 ? (e - s0) * (long long)a.es : 0;
+    }
+    // points [s0, s0+len) of every `in` array into the pinned slab (to_slab) or of every `home` array out of it, on the
+    // copy threads
+    void bounce(bool to_slab, long long s0, long long len)
+    {
+        static thread_local std::vector<CopyPiece> pieces;
+        pieces.clear();
+        for (const Array &a : arrays) {
+            const long long b = (to_slab ? a.in : a.home) ? range_bytes(a, s0, len) : 0;
+            if (b <= 0) continue;
+            char *u = a.host + s0 * (long long)a.es, *s = g.h_slab + a.off + s0 * (long long)a.es;
+            if (to_slab) add_pieces(pieces, s, u, (size_t)b);
+            else add_pieces(pieces, u, s, (size_t)b);
+        }
+        pool_run(pieces.data(), (int)pieces.size());
+    }
+    // H2D of points [s0, s0+len) of every `in` array (h2d) or D2H of every `home` array, on stream st; the host side is
+    // the pinned slab under slab_first, else the caller's arrays.  Consecutive arrays whose host sides are equally spaced
+    // in memory (a caller that keeps its fields in one slab; the pinned slab) go in ONE pitched copy: with H2D and D2H
+    // running concurrently in 0.4-3 MB pieces the DMA engines reach 62 GB/s aggregate, with one pitched copy per chunk
+    // 72 GB/s (tools/probes/duplex_probe.cu on this pool's B200: 1.86 -> 1.62 ms per 1 M-point skin call).
+    int copy(bool h2d, long long s0, long long len, cudaStream_t st)
+    {
+        const long long MAX_PITCH_BYTES = 0x7fffffffLL;   // cudaDevAttrMaxPitch
+        struct Row {
+            char *h, *d;
+            long long bytes;
+        };
+        static thread_local std::vector<Row> rows;
+        rows.clear();
+        for (const Array &a : arrays) {
+            const long long b = (h2d ? a.in : a.home) ? range_bytes(a, s0, len) : 0;
+            if (b <= 0) continue;
+            const long long o = s0 * (long long)a.es;
+            rows.push_back({(slab_first ? g.h_slab + a.off : a.host) + o, a.dev + o, b});
+        }
+        size_t k = 0;
+        while (k < rows.size()) {
+            const Row &r = rows[k];
+            const bool next = k + 1 < rows.size();
+            const long long dh = next ? rows[k + 1].h - r.h : 0, dd = next ? rows[k + 1].d - r.d : 0;
+            size_t run = 1;
+            if (dh >= r.bytes && dh <= MAX_PITCH_BYTES && dd >= r.bytes && dd <= MAX_PITCH_BYTES)
+                while (k + run < rows.size() && rows[k + run].bytes == r.bytes && rows[k + run].h - rows[k + run - 1].h == dh &&
+                       rows[k + run].d - rows[k + run - 1].d == dd)
+                    ++run;
+            if (run > 1 && g.pitched_ok) {
+                const size_t w = (size_t)r.bytes;
+                const cudaError_t e = h2d ? cudaMemcpy2DAsync(r.d, (size_t)dd, r.h, (size_t)dh, w, run, cudaMemcpyHostToDevice, st)
+                                          : cudaMemcpy2DAsync(r.h, (size_t)dh, r.d, (size_t)dd, w, run, cudaMemcpyDeviceToHost, st);
+                if (e == cudaErrorInvalidValue) {
+                    // equally spaced but SEPARATE pinned allocations: the driver refuses a pitched copy that spans them.
+                    // Nothing was enqueued; use plain copies from now on.
+                    cudaGetLastError();
+                    g.pitched_ok = false;
+                    continue;
+                }
+                CUDA_TRY(e);
+            } else {
+                for (size_t j = k; j < k + run; ++j) {
+                    const Row &q = rows[j];
+                    if (h2d) CUDA_TRY(cudaMemcpyAsync(q.d, q.h, (size_t)q.bytes, cudaMemcpyHostToDevice, st));
+                    else CUDA_TRY(cudaMemcpyAsync(q.h, q.d, (size_t)q.bytes, cudaMemcpyDeviceToHost, st));
+                }
+            }
+            k += run;
+        }
+        return 0;
+    }
+    // the inputs of a whole call, before its launch
+    int copy_in()
+    {
+        if (path == BOUNCE) bounce(true, 0, longest);
+        return path == STAGED ? copy(true, 0, longest, compute_stream()) : 0;
+    }
+    // the outputs of a whole call, after its launch; the host paths block
+    int close()
+    {
+        if (path == DEVICE) return 0;
+        if (path == STAGED) {
+            const int rc = copy(false, 0, longest, compute_stream());
+            if (rc) return rc;
+        }
+        CUDA_TRY(cudaStreamSynchronize(compute_stream()));
+        if (path == BOUNCE) bounce(false, 0, longest);
+        return 0;
+    }
+};
 
 int algo_id(const char *calgo)
 {
@@ -905,45 +1002,29 @@ int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, d
         if (rc) return rc;
     }
 
-    // rad_lw before rad_sw: a caller slab [sst .. slp, rad_lw] with a per-step rad_sw elsewhere is one run + one array
-    auto in_p = [](const void *p) { return static_cast<const char *>(p); };
-    auto out_p = [](void *p) { return static_cast<char *>(p); };
-    const char *in_h[8] = {in_p(sst), in_p(t_zt), in_p(hum_zt), in_p(U_zu), in_p(V_zu), in_p(slp),
-                           lsrad ? in_p(rad_lw) : nullptr, lsrad ? in_p(rad_sw) : nullptr};
-    char *out_h[6] = {out_p(QL), out_p(QH), out_p(Tau_x), out_p(Tau_y), out_p(Evap), lsrad ? out_p(T_s) : nullptr};
-    const char *in_d[8] = {};   // what the kernels read and write
-    char *out_d[6] = {};
-    const long long row = n * (long long)es;   // bytes per field
-
-    // How the arrays reach the kernel, chosen once per call, in this order:
-    //   DEVICE  device pointers (aerobulk_gpu_model_device): one launch on them;
-    //   ALIAS   jt > 1 or AEROBULK_INIT already done, every array pinned: one launch on their device aliases, no sort;
-    //   BOUNCE  jt > 1, pageable arrays of BOUNCE_MIN_POINTS or more, and the pinned slab fits: the copy threads move kind-2
-    //           chunks between the caller's arrays and the slab, the kernel works on the slab zero-copy, no sort, and the
-    //           outputs go home two chunks behind the GPU;
-    //   STAGED  anything else: H2D | kernel | D2H through the device staging arrays, kind-1 chunks.
+    // How the arrays reach the kernel (Transport), chosen once per call:
+    //   DEVICE  one launch on the caller's device pointers (aerobulk_gpu_model_device);
+    //   ALIAS   one launch on the device aliases of pinned arrays, no sort;
+    //   BOUNCE  kind-2 chunks: the copy threads move them between the caller's arrays and the pinned slab, the kernel
+    //           works on the slab zero-copy, no sort, and the outputs go home two chunks behind the GPU;
+    //   STAGED  H2D | kernel | D2H through the device slab, kind-1 chunks.
     // At jt == 1 with AEROBULK_INIT still to run the path is STAGED whatever the arrays, with kind-3 chunks; `spec_init`:
     // there are two or more of them and AEROBULK_INIT runs speculatively chunk by chunk (below), otherwise the statistics
-    // are taken once all inputs are in.  `slab_first`: the arrays are pageable, BOUNCE_MIN_POINTS or more, and the pinned
-    // slab fits, so the pipeline copies from / to the slab and the copy threads feed it -- chunk by chunk under
-    // spec_init, otherwise whole.
-    enum Path { DEVICE, ALIAS, BOUNCE, STAGED } path = device_ptrs ? DEVICE : STAGED;
+    // are taken once all inputs are in.  `slab_first`: the path would have been BOUNCE, so the pipeline copies from / to
+    // the pinned slab and the copy threads feed it -- chunk by chunk under spec_init, otherwise whole.
+    // rad_lw before rad_sw: a caller slab [sst .. slp, rad_lw] with a per-step rad_sw elsewhere is one run + one array
+    const void *const in_h[8] = {sst, t_zt, hum_zt, U_zu, V_zu, slp, lsrad ? rad_lw : nullptr, lsrad ? rad_sw : nullptr};
+    void *const out_h[6] = {QL, QH, Tau_x, Tau_y, Evap, lsrad ? T_s : nullptr};
+    const char *in_d[8] = {};   // what the kernels read and write
+    char *out_d[6] = {};
+    Transport t;
+    for (int k = 0; k < 8; ++k) t.add(&in_d[k], in_h[k], n, es, true, false);
+    for (int k = 0; k < 6; ++k) t.add(&out_d[k], out_h[k], n, es, false, true);
     const bool init_stats = jt == 1 && !g.preinit_done;   // this call takes AEROBULK_INIT's field statistics
-    const bool slab_ok = bounce_on() && zerocopy_on() && n >= BOUNCE_MIN_POINTS;   // the kernel reads the slab zero-copy
-    auto alias_all = [&] {   // device aliases of every array into in_d / out_d; false at the first array without one
-        for (int k = 0; k < 8; ++k)
-            if (in_h[k] && !(in_d[k] = device_alias(in_h[k]))) return false;
-        for (int k = 0; k < 6; ++k)
-            if (out_h[k] && !(out_d[k] = device_alias(out_h[k]))) return false;
-        return true;
-    };
-    bool slab_first = false;
-    if (!device_ptrs && init_stats) {
-        slab_first = slab_ok && !alias_all() && ensure_bounce(row);
-    } else if (!device_ptrs) {
-        if (n > 0 && zerocopy_on() && alias_all()) path = ALIAS;
-        else if (slab_ok && ensure_bounce(row)) path = BOUNCE;
-    }
+    rc = t.open(device_ptrs, init_stats);
+    if (rc) return rc;
+    const Path path = t.path;
+    const bool slab_first = t.slab_first;
     long long cstart[MAX_CHUNKS + 1];
     const int nchunks = plan_chunks(n, path == BOUNCE ? 2 : path == STAGED ? (init_stats ? 3 : 1) : 0, cstart);
     // Speculative AEROBULK_INIT (jt == 1 of a staged host-array call with >= 2 chunks).  The reference judges the WHOLE
@@ -956,40 +1037,13 @@ int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, d
     // written are then undefined.  Same results, H2D and D2H overlapped: C5 end to end 0.54 -> ~1 Gpt/s.
     const bool spec_init = path == STAGED && init_stats && nchunks >= 2;
 
-    // through the slab: the caller's arrays move to user_in / user_out, in_h / out_h name the slab rows
-    char *user_in[8] = {}, *user_out[6] = {};
-    if (slab_first || path == BOUNCE) {
-        for (int k = 0; k < 8; ++k) {
-            user_in[k] = const_cast<char *>(in_h[k]);
-            in_h[k] = in_h[k] ? g.hb + (long long)k * g.cap_hb : nullptr;
-        }
-        for (int k = 0; k < 6; ++k) {
-            user_out[k] = out_h[k];
-            out_h[k] = out_h[k] ? g.hb + (long long)(8 + k) * g.cap_hb : nullptr;
-        }
-    }
-    if (path == STAGED) {
-        rc = ensure_staging(row);
-        if (rc) return rc;
-    }
-    for (int k = 0; k < 8; ++k) {
-        if (!in_h[k] || path == DEVICE) in_d[k] = in_h[k];
-        else if (path == BOUNCE) in_d[k] = g.hb_dev + (long long)k * g.cap_hb;
-        else if (path == STAGED) in_d[k] = g.d_in[k];
-    }
-    for (int k = 0; k < 6; ++k) {
-        if (!out_h[k] || path == DEVICE) out_d[k] = out_h[k];
-        else if (path == BOUNCE) out_d[k] = g.hb_dev + (long long)(8 + k) * g.cap_hb;
-        else if (path == STAGED) out_d[k] = g.d_out[k];
-    }
-
-    if (slab_first && !spec_init) bounce_copy(8, user_in, 0, 0, n, es, true);
+    if (slab_first && !spec_init) t.bounce(true, 0, n);
     // H2D of chunk c on the copy-in stream (preceded by its way into the slab on the copy threads where that applies)
     auto enqueue_h2d = [&](int c) -> int {
         const long long s0 = cstart[c], len = cstart[c + 1] - s0;
         if (len > 0 && path == STAGED) {
-            if (slab_first && spec_init) bounce_copy(8, user_in, 0, s0, len, es, true);
-            const int r = copy_fields(8, g.d_in, const_cast<char *const *>(in_h), g.cap, s0, len, es, true, g.in_stream);
+            if (slab_first && spec_init) t.bounce(true, s0, len);
+            const int r = t.copy(true, s0, len, g.in_stream);
             if (r) return r;
         }
         CUDA_TRY(cudaEventRecord(g.ev_in[c], g.in_stream));
@@ -1133,7 +1187,7 @@ int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, d
         CUDA_TRY(cudaEventRecord(g.ev_k[c], cs));
         CUDA_TRY(cudaStreamWaitEvent(g.out_stream, g.ev_k[c], 0));
         if (path != STAGED) return 0;
-        return copy_fields(6, g.d_out, out_h, g.cap, cstart[c], cstart[c + 1] - cstart[c], es, false, g.out_stream);
+        return t.copy(false, cstart[c], cstart[c + 1] - cstart[c], g.out_stream);
     };
 
     int launched[MAX_CHUNKS], n_launched = 0, n_home = 0;
@@ -1141,7 +1195,7 @@ int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, d
     for (int c = 0; c < nchunks; ++c) {
         const long long s0 = cstart[c], len = cstart[c + 1] - s0;
         if (len <= 0) continue;
-        if (path == BOUNCE) bounce_copy(8, user_in, 0, s0, len, es, true);
+        if (path == BOUNCE) t.bounce(true, s0, len);
         while (slab_first && spec_init && h2d_next <= c) {   // (normally enqueued one iteration ahead, below)
             rc = enqueue_h2d(h2d_next++);
             if (rc) return rc;
@@ -1173,7 +1227,7 @@ int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, d
             // ... and the chunks whose results have landed in the slab go home
             while (n_home < n_launched && cudaEventQuery(g.ev_out[launched[n_home]]) == cudaSuccess) {
                 const int h = launched[n_home++];
-                bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], es, false);
+                t.bounce(false, cstart[h], cstart[h + 1] - cstart[h]);
                 home[h] = true;
             }
         }
@@ -1182,7 +1236,7 @@ int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, d
             if (n_launched - n_home > 2) {
                 const int h = launched[n_home++];
                 CUDA_TRY(cudaEventSynchronize(g.ev_k[h]));
-                bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], es, false);
+                t.bounce(false, cstart[h], cstart[h + 1] - cstart[h]);
             }
         }
     }
@@ -1217,7 +1271,7 @@ int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, d
     while (path == BOUNCE && n_home < n_launched) {
         const int h = launched[n_home++];
         CUDA_TRY(cudaEventSynchronize(g.ev_k[h]));
-        bounce_copy(6, user_out, 8, cstart[h], cstart[h + 1] - cstart[h], es, false);
+        t.bounce(false, cstart[h], cstart[h + 1] - cstart[h]);
     }
     CUDA_TRY(cudaMemcpyAsync(g.h_bad, g.d_bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, cs));
     CUDA_TRY(cudaEventRecord(g.ev_bad, cs));
@@ -1236,7 +1290,7 @@ int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, d
         if (slab_first) {   // what is not home yet (everything, without the chunk-wise feed)
             for (int c = 0; c < nchunks; ++c) {
                 const long long s0 = cstart[c], len = cstart[c + 1] - s0;
-                if (len > 0 && !home[c]) bounce_copy(6, user_out, 8, s0, len, es, false);
+                if (len > 0 && !home[c]) t.bounce(false, s0, len);
             }
         }
         rc = resolve_init();   // an asynchronous AEROBULK_INIT of this session reports first, as in the reference
@@ -1264,7 +1318,7 @@ int model_impl(bool device_ptrs, size_t es, int jt, int Nt, const char *calgo, d
 // The caller makes the reference's call -- whole (Ni,Nj) fields, host arrays, src/mod_aerobulk.f90:176-269 -- and the
 // library partitions the flat point range into n contiguous shards (boundaries on multiples of 2048 points; for a
 // 2-D field these are latitude row blocks up to that rounding), one per GPU, each with its own session: streams,
-// staging, pinned bounce slab, warm-layer state, tau > 10 flag.  Points are independent, so there is no data-path
+// slabs, warm-layer state, tau > 10 flag.  Points are independent, so there is no data-path
 // exchange; the only combine is AEROBULK_INIT's field statistics at jt == 1 (StatsHook, in host memory: the devices
 // belong to one process).  Device 0's shard runs on the calling thread, the others on persistent host threads.
 // ---------------------------------------------------------------------------
@@ -1466,120 +1520,6 @@ int model_device(size_t es, int jt, int Nt, const char *calgo, double zt, double
     return rc;
 }
 
-// device slab of the staged host-array calls and of device-only scratch (grow-only)
-int ensure_turb_slab(long long need)
-{
-    if (need > g.cap_turb) {
-        if (g.d_turb) cudaFree(g.d_turb);
-        g.d_turb = nullptr;
-        g.cap_turb = 0;
-        if (need > 0) CUDA_TRY(cudaMalloc(&g.d_turb, sizeof(double) * (size_t)need));
-        g.cap_turb = need;
-    }
-    return 0;
-}
-
-// ---------------------------------------------------------------------------
-// Caller arrays of the entry points other than aerobulk_gpu_model (turb, series, turb_ice, oce_ice, series_ice).  The
-// entry point registers each array with its length and role and asks for device-only scratch; open() stores a device
-// pointer in every registered slot, close() brings the outputs home.  open() picks the first mode that applies:
-//   DEVICE  the caller passed device pointers: they pass through, nothing moves, close() does nothing;
-//   ALIAS   every array is pinned (cudaHostAlloc / cudaHostRegister) and zerocopy_on(): the kernel works on the
-//           caller's memory through its device aliases;
-//   BOUNCE  from BOUNCE_MIN_POINTS elements up, the copy threads pack the inputs into the pinned slab g.hx, the kernel
-//           works on the slab zero-copy and the copy threads bring the outputs home (pageable cudaMemcpy is staged by
-//           the driver on one thread at ~14 GB/s; the copy threads move 55-70 GB/s);
-//   STAGED  cudaMemcpyAsync through the device slab g.d_turb on the compute stream.
-// The three host modes block in close().  Scratch lives in g.d_turb in every mode.
-// ---------------------------------------------------------------------------
-struct HostTransport {
-    enum Mode { DEVICE, ALIAS, BOUNCE, STAGED };
-    struct Array {
-        double **slot;          // receives the device pointer
-        double *host;           // the caller's pointer; NULL: absent (the slot gets NULL)
-        long long len, off;     // elements; offset in the packed slab
-        bool in, home;          // copied in before the launch / home after it
-        double *dev;            // what open() stores in the slot
-    };
-    std::vector<Array> arrays, scratch_rows;
-    Mode mode = DEVICE;
-
-    void in(const double **slot, const double *h, long long len)
-    {
-        arrays.push_back({const_cast<double **>(slot), const_cast<double *>(h), len, 0, true, false, nullptr});
-    }
-    void out(double **slot, double *h, long long len, bool home = true) { arrays.push_back({slot, h, len, 0, false, home, nullptr}); }
-    void inout(double **slot, double *h, long long len, bool home) { arrays.push_back({slot, h, len, 0, true, home, nullptr}); }
-    void scratch(double **slot, long long len) { scratch_rows.push_back({slot, nullptr, len, 0, false, false, nullptr}); }
-
-    Mode pick(long long total, long long longest)
-    {
-        if (!zerocopy_on()) return STAGED;
-        bool pinned = true;
-        for (Array &a : arrays)
-            if (a.host && !(a.dev = device_alias(a.host))) {
-                pinned = false;
-                break;
-            }
-        if (pinned) return ALIAS;
-        if (!bounce_on() || longest < BOUNCE_MIN_POINTS || sizeof(double) * (size_t)total > bounce_max_bytes() ||
-            !grow_mapped(g.hx, g.hx_dev, g.cap_hx, total, 1))
-            return STAGED;
-        return BOUNCE;
-    }
-    // the copy threads move every array with `in` (to the slab) or `home` (from it)
-    void bounce(bool to_slab)
-    {
-        std::vector<CopyPiece> pieces;
-        for (const Array &a : arrays)
-            if (a.host && (to_slab ? a.in : a.home)) {
-                if (to_slab) add_pieces(pieces, g.hx + a.off, a.host, sizeof(double) * (size_t)a.len);
-                else add_pieces(pieces, a.host, g.hx + a.off, sizeof(double) * (size_t)a.len);
-            }
-        pool_run(pieces.data(), (int)pieces.size());
-    }
-    int open(int on_device)
-    {
-        long long total = 0, longest = 0;
-        for (Array &a : arrays) {
-            const long long m = (a.host && a.len > 0) ? a.len : 0;
-            a.off = total;
-            total += (m + 63) / 64 * 64;   // rows start on 512-byte boundaries
-            longest = m > longest ? m : longest;
-        }
-        mode = on_device ? DEVICE : pick(total, longest);
-        long long need = mode == STAGED ? total : 0;
-        for (Array &s : scratch_rows) {
-            s.off = need;
-            need += (s.len + 63) / 64 * 64;
-        }
-        const int rc = ensure_turb_slab(need);
-        if (rc) return rc;
-        for (Array &s : scratch_rows) *s.slot = g.d_turb + s.off;
-        for (Array &a : arrays) {
-            if (!a.host || mode == DEVICE) a.dev = a.host;
-            else if (mode == BOUNCE) a.dev = g.hx_dev + a.off;
-            else if (mode == STAGED) a.dev = g.d_turb + a.off;
-            if (mode == STAGED && a.host && a.in && a.len > 0)
-                CUDA_TRY(cudaMemcpyAsync(a.dev, a.host, sizeof(double) * (size_t)a.len, cudaMemcpyHostToDevice, compute_stream()));
-            *a.slot = a.dev;
-        }
-        if (mode == BOUNCE) bounce(true);
-        return 0;
-    }
-    int close()
-    {
-        if (mode == DEVICE) return 0;
-        if (mode == STAGED)
-            for (const Array &a : arrays)
-                if (a.host && a.home && a.len > 0)
-                    CUDA_TRY(cudaMemcpyAsync(a.host, a.dev, sizeof(double) * (size_t)a.len, cudaMemcpyDeviceToHost, compute_stream()));
-        CUDA_TRY(cudaStreamSynchronize(compute_stream()));
-        if (mode == BOUNCE) bounce(false);
-        return 0;
-    }
-};
-
 // ---------------------------------------------------------------------------
 // TURB_* (SURVEY.md 8f row 1)
 // ---------------------------------------------------------------------------
@@ -1630,7 +1570,7 @@ int turb_impl(const char *calgo, int kt, double zt, double zu, int Ni, int Nj, d
     double *optp[10] = {nullptr};
     static_assert(sizeof(aerobulk_gpu_turb_optional) == 10 * sizeof(double *), "10 optional outputs");
     if (opt) memcpy(optp, opt, sizeof(*opt));
-    HostTransport t;
+    Transport t;
     t.inout(&a.T_s, T_s, n, cs || wl);   // T_s, q_s come back only from the skin schemes
     t.inout(&a.q_s, q_s, n, cs || wl);
     t.in(&a.t_zt, t_zt, n); t.in(&a.q_zt, q_zt, n); t.in(&a.U_zu, U_zu, n);
@@ -1639,6 +1579,7 @@ int turb_impl(const char *calgo, int kt, double zt, double zu, int Ni, int Nj, d
     t.out(&a.Ubzu, Ubzu, n);
     for (int k = 0; k < 10; ++k) t.out(&a.opt[k], optp[k], n);
     rc = t.open(on_device);
+    if (!rc) rc = t.copy_in();
     if (rc) return rc;
     if (wl) bind_wl_state(a, ialgo, 0);
     CUDA_TRY(abk::launch_turb(ialgo, cs, wl, zt_eq_zu(zt, zu), a, cs_));
@@ -1692,17 +1633,18 @@ int series_impl(const char *calgo, int Nt, long long S, double zt, double zu, co
     a.u = make_uniform(zt, zu);
     a.bad_index = g.d_bad;
 
-    HostTransport t;
-    double *d_isd;   // isecday_utc is a host array in every mode
-    t.scratch(&d_isd, ((long long)Nt * (long long)sizeof(int) + 7) / 8);
+    Transport t;
+    int *d_isd;   // isecday_utc is a host array in every mode
+    t.scratch(&d_isd, (long long)sizeof(int) * Nt);
     t.in(&a.lon, lon, S);
     t.in(&a.sst, sst, n); t.in(&a.t_zt, t_zt, n); t.in(&a.hum_zt, hum_zt, n); t.in(&a.wnd, wind, n); t.in(&a.slp, slp, n);
     t.in(&a.rad_sw, rad_sw, n); t.in(&a.rad_lw, rad_lw, n);
     for (int k = 0; k < abk::NSERIES_OUT; ++k) t.out(&a.out[k], hout[k], n);
     rc = t.open(on_device);
+    if (!rc) rc = t.copy_in();
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(d_isd, isd, sizeof(int) * (size_t)Nt, cudaMemcpyHostToDevice, cs_));
-    a.isd = reinterpret_cast<const int *>(d_isd);
+    a.isd = d_isd;
     CUDA_TRY(abk::launch_series(ialgo, skin, zt_eq_zu(zt, zu), a, cs_));
     g.launches += 1;
     CUDA_TRY(cudaMemcpyAsync(g.h_bad, g.d_bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, cs_));
@@ -1968,13 +1910,14 @@ int turb_ice_impl(const char *calgo, double zt, double zu, int Ni, int Nj, const
     if (opt) memcpy(optp, opt, sizeof(*opt));
     abk::IceTurbArgs a;
     memset(&a, 0, sizeof(a));
-    HostTransport t;
+    Transport t;
     t.in(&a.Ts_i, Ts_i, n); t.in(&a.t_zt, t_zt, n); t.in(&a.qs_i, qs_i, n); t.in(&a.q_zt, q_zt, n); t.in(&a.U_zu, U_zu, n);
     t.in(&a.frice, need_frice ? frice : nullptr, n);
     t.out(&a.Cd, Cd, n); t.out(&a.Ch, Ch, n); t.out(&a.Ce, Ce, n); t.out(&a.t_zu, t_zu, n); t.out(&a.q_zu, q_zu, n);
     t.out(&a.Ubzu, Ubzu, n);
     for (int k = 0; k < 8; ++k) t.out(&a.opt[k], optp[k], n);
     rc = t.open(on_device);
+    if (!rc) rc = t.copy_in();
     if (rc) return rc;
     a.n = n;
     a.form_index = g.ice_form_per_point ? -1 : n - 1;
@@ -2016,15 +1959,16 @@ int oce_ice_impl(const char *calgo_ice, const char *calgo_oce, double zt, double
         out->UN10_w, out->Tau_w, out->QH_w, out->QL_w, out->Evap_w, out->Tau, out->QH, out->QL, out->Evap};
     abk::OceIceArgs a;
     memset(&a, 0, sizeof(a));
-    HostTransport t;
+    Transport t;
     t.in(&a.sit, sit, n); t.in(&a.sst, oalgo ? sst : nullptr, n); t.in(&a.t_zt, t_zt, n); t.in(&a.hum_zt, hum_zt, n);
     t.in(&a.wnd, wind, n); t.in(&a.slp, slp, n); t.in(&a.frice, frice, n);
     // the leads kernel writes out[17..34]: without leads they stay as the caller passed them
     for (int k = 0; k < abk::NOCEICE_OUT; ++k) t.out(&a.out[k], hout[k], n, oalgo || k < 17);
     // scratch for the four ice fluxes the cell means need when the caller does not want them
     for (int k = 0; k < 4 && oalgo; ++k)
-        if (!hout[13 + k]) t.scratch(&a.ice_flux[k], n);
+        if (!hout[13 + k]) t.scratch(&a.ice_flux[k], (long long)sizeof(double) * n);
     rc = t.open(on_device);
+    if (!rc) rc = t.copy_in();
     if (rc) return rc;
     for (int k = 0; k < 4 && oalgo; ++k)
         if (hout[13 + k]) a.ice_flux[k] = a.out[13 + k];
@@ -2074,11 +2018,12 @@ int series_ice_impl(const char *calgo, double zt, double zu, long long n, const 
     memcpy(hout, out, sizeof(hout));
     abk::IceSeriesArgs a;
     memset(&a, 0, sizeof(a));
-    HostTransport t;
+    Transport t;
     t.in(&a.sic, sic, n); t.in(&a.sit, sit, n); t.in(&a.t_zt, t_zt, n); t.in(&a.hum_zt, hum_zt, n); t.in(&a.wnd, wind, n);
     t.in(&a.slp, slp, n); t.in(&a.rad_sw, rad_sw, n); t.in(&a.rad_lw, rad_lw, n);
     for (int k = 0; k < abk::NICESERIES_OUT; ++k) t.out(&a.out[k], hout[k], n);
     rc = t.open(on_device);
+    if (!rc) rc = t.copy_in();
     if (rc) return rc;
     a.n = n;
     a.hum_kind = hum_kind;
@@ -2108,21 +2053,11 @@ int diag_impl(long long n, const double *const *fields, double *stats, int on_de
     a.n = n;
     a.partials = g.d_partials;
     a.out = g.d_stats;
-    if (on_device) {
-        for (int f = 0; f < abk::NDIAG_FIELDS; ++f) a.field[f] = fields[f];
-    } else {
-        int nf = 0;
-        for (int f = 0; f < abk::NDIAG_FIELDS; ++f) nf += fields[f] ? 1 : 0;
-        rc = ensure_turb_slab(n * nf);
-        if (rc) return rc;
-        double *p = g.d_turb;
-        for (int f = 0; f < abk::NDIAG_FIELDS; ++f) {
-            if (!fields[f] || n == 0) continue;
-            CUDA_TRY(cudaMemcpyAsync(p, fields[f], sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, cs_));
-            a.field[f] = p;
-            p += n;
-        }
-    }
+    Transport t;
+    for (int f = 0; f < abk::NDIAG_FIELDS; ++f) t.in(&a.field[f], fields[f], n);
+    rc = t.open(on_device);
+    if (!rc) rc = t.copy_in();
+    if (rc) return rc;
     const long long want = (n + 255) / 256;
     const int nblocks = (int)(want < 1 ? 1 : (want > abk::stats_max_blocks() ? abk::stats_max_blocks() : want));
     CUDA_TRY(abk::launch_diag(a, nblocks, cs_));
@@ -2452,13 +2387,12 @@ int aerobulk_gpu_init(int Nt, const char *calgo, int Ni, int Nj, const double *s
     double st[abk::NSTATS];
     memset(st, 0, sizeof(st));
     if (n > 0) {
-        rc = ensure_staging(n * (long long)sizeof(double));
-        if (rc) return rc;
-        cudaStream_t cs = compute_stream();
-        const double *h[7] = {sst, t_zt, hum_zt, U_zu, V_zu, slp, lsrad ? rad_lw : nullptr};
-        for (int k = 0; k < 7; ++k)
-            if (h[k]) CUDA_TRY(cudaMemcpyAsync(g.d_in[k], h[k], sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, cs));
-        rc = local_stats(n, sizeof(double), g.d_in[0], g.d_in[1], g.d_in[2], g.d_in[3], g.d_in[4], g.d_in[5], lsrad ? g.d_in[6] : nullptr, cs, st);
+        const double *h[7] = {sst, t_zt, hum_zt, U_zu, V_zu, slp, lsrad ? rad_lw : nullptr}, *d[7];
+        Transport t;
+        for (int k = 0; k < 7; ++k) t.in(&d[k], h[k], n);
+        rc = t.open(false);
+        if (!rc) rc = t.copy_in();
+        if (!rc) rc = local_stats(n, sizeof(double), d[0], d[1], d[2], d[3], d[4], d[5], d[6], compute_stream(), st);
         if (rc) return rc;
     }
     const bool skin_before = g.l_use_skin_schemes;
@@ -2563,17 +2497,13 @@ static void reset_session()   // the session of `cur`
         cudaDeviceSynchronize();
         free_coare_state();
         free_ecmwf_state();
-        free_bounce();
-        if (g.d_in[0]) cudaFree(g.d_in[0]);   // one slab, see ensure_staging
-        for (int k = 0; k < 8; ++k) g.d_in[k] = nullptr;
-        for (int k = 0; k < 6; ++k) g.d_out[k] = nullptr;
-        g.cap = 0;
+        free_pinned_slab();
+        if (g.d_slab) cudaFree(g.d_slab);
+        g.d_slab = nullptr;
+        g.cap_d_slab = 0;
         if (g.d_perm) cudaFree(g.d_perm);
         g.d_perm = nullptr;
         g.cap_perm = 0;
-        if (g.d_turb) cudaFree(g.d_turb);
-        g.d_turb = nullptr;
-        g.cap_turb = 0;
         if (g.h_bad) g.h_bad[0] = g.h_bad[1] = ~0ull;
         if (g.d_bad) cudaMemset(g.d_bad, 0xFF, 2 * sizeof(unsigned long long));
     }
@@ -2813,16 +2743,17 @@ int aerobulk_gpu_probe(int func, long long n, int nargs, const double *args, dou
     int rc = ensure_device();
     if (rc) return rc;
     if (n == 0) return 0;
-    rc = ensure_turb_slab(n * (nargs + 1));
+    const double *d_args;
+    double *d_out;
+    Transport t;
+    t.in(&d_args, args, n * nargs);   // nargs rows of n
+    t.out(&d_out, out, n);
+    rc = t.open(false);
+    if (!rc) rc = t.copy_in();
     if (rc) return rc;
-    cudaStream_t cs_ = compute_stream();
-    CUDA_TRY(cudaMemcpyAsync(g.d_turb, args, sizeof(double) * (size_t)n * nargs, cudaMemcpyHostToDevice, cs_));
-    double *d_out = g.d_turb + n * nargs;
-    CUDA_TRY(abk::launch_probe(func, n, nargs, g.d_turb, d_out, cs_));
+    CUDA_TRY(abk::launch_probe(func, n, nargs, d_args, d_out, compute_stream()));
     g.launches += 1;
-    CUDA_TRY(cudaMemcpyAsync(out, d_out, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, cs_));
-    CUDA_TRY(cudaStreamSynchronize(cs_));
-    return 0;
+    return t.close();
 }
 
 }  // extern "C"

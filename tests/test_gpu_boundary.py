@@ -381,7 +381,7 @@ def test_deferred_wind_stress_error_on_device_api(ab):
 
 def test_fields_in_one_slab_use_pitched_copies_and_agree(ab):
     """A caller that keeps its fields equally spaced in one slab gets one pitched copy per pipeline chunk
-    (copy_fields in ab_api.cu); results are bit-identical to separate arrays -- pageable and pinned slabs."""
+    (Transport::copy in ab_api.cu); results are bit-identical to separate arrays -- pageable and pinned slabs."""
     import torch
     Ni, Nj = 640, 400                      # 256 000 points: 1 chunk; plus a 3-chunk case below
     for (ni, nj) in ((Ni, Nj), (1440, 500)):

@@ -1,7 +1,7 @@
 """How the caller's arrays reach the kernel must not change what the turb, series and sea-ice entry points compute.
 
 Every case runs on 80 000 points (above the 65 536-point bounce threshold) through each transport of
-aerobulk_b200/csrc/ab_api.cu (HostTransport):
+aerobulk_b200/csrc/ab_api.cu (Transport):
   - pageable numpy arrays: the copy threads and the pinned bounce slab;
   - pinned torch tensors: device aliases of the caller's memory (zero-copy);
   - CUDA tensors with on_device = 1: the caller's device pointers;

@@ -1,10 +1,10 @@
 """How the caller's arrays reach the kernel must change neither what aerobulk_gpu_model computes nor how many kernels each
 call launches.
 
-model_impl (aerobulk_b200/csrc/ab_api.cu) takes one of four paths per call: the caller's device pointers; the device
-aliases of pinned arrays (zero-copy, jt > 1); pageable arrays through the library's pinned slab (jt > 1, from 65 536
-points up); staged copies.  At jt == 1 the staged pipeline runs with the speculative AEROBULK_INIT, fed from the slab when
-the arrays are pageable.  One session, jt = 1..3 of Nt = 3 with the warm-layer state carried on the device, runs through:
+model_impl (aerobulk_b200/csrc/ab_api.cu) takes one of the four paths of its Transport per call: the caller's device
+pointers; the device aliases of pinned arrays (zero-copy, jt > 1); pageable arrays through the library's pinned slab
+(jt > 1, from 65 536 points up); staged copies.  At jt == 1 the staged pipeline runs with the speculative AEROBULK_INIT,
+fed from the slab when the arrays are pageable.  One session, jt = 1..3 of Nt = 3 with the warm-layer state carried on the device, runs through:
   - CUDA tensors (aerobulk_gpu_model_device);
   - pinned torch tensors: staged with the speculative AEROBULK_INIT at jt == 1, zero-copy after;
   - pageable numpy arrays: the slab-fed speculative pipeline at jt == 1, the slab after;

@@ -1,5 +1,5 @@
 """Pageable (ordinary) host arrays of 65536 elements or more: the host-array entry points other than aerobulk_model move
-them through the library's pinned slab on its copy threads (aerobulk_b200/csrc/ab_api.cu: HostTransport) instead of
+them through the library's pinned slab on its copy threads (aerobulk_b200/csrc/ab_api.cu: Transport) instead of
 driver-staged copies.  Every point (station) is independent, so the same input cut in two pieces that each stay below the
 threshold (staged path) must give the same bits."""
 import numpy as np
